@@ -2,6 +2,7 @@
 import ctypes as C
 import os
 import subprocess
+import tempfile
 
 import numpy as np
 
@@ -12,7 +13,6 @@ ORACLE_DIR = os.path.join(ROOT, "oracle")
 ORACLE_SO = os.path.join(ORACLE_DIR, "liblancet_oracle.so")
 REF_SO = os.path.join(ORACLE_DIR, "_ref", "liblancet_ref_scoring.so")
 
-NATIVE_SO = os.path.join(ORACLE_DIR, "_native", "liblancet_oracle_native.so")
 NATIVE_FLAGS = "-O3 -march=native -std=c++17 -fPIC -ffp-contract=off -pthread"
 PORTABLE_FLAGS = "-O2 -std=c++17 -fPIC -ffp-contract=off -pthread"
 
@@ -26,25 +26,20 @@ def build_oracle():
 
 def load_native_oracle():
     """The oracle compiled ON THIS HOST with -O3 -march=native (SURVEY.md §8d asks for that build as the
-    CPU baseline).  The portable -O2 library travels with the repo; a -march=native binary cannot
-    (the build container and the GPU box have different CPUs), so it is built where it runs, into
-    oracle/_native/ (git-ignored).  Returns (lib, flags); falls back to the portable build."""
+    CPU baseline).  build() makes the portable -O2 library; a -march=native binary cannot travel to
+    another machine's CPU, so it is compiled where it runs, into a temporary directory that is removed
+    once the library is loaded (the repository tree may be read-only).  Returns (lib, flags); falls back
+    to the portable build."""
     global _native
     if _native is not None:
         return _native
     try:
         srcs = [os.path.join(ORACLE_DIR, f) for f in ("mm2_restate.cpp", "genotype_oracle.cpp")]
-        newest = max(os.path.getmtime(x) for x in srcs + [os.path.join(ORACLE_DIR, "mm2_restate.hpp")])
-        marker = NATIVE_SO + ".host"
-        host = open("/proc/cpuinfo").read().split("model name")[1].split("\n")[0] if os.path.exists("/proc/cpuinfo") else ""
-        if (not os.path.exists(NATIVE_SO) or os.path.getmtime(NATIVE_SO) < newest or not os.path.exists(marker)
-                or open(marker).read() != host):
-            os.makedirs(os.path.dirname(NATIVE_SO), exist_ok=True)
-            subprocess.check_call(["g++"] + NATIVE_FLAGS.split() + ["-shared", "-o", NATIVE_SO] + srcs,
+        with tempfile.TemporaryDirectory(prefix="lancet2_b200_oracle_") as tmp:
+            so = os.path.join(tmp, "liblancet_oracle_native.so")
+            subprocess.check_call(["g++"] + NATIVE_FLAGS.split() + ["-shared", "-o", so] + srcs,
                                   stdout=subprocess.DEVNULL, stderr=subprocess.DEVNULL)
-            with open(marker, "w") as fh:
-                fh.write(host)
-        _native = (_bind(C.CDLL(NATIVE_SO)), NATIVE_FLAGS)
+            _native = (_bind(C.CDLL(so)), NATIVE_FLAGS)
     except Exception:  # noqa: BLE001 — no compiler on the box: the portable build is still a valid baseline
         _native = (load_oracle(), PORTABLE_FLAGS)
     return _native
