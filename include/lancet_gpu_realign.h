@@ -499,10 +499,15 @@ void lgr_repeat_destroy(lgr_rep_ctx* ctx);
 const char* lgr_repeat_last_error(const lgr_rep_ctx* ctx);
 /* H2D of the sequences and jobs, k_repeat_scan, D2H of one byte per job (0 / 1 / LGR_REPEAT_TOO_LONG).  Consecutive
  * jobs with the same seq_off, seq_len and max_mismatches (a window's k-loop) are answered together from shared mismatch
- * masks — keep them adjacent in `jobs`;
+ * masks — keep them adjacent in `jobs`.  A batch of fewer such groups than the GPU has resident CTAs spreads each group's
+ * diagonals over several CTAs (same answers);
  * ms_kernels (may be NULL) = CUDA-event time of the kernel. */
 int lgr_repeat_scan(lgr_rep_ctx* ctx, const uint8_t* seqs, int64_t seq_bytes, const lgr_repeat_job* jobs, int32_t n_jobs,
                     uint8_t* has_repeat, float* ms_kernels);
+/* allocate the device buffers of a batch of up to n_jobs jobs over up to seq_bytes bytes now: lgr_repeat_scan then never
+ * regrows them within these sizes (a regrow frees and allocates device memory, which synchronises the whole device and
+ * so stalls other work on it, e.g. a realignment batcher on the same GPU). */
+int lgr_repeat_reserve(lgr_rep_ctx* ctx, int64_t seq_bytes, int32_t n_jobs);
 
 #ifdef __cplusplus
 }

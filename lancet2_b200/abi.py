@@ -431,7 +431,7 @@ _SYMBOLS = [
     "lgr_set_notify", "lgr_reserve", "lgr_arena_bytes", "lgr_check_limits", "lgr_packed_group_bytes", "lgr_pack_group", "lgr_genotype_packed", "lgr_submit_packed", "lgr_upload_packed",
     "lgr_format_create", "lgr_format_destroy", "lgr_format_last_error", "lgr_format_metrics",
     "lgr_format_from_assign", "lgr_resident_assign", "lgr_format_debug_evidence",
-    "lgr_repeat_create", "lgr_repeat_destroy", "lgr_repeat_last_error", "lgr_repeat_scan",
+    "lgr_repeat_create", "lgr_repeat_destroy", "lgr_repeat_last_error", "lgr_repeat_scan", "lgr_repeat_reserve",
 ]
 
 
@@ -523,4 +523,6 @@ def load_library(path: Optional[str] = None) -> C.CDLL:
     lib.lgr_repeat_last_error.restype = C.c_char_p
     lib.lgr_repeat_scan.argtypes = [C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p, C.c_int32, C.c_void_p, C.POINTER(C.c_float)]
     lib.lgr_repeat_scan.restype = C.c_int
+    lib.lgr_repeat_reserve.argtypes = [C.c_void_p, C.c_int64, C.c_int32]
+    lib.lgr_repeat_reserve.restype = C.c_int
     return lib

@@ -17,6 +17,11 @@
 // same sequence with the same threshold (a window's whole k-loop) share one CTA: the mask of a diagonal is built once and
 // every still-open k is answered from it.  A job is closed at its first hit; the CTA stops when all its jobs are closed.
 // Byte compares on the raw ASCII, like the reference (case and IUPAC letters count as written).
+// A batch of few windows would leave most SMs idle under one CTA per group, so the unit of work is a (group, diagonal
+// slice) pair: the host splits each group into S slices (about resident CTAs / groups, at least one diagonal per warp)
+// and slice s takes diagonals 1 + s * 8 + warp, stepping by S * 8.  The slices of a group share a found word in global
+// memory for the early exit; the last slice to finish writes the answers.  Big batches get S = 1, the one-CTA schedule.
+// -DLGR_REPEAT_ONE_SLICE forces S = 1 (A/B builds).
 // There is no CPU fallback: lgr_repeat_create returns LGR_E_NO_DEVICE without a GPU.
 #include <cuda_runtime.h>
 
@@ -35,45 +40,57 @@ constexpr int kRepWarps = kRepThreads / 32;
 constexpr int kRepMaxLen = LGR_REPEAT_MAX_LEN;        // bases of one job's sequence (staged in shared memory)
 constexpr int kRepWords = kRepMaxLen / 32 + 2;        // mask words of one diagonal
 
-struct RepGroup {  // consecutive jobs over the same sequence with the same max_mismatches: they share the mismatch masks
-  int32_t first, n;
+constexpr int kRepCtasPerSm = 8;  // CTAs launched per SM: 2,048 threads, all resident with k_repeat_scan<true>'s 32 registers
+
+// one slice of a job group: consecutive jobs over the same sequence with the same max_mismatches share the mismatch masks
+struct RepItem {
+  int32_t first, n;       // the group's jobs
+  int32_t gid;            // the group's found / done words (slices > 1 only)
+  int16_t slice, slices;  // diagonals 1 + slice * kRepWarps + warp, stepping by slices * kRepWarps
 };
 
 struct RepDev {
   const uint8_t* seqs;
   const lgr_repeat_job* jobs;
-  const RepGroup* groups;
+  const RepItem* items;
   uint8_t* out;
-  int* next_group;  // work counter (groups differ by 20x in cost: a static stride would pair the heavy ones up)
-  int n_groups;
+  int* next_item;    // work counter (groups differ by 20x in cost: a static stride would pair the heavy ones up)
+  unsigned* found;   // per sliced group, zeroed before the launch: bit j = job j has its repeat (OR over the slices)
+  unsigned* done;    // per sliced group, zeroed before the launch: slices finished
+  int n_items;
 };
 
-constexpr int kRepGroupJobs = 32;  // k values handled by one CTA (a window's k-loop has 20)
+constexpr int kRepGroupJobs = 32;  // k values handled by one group (a window's k-loop has 20)
 
-// One CTA per job group.  The mismatch mask of a diagonal depends on the sequence and the offset only, not on k, so
+// One CTA per work item.  The mismatch mask of a diagonal depends on the sequence and the offset only, not on k, so
 // the warp builds it once and then answers every still-open k of the group from it: (1 + K) * n / 32 warp steps per
-// diagonal instead of 2 K * n / 32 (K = 20 for a window's k-loop: 1.9x fewer steps).
+// diagonal instead of 2 K * n / 32 (K = 20 for a window's k-loop: 1.9x fewer steps).  kSliced = false: every item is a
+// whole group (S = 1), compiled without the slice arithmetic and the global flags.
+template <bool kSliced>
 __global__ void __launch_bounds__(kRepThreads) k_repeat_scan(const RepDev D) {
   __shared__ uint8_t s_seq[kRepMaxLen];
   __shared__ uint32_t s_mask[kRepWarps][kRepWords];
   __shared__ uint16_t s_pre[kRepWarps][kRepWords];
   __shared__ int s_k[kRepGroupJobs];
-  __shared__ unsigned s_found;  // bit j: job j of the group has its repeat
+  __shared__ unsigned s_found;  // bit j: job j of the group has its repeat (this CTA's hits; a cache of *g_found when sliced)
+  __shared__ bool s_last;
   const unsigned full = 0xffffffffu;
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-  __shared__ int s_grp;
+  __shared__ int s_item;
   for (;;) {
-    __syncthreads();  // the previous group is finished with the shared arrays (and with s_grp)
-    if (threadIdx.x == 0) s_grp = atomicAdd(D.next_group, 1);
+    __syncthreads();  // the previous item is finished with the shared arrays (and with s_item)
+    if (threadIdx.x == 0) s_item = atomicAdd(D.next_item, 1);
     __syncthreads();
-    const int grp = s_grp;
-    if (grp >= D.n_groups) break;
-    const RepGroup G = D.groups[grp];
+    const int item = s_item;
+    if (item >= D.n_items) break;
+    const RepItem G = D.items[item];
+    const bool sliced = kSliced && G.slices > 1;
+    unsigned* g_found = D.found + G.gid;  // dereferenced only when sliced
     const lgr_repeat_job j0 = D.jobs[G.first];
     const int len = j0.seq_len, mm = j0.max_mismatches;
     if (threadIdx.x == 0) s_found = 0;
     if (threadIdx.x < G.n) s_k[threadIdx.x] = D.jobs[G.first + threadIdx.x].k;
-    if (len > kRepMaxLen) {  // not computed: flagged for the host
+    if (len > kRepMaxLen) {  // not computed: flagged for the host (such a group has one slice)
       if (threadIdx.x < G.n) D.out[G.first + threadIdx.x] = LGR_REPEAT_TOO_LONG;
       continue;
     }
@@ -86,11 +103,15 @@ __global__ void __launch_bounds__(kRepThreads) k_repeat_scan(const RepDev D) {
     const int d_end = len - k_min + 1;  // diagonals of the smallest k (base::SlidingView: none when the sequence is shorter than k)
     uint32_t* mask = s_mask[warp];
     uint16_t* pre = s_pre[warp];
-    for (int d = 1 + warp; d < d_end; d += kRepWarps) {
+    const int step = kSliced ? G.slices * kRepWarps : kRepWarps;
+    for (int d = 1 + (kSliced ? G.slice * kRepWarps : 0) + warp; d < d_end; d += step) {
       // which jobs are still open: one lane reads the flags (atomics on both sides, no data race) and the whole
       // warp follows its answer, so the lanes can never disagree about leaving the loop
       unsigned found = 0;
-      if (lane == 0) found = atomicOr(&s_found, 0u);
+      if (lane == 0) {
+        found = atomicOr(&s_found, 0u);
+        if (sliced) found |= atomicOr(g_found, 0u);  // the other slices' hits
+      }
       found = __shfl_sync(full, found, 0);
       if (found == all) break;
       const int span = len - d;  // positions p with a partner p + d
@@ -122,11 +143,27 @@ __global__ void __launch_bounds__(kRepThreads) k_repeat_scan(const RepDev D) {
         }
         if (__any_sync(full, hit)) newly |= 1u << q;
       }
-      if (newly && lane == 0) atomicOr(&s_found, newly);
+      if (newly && lane == 0) {
+        atomicOr(&s_found, newly);
+        if (sliced) atomicOr(g_found, newly);
+      }
       __syncwarp();
     }
     __syncthreads();
-    if (threadIdx.x < G.n) D.out[G.first + threadIdx.x] = (uint8_t)(s_found >> threadIdx.x & 1u);
+    if (!sliced) {
+      if (threadIdx.x < G.n) D.out[G.first + threadIdx.x] = (uint8_t)(s_found >> threadIdx.x & 1u);
+      continue;
+    }
+    // the last slice to finish writes the answers: the OR of the per-diagonal hits over a partition of the diagonals
+    if (threadIdx.x == 0) {
+      __threadfence();  // this slice's atomicOr on *g_found is ordered before its count
+      s_last = atomicAdd(D.done + G.gid, 1) == G.slices - 1;
+    }
+    __syncthreads();
+    if (s_last) {
+      __threadfence();
+      if (threadIdx.x < G.n) D.out[G.first + threadIdx.x] = (uint8_t)(atomicOr(g_found, 0u) >> threadIdx.x & 1u);
+    }
   }
 }
 
@@ -136,8 +173,13 @@ struct lgr_rep_ctx {
   int device = 0, sm_count = 0;
   cudaStream_t stream = nullptr;
   cudaEvent_t ev0 = nullptr, ev1 = nullptr;
-  void *d_seq = nullptr, *d_jobs = nullptr, *d_out = nullptr, *d_groups = nullptr, *d_ctr = nullptr;
-  size_t cap_seq = 0, cap_jobs = 0, cap_out = 0, cap_groups = 0, cap_ctr = 0;
+  void *d_seq = nullptr, *d_jobs = nullptr, *d_out = nullptr, *d_items = nullptr, *d_ctr = nullptr;
+  size_t cap_seq = 0, cap_jobs = 0, cap_out = 0, cap_items = 0, cap_ctr = 0;
+  struct Group {
+    int32_t first, n, k_min;
+  };
+  std::vector<Group> groups;  // host scratch of lgr_repeat_scan, kept to reuse its storage
+  std::vector<RepItem> items;
   std::string err;
 };
 
@@ -152,18 +194,31 @@ static thread_local std::string g_rep_create_err;
     }                                                                          \
   } while (0)
 
-static int rep_ensure(lgr_rep_ctx* c, void** p, size_t* cap, size_t bytes) {
+// grows *p to at least `bytes` (half as much again on a regrow inside lgr_repeat_scan, exactly on a reservation)
+static int rep_ensure(lgr_rep_ctx* c, void** p, size_t* cap, size_t bytes, bool exact = false) {
   if (bytes < 256) bytes = 256;
   if (*cap >= bytes) return LGR_OK;
   if (*p) cudaFree(*p);
   *p = nullptr, *cap = 0;
-  if (cudaMalloc(p, bytes + bytes / 2) != cudaSuccess) {
+  const size_t want = exact ? bytes : bytes + bytes / 2;
+  if (cudaMalloc(p, want) != cudaSuccess) {
     c->err = "cudaMalloc failed";
     (void)cudaGetLastError();
     return LGR_E_NOMEM;
   }
-  *cap = bytes + bytes / 2;
+  *cap = want;
   return LGR_OK;
+}
+
+// device buffers of a batch of n_jobs jobs over seq_bytes bytes: the work items are at most max(n_jobs, resident CTAs)
+// (a group gets several slices only while there are fewer groups than resident CTAs), the counter words 1 + 2 per group
+static int rep_buffers(lgr_rep_ctx* c, size_t seq_bytes, size_t n_jobs, size_t n_items, size_t ctr_words, bool exact) {
+  int rc;
+  if ((rc = rep_ensure(c, &c->d_seq, &c->cap_seq, seq_bytes, exact)) != LGR_OK) return rc;
+  if ((rc = rep_ensure(c, &c->d_jobs, &c->cap_jobs, sizeof(lgr_repeat_job) * n_jobs, exact)) != LGR_OK) return rc;
+  if ((rc = rep_ensure(c, &c->d_out, &c->cap_out, n_jobs, exact)) != LGR_OK) return rc;
+  if ((rc = rep_ensure(c, &c->d_items, &c->cap_items, sizeof(RepItem) * n_items, exact)) != LGR_OK) return rc;
+  return rep_ensure(c, &c->d_ctr, &c->cap_ctr, sizeof(unsigned) * ctr_words, exact);
 }
 
 extern "C" {
@@ -198,7 +253,7 @@ void lgr_repeat_destroy(lgr_rep_ctx* c) {
   if (c->d_seq) cudaFree(c->d_seq);
   if (c->d_jobs) cudaFree(c->d_jobs);
   if (c->d_out) cudaFree(c->d_out);
-  if (c->d_groups) cudaFree(c->d_groups);
+  if (c->d_items) cudaFree(c->d_items);
   if (c->d_ctr) cudaFree(c->d_ctr);
   if (c->ev0) cudaEventDestroy(c->ev0);
   if (c->ev1) cudaEventDestroy(c->ev1);
@@ -221,37 +276,56 @@ int lgr_repeat_scan(lgr_rep_ctx* c, const uint8_t* seqs, int64_t seq_bytes, cons
       return c->err = "bad repeat job (offsets outside the sequence buffer, k <= 0 or max_mismatches < 0)", LGR_E_ARG;
     too_long |= j.seq_len > LGR_REPEAT_MAX_LEN;
   }
-  // consecutive jobs over the same sequence with the same threshold share one CTA (and its mismatch masks)
-  std::vector<RepGroup> groups;
+  // consecutive jobs over the same sequence with the same threshold form a group (sharing its mismatch masks)
+  std::vector<lgr_rep_ctx::Group>& groups = c->groups;
+  groups.clear();
   for (int i = 0; i < n_jobs;) {
-    int n = 1;
+    int n = 1, k_min = jobs[i].k;
     while (i + n < n_jobs && n < kRepGroupJobs && jobs[i + n].seq_off == jobs[i].seq_off && jobs[i + n].seq_len == jobs[i].seq_len &&
            jobs[i + n].max_mismatches == jobs[i].max_mismatches)
-      ++n;
-    groups.push_back(RepGroup{i, n});
+      k_min = std::min(k_min, jobs[i + n].k), ++n;
+    groups.push_back(lgr_rep_ctx::Group{i, n, k_min});
     i += n;
   }
   // the queue hands out the expensive groups first (cost ~ jobs x length^2): a short tail
-  std::stable_sort(groups.begin(), groups.end(), [&](const RepGroup& a, const RepGroup& b) {
+  std::stable_sort(groups.begin(), groups.end(), [&](const lgr_rep_ctx::Group& a, const lgr_rep_ctx::Group& b) {
     const int64_t la = jobs[a.first].seq_len, lb = jobs[b.first].seq_len;
     return (int64_t)(a.n + 1) * la * la > (int64_t)(b.n + 1) * lb * lb;
   });
+  // slices per group: enough work items to fill the resident CTAs, at least one diagonal per warp of a slice
+  const int n_groups = (int)groups.size(), resident = c->sm_count * kRepCtasPerSm;
+#ifdef LGR_REPEAT_ONE_SLICE
+  const int per_group = 1;
+#else
+  const int per_group = std::min(std::max(resident / n_groups, 1), (int)INT16_MAX);
+#endif
+  std::vector<RepItem>& items = c->items;
+  items.clear();
+  int n_sliced = 0;
+  for (const lgr_rep_ctx::Group& g : groups) {
+    const int len = jobs[g.first].seq_len, diagonals = len - g.k_min;  // d = 1 .. len - k_min
+    const int slices = len > kRepMaxLen ? 1 : std::max(1, std::min(per_group, diagonals / kRepWarps));
+    const int gid = slices > 1 ? n_sliced++ : 0;
+    for (int s = 0; s < slices; ++s) items.push_back(RepItem{g.first, g.n, gid, (int16_t)s, (int16_t)slices});
+  }
+  const int n_items = (int)items.size();
+  const size_t ctr_words = 1 + 2 * (size_t)n_sliced;  // queue counter, then found[n_sliced], done[n_sliced]
   REP_CUDA(c, cudaSetDevice(c->device));
   int rc;
-  if ((rc = rep_ensure(c, &c->d_seq, &c->cap_seq, (size_t)seq_bytes)) != LGR_OK) return rc;
-  if ((rc = rep_ensure(c, &c->d_jobs, &c->cap_jobs, sizeof(lgr_repeat_job) * (size_t)n_jobs)) != LGR_OK) return rc;
-  if ((rc = rep_ensure(c, &c->d_out, &c->cap_out, (size_t)n_jobs)) != LGR_OK) return rc;
-  if ((rc = rep_ensure(c, &c->d_groups, &c->cap_groups, sizeof(RepGroup) * groups.size())) != LGR_OK) return rc;
-  if ((rc = rep_ensure(c, &c->d_ctr, &c->cap_ctr, sizeof(int))) != LGR_OK) return rc;
-  REP_CUDA(c, cudaMemsetAsync(c->d_ctr, 0, sizeof(int), c->stream));
+  if ((rc = rep_buffers(c, (size_t)seq_bytes, (size_t)n_jobs, (size_t)n_items, ctr_words, false)) != LGR_OK) return rc;
+  REP_CUDA(c, cudaMemsetAsync(c->d_ctr, 0, sizeof(unsigned) * ctr_words, c->stream));
   if (seq_bytes > 0) REP_CUDA(c, cudaMemcpyAsync(c->d_seq, seqs, (size_t)seq_bytes, cudaMemcpyHostToDevice, c->stream));
   REP_CUDA(c, cudaMemcpyAsync(c->d_jobs, jobs, sizeof(lgr_repeat_job) * (size_t)n_jobs, cudaMemcpyHostToDevice, c->stream));
-  REP_CUDA(c, cudaMemcpyAsync(c->d_groups, groups.data(), sizeof(RepGroup) * groups.size(), cudaMemcpyHostToDevice, c->stream));
-  RepDev D{(const uint8_t*)c->d_seq, (const lgr_repeat_job*)c->d_jobs, (const RepGroup*)c->d_groups, (uint8_t*)c->d_out, (int*)c->d_ctr, (int)groups.size()};
+  REP_CUDA(c, cudaMemcpyAsync(c->d_items, items.data(), sizeof(RepItem) * items.size(), cudaMemcpyHostToDevice, c->stream));
+  unsigned* ctr = (unsigned*)c->d_ctr;
+  RepDev D{(const uint8_t*)c->d_seq, (const lgr_repeat_job*)c->d_jobs, (const RepItem*)c->d_items, (uint8_t*)c->d_out,
+           (int*)ctr, ctr + 1, ctr + 1 + n_sliced, n_items};
   REP_CUDA(c, cudaEventRecord(c->ev0, c->stream));
-  const int n_groups = (int)groups.size();
-  const int grid = n_groups < c->sm_count * 8 ? n_groups : c->sm_count * 8;
-  k_repeat_scan<<<grid, kRepThreads, 0, c->stream>>>(D);
+  const int grid = n_items < resident ? n_items : resident;
+  if (n_sliced > 0)
+    k_repeat_scan<true><<<grid, kRepThreads, 0, c->stream>>>(D);
+  else
+    k_repeat_scan<false><<<grid, kRepThreads, 0, c->stream>>>(D);
   REP_CUDA(c, cudaGetLastError());
   REP_CUDA(c, cudaEventRecord(c->ev1, c->stream));
   REP_CUDA(c, cudaMemcpyAsync(has_repeat, c->d_out, (size_t)n_jobs, cudaMemcpyDeviceToHost, c->stream));
@@ -262,6 +336,17 @@ int lgr_repeat_scan(lgr_rep_ctx* c, const uint8_t* seqs, int64_t seq_bytes, cons
     return LGR_E_PARTIAL;
   }
   return LGR_OK;
+}
+
+int lgr_repeat_reserve(lgr_rep_ctx* c, int64_t seq_bytes, int32_t n_jobs) {
+  if (!c || seq_bytes < 0 || n_jobs < 0) return LGR_E_ARG;
+  c->err.clear();
+  REP_CUDA(c, cudaSetDevice(c->device));
+  const size_t resident = (size_t)c->sm_count * kRepCtasPerSm;
+  const int rc = rep_buffers(c, (size_t)seq_bytes, (size_t)n_jobs, std::max((size_t)n_jobs, resident), 1 + 2 * (size_t)n_jobs, true);
+  c->groups.reserve((size_t)n_jobs);
+  c->items.reserve(std::max((size_t)n_jobs, resident));
+  return rc;
 }
 
 }  // extern "C"

@@ -2,6 +2,7 @@
 // drive the C++ adapter (ctypes) without a C++ test runner.  Test support only; the product
 // boundary is include/lancet_gpu_realign.h + host/gpu_genotyper.h.
 #include <algorithm>
+#include <atomic>
 #include <chrono>
 #include <cstdio>
 #include <cstring>
@@ -12,6 +13,7 @@
 #include <vector>
 
 #include "gpu_genotyper.h"
+#include "gpu_repeat.h"
 
 namespace {
 
@@ -438,6 +440,156 @@ int lgr_adapter_format_metrics(int device, const lgr_batch_in* in, const char* n
     std::snprintf(err, (size_t)err_cap, "%s", e.what());
     return -2;
   }
+}
+
+}  // extern "C"
+
+namespace {
+
+// The windows of a RepeatChecker run: window w = seqs[seq_off[w], seq_off[w] + seq_len[w]) with questions
+// q_begin[w] .. q_begin[w + 1] of (q_k, q_mm); its answers go to answers[q_begin[w] ..].
+struct RepeatWindows {
+  const unsigned char* seqs;
+  const long long* seq_off;
+  const int* seq_len;
+  int n_windows;
+  const int* q_begin;
+  const int* q_k;
+  const int* q_mm;
+  std::string_view Seq(int w) const { return {reinterpret_cast<const char*>(seqs) + seq_off[w], (std::size_t)seq_len[w]}; }
+  std::vector<lancet_gpu::RepeatQuestion> Questions(int w) const {
+    std::vector<lancet_gpu::RepeatQuestion> q;
+    for (int i = q_begin[w]; i < q_begin[w + 1]; ++i) q.push_back(lancet_gpu::RepeatQuestion{q_k[i], q_mm[i]});
+    return q;
+  }
+};
+
+// n_threads threads; thread t asks windows t, t + n_threads, ... (only window t when one_each), one blocking call each,
+// in order.  ask(w, t) returns the answers of window w; status[w] = 0 ok, 1 std::invalid_argument, 2 any other
+// exception.  after_start(returned) runs on the calling thread once every thread is running; returned counts the calls
+// that have come back.  Returns the wall nanoseconds from the start to the last join.
+template <typename Ask, typename AfterStart>
+unsigned long long RunWindows(const RepeatWindows& win, int n_threads, bool one_each, unsigned char* answers, int* status,
+                              Ask ask, AfterStart after_start) {
+  std::atomic<int> started{0}, returned{0};
+  std::vector<std::thread> threads;
+  const auto t0 = std::chrono::steady_clock::now();
+  for (int t = 0; t < n_threads; ++t) {
+    threads.emplace_back([&, t] {
+      started.fetch_add(1);
+      for (int w = t; w < win.n_windows; w += n_threads) {
+        try {
+          const std::vector<std::uint8_t> a = ask(w, t);
+          std::memcpy(answers + win.q_begin[w], a.data(), a.size());
+          status[w] = 0;
+        } catch (const std::invalid_argument&) {
+          status[w] = 1;
+        } catch (const std::exception&) {
+          status[w] = 2;
+        }
+        returned.fetch_add(1);
+        if (one_each) break;
+      }
+    });
+  }
+  while (started.load() < n_threads) std::this_thread::yield();
+  after_start(returned);
+  for (auto& th : threads) th.join();
+  return (unsigned long long)std::chrono::duration_cast<std::chrono::nanoseconds>(std::chrono::steady_clock::now() - t0).count();
+}
+
+}  // namespace
+
+extern "C" {
+
+// lancet_gpu::RepeatChecker for the tests and tools/bench_repeat_checker.py.  NULL (message in err) when construction
+// throws, e.g. without a GPU.
+void* lgr_adapter_repeat_checker_create(int device, long long max_seq_bytes, long long max_questions, char* err, int err_cap) {
+  try {
+    lancet_gpu::RepeatChecker::Options opt;
+    opt.device = device;
+    if (max_seq_bytes > 0) opt.max_seq_bytes = (std::size_t)max_seq_bytes;
+    if (max_questions > 0) opt.max_questions = (std::size_t)max_questions;
+    return new lancet_gpu::RepeatChecker(opt);
+  } catch (const std::exception& e) {
+    if (err && err_cap > 0) std::snprintf(err, (size_t)err_cap, "%s", e.what());
+    return nullptr;
+  }
+}
+
+void lgr_adapter_repeat_checker_destroy(void* checker) { delete static_cast<lancet_gpu::RepeatChecker*>(checker); }
+
+// n_threads C++ threads call RepeatChecker::Check on their share of the windows (see RunWindows).  counters[7] =
+// batches, windows, questions, max windows in a batch, checker-thread ns inside lgr_repeat_scan, wall ns of the run,
+// callers waiting when the checker was destroyed.  destroy != 0: thread t asks window t only (status of the windows
+// beyond n_threads: -1), and once every thread is inside Check or back from it, the checker is destroyed while its
+// callers wait (the caller must not destroy it again; counters[0..4] are then 0).
+int lgr_adapter_repeat_checker_run(void* checker, const unsigned char* seqs, const long long* seq_off, const int* seq_len,
+                                   int n_windows, const int* q_begin, const int* q_k, const int* q_mm, int n_threads,
+                                   int destroy, unsigned char* answers, int* status, unsigned long long* counters) {
+  if (!checker || n_threads <= 0 || n_windows < 0) return -1;
+  auto* chk = static_cast<lancet_gpu::RepeatChecker*>(checker);
+  const RepeatWindows win{seqs, seq_off, seq_len, n_windows, q_begin, q_k, q_mm};
+  for (int i = 0; i < 7; ++i) counters[i] = 0;
+  for (int w = 0; w < n_windows; ++w) status[w] = -1;
+  const int askers = destroy ? std::min(n_threads, n_windows) : n_threads;
+  const unsigned long long wall = RunWindows(
+      win, askers, destroy != 0, answers, status,
+      [&](int w, int) {
+        const std::vector<lancet_gpu::RepeatQuestion> q = win.Questions(w);
+        return chk->Check(win.Seq(w), q.data(), q.size());
+      },
+      [&](const std::atomic<int>& returned) {
+        if (!destroy) return;
+        // a thread that has not reached Check yet must not find the checker gone: wait until every one is inside
+        // (counted by Callers) or back (returned, read first so that no thread is missed by both reads)
+        for (;;) {
+          const int back = returned.load();
+          const std::size_t inside = chk->Callers();
+          if (back + (int)inside >= askers) {
+            counters[6] = inside;
+            break;
+          }
+          std::this_thread::yield();
+        }
+        delete chk;
+      });
+  if (!destroy) {
+    const lancet_gpu::RepeatChecker::Counters c = chk->Stats();
+    counters[0] = c.batches, counters[1] = c.windows, counters[2] = c.questions, counters[3] = c.max_windows_in_batch;
+    counters[4] = c.ns_wait;
+  }
+  counters[5] = wall;
+  return 0;
+}
+
+// The binding without the checker, for comparison: every thread owns an lgr_rep_ctx (created before the clock starts)
+// and makes one lgr_repeat_scan per window.  Returns the wall ns of the run, < 0 when a context cannot be created.
+long long lgr_adapter_repeat_private_run(int device, const unsigned char* seqs, const long long* seq_off, const int* seq_len,
+                                         int n_windows, const int* q_begin, const int* q_k, const int* q_mm, int n_threads,
+                                         unsigned char* answers, int* status) {
+  if (n_threads <= 0 || n_windows < 0) return -1;
+  std::vector<lgr_rep_ctx*> ctx((size_t)n_threads, nullptr);
+  bool ok = true;
+  for (auto& c : ctx) ok = ok && lgr_repeat_create(device, &c) == LGR_OK;
+  long long wall = -1;
+  if (ok) {
+    const RepeatWindows win{seqs, seq_off, seq_len, n_windows, q_begin, q_k, q_mm};
+    wall = (long long)RunWindows(
+        win, n_threads, false, answers, status,
+        [&](int w, int t) {
+          const int n = win.q_begin[w + 1] - win.q_begin[w];
+          std::vector<lgr_repeat_job> jobs((size_t)n);
+          for (int i = 0; i < n; ++i) jobs[(size_t)i] = lgr_repeat_job{0, win.seq_len[w], win.q_k[win.q_begin[w] + i], win.q_mm[win.q_begin[w] + i], 0};
+          std::vector<std::uint8_t> a((size_t)n);
+          const int rc = lgr_repeat_scan(ctx[(size_t)t], seqs + win.seq_off[w], win.seq_len[w], jobs.data(), n, a.data(), nullptr);
+          if (rc != LGR_OK && rc != LGR_E_PARTIAL) throw std::runtime_error(lgr_repeat_last_error(ctx[(size_t)t]));
+          return a;
+        },
+        [](const std::atomic<int>&) {});
+  }
+  for (auto* c : ctx) lgr_repeat_destroy(c);
+  return wall;
 }
 
 }  // extern "C"

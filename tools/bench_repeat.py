@@ -26,10 +26,11 @@ def main():
     ap.add_argument("--steps", type=int, default=5)
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--cpu-jobs", type=int, default=60)
+    ap.add_argument("--library", default=None, help="a stand-alone build of lgr_repeat.cu instead of the main library (A/B runs)")
     args = ap.parse_args()
     kvals = tuple(range(13, 128, 6))          # Lancet2 defaults: min_k 13, max_k 127, step 6
     jobs = repeat_lib.window_jobs(20261017, args.windows, k_values=kvals, lengths=(1000,))
-    scan = GpuRepeatScan()
+    scan = GpuRepeatScan(library=args.library)
     for _ in range(args.warmup):
         got, _ = scan.scan(jobs)
     t0 = time.perf_counter()
@@ -51,7 +52,7 @@ def main():
     assert [int(got[i]) for i in idx] == cpu, "GPU and CPU answers differ"
     print(json.dumps({
         "metric": "repeat_jobs_per_sec", "unit": "jobs/s", "jobs": len(jobs), "windows": args.windows,
-        "k_values": list(kvals), "window_len": "1000-1049", "repeat_fraction": round(float((got == 1).mean()), 4),
+        "library": args.library or "main", "k_values": list(kvals), "window_len": "1000-1049", "repeat_fraction": round(float((got == 1).mean()), 4),
         "e2e": {"value": len(jobs) / wall, "ms_per_call": wall * 1e3, "note": "lgr_repeat_scan with host buffers"},
         "kernel": {"value": len(jobs) / (kms * 1e-3), "ms": kms, "kmer_pairs_upper_bound_per_s": pairs / (kms * 1e-3)},
         "cpu_baseline": {"value": len(idx) / cpu_s, "unit": "jobs/s", "cores": 1, "kind": kind,
