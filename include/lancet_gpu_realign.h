@@ -191,7 +191,7 @@ typedef struct lgr_stats {
   float ms_h2d, ms_kernels, ms_d2h; /* CUDA-event times on the ctx stream */
   float ms_k_index;                 /* encode + haplotype sketch/sort/mid_occ, with the read sketch beside it on the second stream */
   float ms_k_sketch;                /* k_read_filter (mm_seed_mz_flt), after the two streams join */
-  float ms_k_map;                   /* k_chain_warp alone (the dominant kernel) */
+  float ms_k_map;                   /* the chain kernels (k_chain_lean + k_chain_cold) */
   float ms_k_ext;                   /* k_chain_overflow + k_ext_warp + k_finish_warp */
   float ms_k_assign;                /* k_assign */
   int64_t n_pairs, n_aligned;

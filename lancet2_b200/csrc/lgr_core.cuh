@@ -559,10 +559,11 @@ enum WsArray {
   A_COUNT
 };
 
-// COMPACT: the layout of the hot chain kernel at 128 anchors (reads beyond 160 bp), which never sorts (the sorted arrays ARE the anchor arrays), never
-// needs the seed arrays once the anchors exist (they share the slots of the chaining arrays, which are written
-// later) and never touches A_Z / A_PERM: 8 anchor-sized arrays instead of 15, so that more CTAs fit an SM.
-template <int S, bool COMPACT = false>
+// LEAN: the layout of the lean chain kernel, which finishes only sorted co-linear pairs.  It never sorts (the
+// sorted arrays ARE the anchor arrays), never needs the seed arrays once the anchors exist (they share the
+// slots of f / p, which are written later), never runs the general chain DP or tail (no t, v, z, perm,
+// compacted anchors) and holds one reg: 5 anchor-sized arrays instead of 15, so that more CTAs fit an SM.
+template <int S, bool LEAN = false>
 struct Ws {
   int32_t* base;  // already offset to this lane
   // capacities, packed (keeps the struct at two words: a third member made nvcc lose track of
@@ -571,19 +572,15 @@ struct Ws {
   // chain/reg-sized arrays (R_*; 0 = same as the anchor arrays).  A pair with more chains
   // than that overflows.
   int caps;
-  static constexpr int kSlots = COMPACT ? 8 : (int)R_SCORE;
+  static constexpr int kSlots = LEAN ? 5 : (int)R_SCORE;
   static LGR_HD constexpr int slot(int k) {
-    if (!COMPACT) return k;
+    if (!LEAN) return k;
     switch (k) {
       case A_AX: case A_SX: return 0;
       case A_AY: case A_SY: return 1;
       case A_F: case A_SEEDQ: return 2;
       case A_P: case A_SEEDN: return 3;
-      case A_T: case A_SEEDS: return 4;
-      case A_V: return 5;
-      case A_CX: return 6;
-      case A_CY: return 7;
-      default: return 5;  // A_Z, A_PERM: not used with this layout
+      default: return 4;  // A_SEEDS; the arrays of the general DP and tail are not used with this layout
     }
   }
   LGR_HD int cap() const { return caps & 0xffff; }

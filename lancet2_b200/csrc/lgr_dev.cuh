@@ -15,7 +15,8 @@ __constant__ double c_phred_err[256] = {
 enum Ctr {
   C_ITEM = 0, C_NTASK, C_NTASK1, C_NTASK2, C_NTASK3, C_NTASK4, C_REGS, C_EXTARENA, C_CIGARENA, C_NOVF, C_ERR, C_EVALS, C_ANCH, C_CELLS, C_CELLSFULL,
   C_ALIGNED, C_TASKPOS, C_TASKPOS1, C_TASKPOS2, C_TASKPOS3, C_TASKPOS4, C_FINPOS, C_OVFPOS, C_OVFNEED, C_NCOLD, C_COLDPOS,
-  C_COLD_HIGH, C_COLD_SORT, C_COLD_TAIL, C_COLD_LONG,  // why pairs went to the cold kernel (diagnostics)
+  C_COLD_HIGH, C_COLD_SORT, C_COLD_LONG,  // why pairs went to the cold kernel (diagnostics)
+  C_LEAN_DEFER,                           // pairs the lean chain kernel queued for the cold kernel (every shape but sorted co-linear)
   C_COUNT
 };
 enum ErrBits { E_REG_ARENA = 1, E_EXT_ARENA = 2, E_CIG_ARENA = 4, E_ANCHOR_CAP = 8, E_CIG_SCRATCH = 16, E_MZ_CAP = 32 };
@@ -95,7 +96,7 @@ struct Dev {      // everything the kernels need, passed by value
   TaskRec* tasks; int64_t tasks_cap;   // [kExtClasses][tasks_cap]
   uint32_t* ext_arena; int64_t ext_arena_cap;
   int32_t* ovf_read; int32_t* ovf_hap; int64_t ovf_cap;
-  int32_t* cold_read; int32_t* cold_hap;   // [n_pairs] pairs the hot chain kernel left to k_chain_cold
+  int32_t* cold_read; int32_t* cold_hap;   // [n_pairs] pairs the lean chain kernel left to k_chain_cold
   // k_ext_big scratch
   uint8_t* dir_scratch; int64_t dir_per_warp;
   int32_t* bnd_scratch; int64_t bnd_per_warp;   // Hb/Fb boundary rows

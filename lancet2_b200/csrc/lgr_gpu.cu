@@ -11,9 +11,11 @@
 //     k_group_mid         effective mid_occ per group
 //     k_read_sketch       one lane per read: sketch (second stream); k_read_filter: mm_seed_mz_flt
 //   lgr_kernels_chain.cuh
-//     k_chain_warp        ONE WARP PER (read, haplotype) PAIR: seeds → anchors → sort → chain DP →
-//                         backtrack → regs → SR stretch; closed-form extensions; regs parked in HBM
-//                         (RegRec), the other extensions queued (TaskRec)
+//     k_chain_lean        ONE WARP PER (read, haplotype) PAIR: seeds → anchors → co-linear chain in
+//                         closed form → reg; closed-form extensions; regs parked in HBM (RegRec), the
+//                         other extensions queued (TaskRec); every other shape queued for k_chain_cold
+//     k_chain_cold        the same, one warp per queued pair, with sort, chain DP, backtrack, several
+//                         regs and SR stretch
 //     k_chain_overflow    the same for pairs whose anchors exceed the shared-memory cap (lane per pair)
 //   lgr_kernels_ext.cuh
 //     k_ext_warp          one warp per queued extension: anti-diagonal wavefront DP with shuffle
@@ -433,15 +435,15 @@ static int plan_batch(lgr_ctx* c, const BatchSizes& z) {
     int per_sm = 0, per_sm_cold = 0;
     cudaError_t e1, e2, e3, e4;
     if (c->warp_cap == 64) {
-      e1 = cudaFuncSetAttribute(k_chain_warp<64>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)c->warp_smem);
-      cudaFuncSetAttribute(k_chain_warp<64>, cudaFuncAttributePreferredSharedMemoryCarveout, LGR_CHAIN_CARVEOUT);
-      e2 = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_chain_warp<64>, kWarpsPerCta * 32, c->warp_smem);
+      e1 = cudaFuncSetAttribute(k_chain_lean<64>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)c->warp_smem);
+      cudaFuncSetAttribute(k_chain_lean<64>, cudaFuncAttributePreferredSharedMemoryCarveout, LGR_CHAIN_CARVEOUT);
+      e2 = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_chain_lean<64>, kWarpsPerCta * 32, c->warp_smem);
       e3 = cudaFuncSetAttribute(k_chain_cold<64>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)c->cold_smem);
       e4 = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm_cold, k_chain_cold<64>, kWarpsPerCta * 32, c->cold_smem);
     } else {
-      e1 = cudaFuncSetAttribute(k_chain_warp<128>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)c->warp_smem);
-      cudaFuncSetAttribute(k_chain_warp<128>, cudaFuncAttributePreferredSharedMemoryCarveout, LGR_CHAIN_CARVEOUT);
-      e2 = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_chain_warp<128>, kWarpsPerCta * 32, c->warp_smem);
+      e1 = cudaFuncSetAttribute(k_chain_lean<128>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)c->warp_smem);
+      cudaFuncSetAttribute(k_chain_lean<128>, cudaFuncAttributePreferredSharedMemoryCarveout, LGR_CHAIN_CARVEOUT);
+      e2 = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_chain_lean<128>, kWarpsPerCta * 32, c->warp_smem);
       e3 = cudaFuncSetAttribute(k_chain_cold<128>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)c->cold_smem);
       e4 = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm_cold, k_chain_cold<128>, kWarpsPerCta * 32, c->cold_smem);
     }
@@ -464,7 +466,7 @@ static int plan_batch(lgr_ctx* c, const BatchSizes& z) {
   c->fin_blocks = (int)std::max<int64_t>(1, std::min<int64_t>(c->fin_blocks_full, (n_pairs + 4 * kFinChunk - 1) / (4 * kFinChunk)));
   // per-warp scratch follows the grid that indexes it: extension / finish kernels vs the chain kernels
   const int64_t ext_warps = (int64_t)std::max(c->ext_blocks, c->fin_blocks) * 4;
-  const int64_t chain_warps = (int64_t)std::max(c->warp_blocks, c->cold_blocks) * kWarpsPerCta;
+  const int64_t chain_warps = (int64_t)c->cold_blocks * kWarpsPerCta;  // the cold kernel's radix scratch
   const int64_t dir_per_warp = (int64_t)((Lm + 31) / 32) * (Tmax + 32) * 32;
   const int64_t bnd_per_warp = 2 * (int64_t)(Tmax + 32);
   const int wcig_cap = 2 * Lm + 8;
@@ -698,10 +700,10 @@ static int run_launch(lgr_ctx* c) {
     launches += 1;
     cudaEventRecord(c->ev[2], s);
     if (c->warp_cap == 64) {
-      k_chain_warp<64><<<c->warp_blocks, kWarpsPerCta * 32, c->warp_smem, s>>>(D);
+      k_chain_lean<64><<<c->warp_blocks, kWarpsPerCta * 32, c->warp_smem, s>>>(D);
       k_chain_cold<64><<<c->cold_blocks, kWarpsPerCta * 32, c->cold_smem, s>>>(D);
     } else {
-      k_chain_warp<128><<<c->warp_blocks, kWarpsPerCta * 32, c->warp_smem, s>>>(D);
+      k_chain_lean<128><<<c->warp_blocks, kWarpsPerCta * 32, c->warp_smem, s>>>(D);
       k_chain_cold<128><<<c->cold_blocks, kWarpsPerCta * 32, c->cold_smem, s>>>(D);
     }
     launches += 2;
@@ -723,7 +725,7 @@ static int run_launch(lgr_ctx* c) {
 }
 
 // Overflow pass, host driven, after the main pass has drained: the pairs whose seeds / anchors /
-// chains did not fit the shared-memory workspace of k_chain_warp (reads inside tandem repeats) were
+// chains did not fit the shared-memory workspace of the chain kernels (reads inside tandem repeats) were
 // listed, not refused.  Now their number and the largest anchor count among them are known, so the
 // HBM workspace is allocated to measure (nothing is reserved up front), k_chain_overflow maps them,
 // and extension / finish / assignment run again over what they added.  Rare: the price is one extra

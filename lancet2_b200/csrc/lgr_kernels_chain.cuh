@@ -1,4 +1,4 @@
-// lgr_kernels_chain.cuh — seeding + chaining: k_chain_overflow, warp_seed_chain, chain tails, closed-form extensions, k_chain_warp
+// lgr_kernels_chain.cuh — seeding + chaining: k_chain_overflow, warp_seed_chain, chain tails, closed-form extensions, k_chain_lean, k_chain_cold
 // Part of the single translation unit lgr_gpu.cu (included there, in order); see that file's header.
 #ifndef LANCET2_B200_LGR_KERNELS_CHAIN_CUH_
 #define LANCET2_B200_LGR_KERNELS_CHAIN_CUH_
@@ -7,9 +7,9 @@ namespace {
 
 // ---------------------------------------------------------------------------------------
 // k_chain_overflow: phase A for the pairs whose seeds/anchors exceeded the shared-memory cap of
-// k_chain_warp (tandem repeats: hundreds to thousands of anchors).  One LANE per pair running the
+// the chain kernels (tandem repeats: hundreds to thousands of anchors).  One LANE per pair running the
 // scalar core (map_chain_phase) over a 16384-anchor HBM workspace interleaved per warp; regs are
-// parked exactly like k_chain_warp does.  Exits immediately when the overflow list is empty.
+// parked exactly like the chain kernels do.  Exits immediately when the overflow list is empty.
 // ---------------------------------------------------------------------------------------
 __global__ void __launch_bounds__(128) k_chain_overflow(const __grid_constant__ Dev D) {
   const int lane = threadIdx.x & 31;
@@ -105,25 +105,26 @@ __global__ void __launch_bounds__(128) k_chain_overflow(const __grid_constant__ 
 #ifndef LGR_CHAIN_LOCKSTEP
 #define LGR_CHAIN_LOCKSTEP 0
 #endif
-#ifndef LGR_HOT_WARP_SORT
-#define LGR_HOT_WARP_SORT 0  // 1: the hot kernel ranks unsorted anchor lists itself instead of queueing the pair for the cold kernel
-#endif
 #ifndef LGR_WARPS_PER_CTA
 #define LGR_WARPS_PER_CTA 4
 #endif
 constexpr int kWarpsPerCta = LGR_WARPS_PER_CTA;
 constexpr int kMapOkColinear = 2;  // warp_seed_chain: chain DP done by the co-linear closed form
-constexpr int kMapCold = -3;       // hot kernel only: a shape whose code lives in the cold kernel (queued, not computed)
+constexpr int kMapCold = -3;       // lean tier only: a shape whose code lives in the cold kernel (queued, not computed)
 
-// HOT: the instantiation inside k_chain_warp's hot kernel.  The rare shapes — a seed above mid_occ
-// (mm_seed_select), anchors that need upstream's radix pass emulated, a chain tail the fast form does
-// not cover — return kMapCold instead of running here, so their (large, lane-0) code is not part of
-// the hot kernel's instruction footprint; the cold kernel is the same source with HOT = false.
+// Which chain kernel a pair runs in.  Lean: k_chain_lean, which every pair enters.  It finishes the
+// sorted co-linear pairs (93 % on cfg2) and returns kMapCold for every other shape — a seed above
+// mid_occ (mm_seed_select), unsorted anchors, a chain the closed form does not cover — so that the
+// general chain DP, the general tail and the multi-reg export are not part of its instruction
+// footprint, registers or workspace.  Cold: k_chain_cold, the complete code, tables read from HBM.
+enum class Tier { Lean, Cold };
+
 // The pair's anchor / evaluation counts are returned to the caller, who commits them only for pairs
-// that finish here (a deferred pair is counted where it is computed).
-template <int CAP, bool HOT>
-__device__ __forceinline__ int warp_seed_chain(const Dev& D, const PairIn& in, const uint16_t* bkt, const Ws<1, (HOT && CAP > 64)>& ws,
+// that finish in this tier (a deferred pair is counted where it is computed).
+template <int CAP, Tier T>
+__device__ __forceinline__ int warp_seed_chain(const Dev& D, const PairIn& in, const uint16_t* bkt, const Ws<1, T == Tier::Lean>& ws,
                                                RadixScratch* rsx, long long* n_eval_out, int* n_a_out, int* need_out) {
+  constexpr bool LEAN = T == Tier::Lean;
   const unsigned full = 0xffffffffu;
   const int lane = threadIdx.x & 31;
   const DevParams& P = D.P;
@@ -175,7 +176,7 @@ __device__ __forceinline__ int warp_seed_chain(const Dev& D, const PairIn& in, c
   if (n_m > CAP) return kMapOverflow;
   __syncwarp();
   if (n_high > 0) {
-    if (HOT) {
+    if (LEAN) {
       if (lane == 0) atomicAdd((unsigned long long*)&D.ctr[C_COLD_HIGH], 1ULL);
       return kMapCold;
     }
@@ -236,9 +237,9 @@ __device__ __forceinline__ int warp_seed_chain(const Dev& D, const PairIn& in, c
     const bool sorted = __all_sync(full, ok);
     const bool strictly = __all_sync(full, strict);
     if (sorted && (n_a <= 64 || strictly)) {
-      if constexpr (!(HOT && CAP > 64))  // the compact hot layout has no separate sorted arrays: sx/sy are ax/ay
+      if constexpr (!LEAN)  // the lean layout has no separate sorted arrays: sx/sy are ax/ay
         for (int i = lane; i < n_a; i += 32) sx[i] = ax[i], sy[i] = ay[i];
-    } else if (HOT && !(LGR_HOT_WARP_SORT && n_a <= 64)) {
+    } else if (LEAN) {
       if (lane == 0) atomicAdd((unsigned long long*)&D.ctr[C_COLD_SORT], 1ULL);
       return kMapCold;
     } else {
@@ -248,8 +249,8 @@ __device__ __forceinline__ int warp_seed_chain(const Dev& D, const PairIn& in, c
       // upstream runs its unstable in-place radix passes: if all keys are distinct there is still only
       // one sorted order and ranking gives it; only a list with tied keys needs the move-for-move
       // emulation on lane 0.  Warp-uniform trip counts on purpose: a lane-dependent loop here cost the
-      // whole kernel its convergence (measured: +0.8 ms on cfg2 when this ran in the hot kernel), so
-      // these pairs stay with the cold kernel.
+      // whole kernel its convergence (measured: +0.8 ms on cfg2 when this ran in the former hot kernel),
+      // so these pairs stay with the cold kernel.
       bool tie = false;
       for (int base = 0; base < n_a; base += 32) {
         const int i = base + lane;
@@ -273,7 +274,6 @@ __device__ __forceinline__ int warp_seed_chain(const Dev& D, const PairIn& in, c
       }
     }
   }
-  for (int i = lane; i < n_a; i += 32) t[i] = 0;
   __syncwarp();
   // ---- mg_lchain_dp ----
   int32_t max_dist_x = P.max_gap_ref > 0 ? P.max_gap_ref : P.max_gap;
@@ -325,126 +325,132 @@ __device__ __forceinline__ int warp_seed_chain(const Dev& D, const PairIn& in, c
       return kMapOkColinear;
     }
   }
-  for (int i = 0; i < n_a; ++i) {
-    const uint32_t xi = (uint32_t)sx[i], yi = (uint32_t)sy[i];
-    while (st < i && ((xi >> 31) != ((uint32_t)sx[st] >> 31) || anchor_rpos(xi) > anchor_rpos((uint32_t)sx[st]) + max_dist_x)) ++st;
-    if (i - st > P.max_iter) st = i - P.max_iter;
-    int32_t max_f = anchor_span(yi);
-    int max_j = -1, n_skip = 0, end_j = st - 1;
-    for (int jb = i - 1; jb >= st; jb -= 32) {
-      const int j = jb - lane;
-      int32_t sc = INT32_MIN;
-      int pj = -1;
-      if (j >= st) {
-        sc = comput_sc(xi, yi, (uint32_t)sx[j], (uint32_t)sy[j], max_dist_x, max_dist_y, P.bw, P.pen_gap, P.pen_skip);
-        if (sc != INT32_MIN) sc += f[j], pj = p[j];
-      }
-      const bool valid = sc != INT32_MIN;
-      // stamps t[p[j]] = i of this chunk: predecessors processed earlier (higher j, lower lane) are
-      // visible to later lanes after the barrier; stamps written by lanes at/after a break only
-      // touch entries that are never read again for this i.
-      if (valid && pj >= 0) t[pj] = i;
-      __syncwarp();
-      const bool stamped = valid && t[j] == i;
-      // record setters of the sequential "sc > max_f" test: lanes whose score exceeds max_f and
-      // every earlier lane of the chunk.  Usually there is at most one, so they are peeled off
-      // with ballots instead of a prefix-max scan.
-      unsigned nmask_all = 0;
-      {
-        int32_t cur = max_f;
-        unsigned cand = __ballot_sync(full, valid && sc > cur);
-        while (cand) {
-          const int l = __ffs(cand) - 1;
-          nmask_all |= 1u << l;
-          cur = __shfl_sync(full, sc, l);
-          cand = __ballot_sync(full, valid && sc > cur) & ~((2u << l) - 1);
+  if constexpr (LEAN) {
+    return kMapCold;  // the general DP below is not part of the lean kernel
+  } else {
+    for (int i = lane; i < n_a; i += 32) t[i] = 0;
+    __syncwarp();
+    for (int i = 0; i < n_a; ++i) {
+      const uint32_t xi = (uint32_t)sx[i], yi = (uint32_t)sy[i];
+      while (st < i && ((xi >> 31) != ((uint32_t)sx[st] >> 31) || anchor_rpos(xi) > anchor_rpos((uint32_t)sx[st]) + max_dist_x)) ++st;
+      if (i - st > P.max_iter) st = i - P.max_iter;
+      int32_t max_f = anchor_span(yi);
+      int max_j = -1, n_skip = 0, end_j = st - 1;
+      for (int jb = i - 1; jb >= st; jb -= 32) {
+        const int j = jb - lane;
+        int32_t sc = INT32_MIN;
+        int pj = -1;
+        if (j >= st) {
+          sc = comput_sc(xi, yi, (uint32_t)sx[j], (uint32_t)sy[j], max_dist_x, max_dist_y, P.bw, P.pen_gap, P.pen_skip);
+          if (sc != INT32_MIN) sc += f[j], pj = p[j];
         }
-      }
-      const bool newmax = (nmask_all >> lane) & 1;
-      const int ev = newmax ? -1 : (stamped ? 1 : 0);
-      const unsigned smask = __ballot_sync(full, ev == 1);
-      int last = 31;
-      unsigned brk = 0;
-      // the skip counter only ever decrements on a record setter; when every record setter comes
-      // before the first stamped lane and the counter enters at 0 (or there is none), the
-      // decrements are no-ops and the counter is a running popcount of the stamped lanes
-      const bool simple = nmask_all == 0 || (n_skip == 0 && (smask == 0 || (31 - __clz(nmask_all)) < (__ffs(smask) - 1)));
-      if (simple) {
-        const int need = P.max_skip + 1 - n_skip;  // stamped lanes until the break
-        const int tot = __popc(smask);
-        if (need <= tot) {
-          last = (int)__fns(smask, 0, need);
-          brk = 1u << last;
-          n_skip = P.max_skip + 1;
-        } else {
-          n_skip += tot;
-        }
-      } else {
-        // general case: n -> max(n + a, b) per lane, composed left to right ((max,+) scan)
-        int a = ev, b = ev == 1 ? 1 : 0;
-        for (int o = 1; o < 32; o <<= 1) {
-          const int au = __shfl_up_sync(full, a, o), bu = __shfl_up_sync(full, b, o);
-          if (lane >= o) {
-            const int nb = bu + a;
-            b = nb > b ? nb : b;
-            a = au + a;
+        const bool valid = sc != INT32_MIN;
+        // stamps t[p[j]] = i of this chunk: predecessors processed earlier (higher j, lower lane) are
+        // visible to later lanes after the barrier; stamps written by lanes at/after a break only
+        // touch entries that are never read again for this i.
+        if (valid && pj >= 0) t[pj] = i;
+        __syncwarp();
+        const bool stamped = valid && t[j] == i;
+        // record setters of the sequential "sc > max_f" test: lanes whose score exceeds max_f and
+        // every earlier lane of the chunk.  Usually there is at most one, so they are peeled off
+        // with ballots instead of a prefix-max scan.
+        unsigned nmask_all = 0;
+        {
+          int32_t cur = max_f;
+          unsigned cand = __ballot_sync(full, valid && sc > cur);
+          while (cand) {
+            const int l = __ffs(cand) - 1;
+            nmask_all |= 1u << l;
+            cur = __shfl_sync(full, sc, l);
+            cand = __ballot_sync(full, valid && sc > cur) & ~((2u << l) - 1);
           }
         }
-        int n_after = n_skip + a;
-        if (b > n_after) n_after = b;
-        brk = __ballot_sync(full, ev == 1 && n_after > P.max_skip);
-        last = brk ? __ffs(brk) - 1 : 31;
-        n_skip = __shfl_sync(full, n_after, last);
+        const bool newmax = (nmask_all >> lane) & 1;
+        const int ev = newmax ? -1 : (stamped ? 1 : 0);
+        const unsigned smask = __ballot_sync(full, ev == 1);
+        int last = 31;
+        unsigned brk = 0;
+        // the skip counter only ever decrements on a record setter; when every record setter comes
+        // before the first stamped lane and the counter enters at 0 (or there is none), the
+        // decrements are no-ops and the counter is a running popcount of the stamped lanes
+        const bool simple = nmask_all == 0 || (n_skip == 0 && (smask == 0 || (31 - __clz(nmask_all)) < (__ffs(smask) - 1)));
+        if (simple) {
+          const int need = P.max_skip + 1 - n_skip;  // stamped lanes until the break
+          const int tot = __popc(smask);
+          if (need <= tot) {
+            last = (int)__fns(smask, 0, need);
+            brk = 1u << last;
+            n_skip = P.max_skip + 1;
+          } else {
+            n_skip += tot;
+          }
+        } else {
+          // general case: n -> max(n + a, b) per lane, composed left to right ((max,+) scan)
+          int a = ev, b = ev == 1 ? 1 : 0;
+          for (int o = 1; o < 32; o <<= 1) {
+            const int au = __shfl_up_sync(full, a, o), bu = __shfl_up_sync(full, b, o);
+            if (lane >= o) {
+              const int nb = bu + a;
+              b = nb > b ? nb : b;
+              a = au + a;
+            }
+          }
+          int n_after = n_skip + a;
+          if (b > n_after) n_after = b;
+          brk = __ballot_sync(full, ev == 1 && n_after > P.max_skip);
+          last = brk ? __ffs(brk) - 1 : 31;
+          n_skip = __shfl_sync(full, n_after, last);
+        }
+        const unsigned nmask = nmask_all & (last == 31 ? 0xffffffffu : ((2u << last) - 1));
+        if (nmask) {
+          const int src = 31 - __clz(nmask);
+          max_f = __shfl_sync(full, sc, src);
+          max_j = jb - src;
+        }
+        const int n_in = jb - st + 1 < 32 ? jb - st + 1 : 32;
+        if (brk) {
+          n_iter += last + 1;
+          end_j = jb - last;
+          break;
+        }
+        n_iter += n_in;
+        __syncwarp();
       }
-      const unsigned nmask = nmask_all & (last == 31 ? 0xffffffffu : ((2u << last) - 1));
-      if (nmask) {
-        const int src = 31 - __clz(nmask);
-        max_f = __shfl_sync(full, sc, src);
-        max_j = jb - src;
+      bool far = true;
+      if (max_ii >= 0) {
+        const uint32_t xm = (uint32_t)sx[max_ii];
+        far = (xi >> 31) != (xm >> 31) || anchor_rpos(xi) - anchor_rpos(xm) > max_dist_x;
       }
-      const int n_in = jb - st + 1 < 32 ? jb - st + 1 : 32;
-      if (brk) {
-        n_iter += last + 1;
-        end_j = jb - last;
-        break;
+      if (max_ii < 0 || far) {
+        int32_t bf = INT32_MIN;
+        int bj = -1;
+        for (int j = i - 1 - lane; j >= st; j -= 32)
+          if (f[j] > bf) bf = f[j], bj = j;
+        for (int o = 16; o > 0; o >>= 1) {
+          const int32_t of = __shfl_xor_sync(full, bf, o);
+          const int oj = __shfl_xor_sync(full, bj, o);
+          if (of > bf || (of == bf && oj > bj)) bf = of, bj = oj;
+        }
+        max_ii = bj;
       }
-      n_iter += n_in;
+      if (max_ii >= 0 && max_ii < end_j) {
+        const int32_t tmp = comput_sc(xi, yi, (uint32_t)sx[max_ii], (uint32_t)sy[max_ii], max_dist_x, max_dist_y, P.bw, P.pen_gap, P.pen_skip);
+        if (tmp != INT32_MIN && max_f < tmp + f[max_ii]) max_f = tmp + f[max_ii], max_j = max_ii;
+      }
+      __syncwarp();
+      if (lane == 0) f[i] = max_f, p[i] = max_j;
+      if (max_ii < 0) {
+        max_ii = i;
+      } else {
+        const uint32_t xm = (uint32_t)sx[max_ii];
+        const bool near = (xi >> 31) == (xm >> 31) && anchor_rpos(xi) - anchor_rpos(xm) <= max_dist_x;
+        if (near && f[max_ii] < max_f) max_ii = i;
+      }
       __syncwarp();
     }
-    bool far = true;
-    if (max_ii >= 0) {
-      const uint32_t xm = (uint32_t)sx[max_ii];
-      far = (xi >> 31) != (xm >> 31) || anchor_rpos(xi) - anchor_rpos(xm) > max_dist_x;
-    }
-    if (max_ii < 0 || far) {
-      int32_t bf = INT32_MIN;
-      int bj = -1;
-      for (int j = i - 1 - lane; j >= st; j -= 32)
-        if (f[j] > bf) bf = f[j], bj = j;
-      for (int o = 16; o > 0; o >>= 1) {
-        const int32_t of = __shfl_xor_sync(full, bf, o);
-        const int oj = __shfl_xor_sync(full, bj, o);
-        if (of > bf || (of == bf && oj > bj)) bf = of, bj = oj;
-      }
-      max_ii = bj;
-    }
-    if (max_ii >= 0 && max_ii < end_j) {
-      const int32_t tmp = comput_sc(xi, yi, (uint32_t)sx[max_ii], (uint32_t)sy[max_ii], max_dist_x, max_dist_y, P.bw, P.pen_gap, P.pen_skip);
-      if (tmp != INT32_MIN && max_f < tmp + f[max_ii]) max_f = tmp + f[max_ii], max_j = max_ii;
-    }
-    __syncwarp();
-    if (lane == 0) f[i] = max_f, p[i] = max_j;
-    if (max_ii < 0) {
-      max_ii = i;
-    } else {
-      const uint32_t xm = (uint32_t)sx[max_ii];
-      const bool near = (xi >> 31) == (xm >> 31) && anchor_rpos(xi) - anchor_rpos(xm) <= max_dist_x;
-      if (near && f[max_ii] < max_f) max_ii = i;
-    }
-    __syncwarp();
+    *n_eval_out = n_iter;
+    return kMapOk;
   }
-  *n_eval_out = n_iter;
-  return kMapOk;
 }
 
 // ---------------------------------------------------------------------------------------
@@ -676,11 +682,12 @@ __device__ __forceinline__ void cold_push(const Dev& D, int r, int h) {
 
 // One (read, haplotype) pair on one warp: seeds → anchors → chain DP → regs, closed-form extensions,
 // the other extensions queued, regs parked for k_finish_warp.  `tab` / `bkt` are the haplotype's
-// sorted minimizer table and bucket directory (shared memory in the hot kernel, HBM in the cold one).
-template <int CAP, bool HOT>
+// sorted minimizer table and bucket directory (shared memory in the lean kernel, HBM in the cold one).
+template <int CAP, Tier T>
 __device__ __forceinline__ void chain_pair(const Dev& D, int r, int h, int g, int h_local, int mid_occ, const uint8_t* hapc, int hlen,
-                                           const uint64_t* tab, int idx_n, const uint16_t* bkt, const Ws<1, (HOT && CAP > 64)>& ws, RadixScratch* rsx,
+                                           const uint64_t* tab, int idx_n, const uint16_t* bkt, const Ws<1, T == Tier::Lean>& ws, RadixScratch* rsx,
                                            RegRec* s_reg, ChainCounters& ctr) {
+  constexpr bool LEAN = T == Tier::Lean;
   const unsigned full = 0xffffffffu;
   const int lane = threadIdx.x & 31;
   const int64_t pair = D.pair_off[r] + h_local;
@@ -690,18 +697,15 @@ __device__ __forceinline__ void chain_pair(const Dev& D, int r, int h, int g, in
   PairIn pin{rv, hapc, hlen, tab, idx_n, D.mz_x + roff, D.mz_y + roff, D.mz_n[r], D.name_hash[r], mid_occ};
   int n_a = 0, n_regs = 0, need = 0;
   long long n_eval = 0;
-  int st = qlen > 0 ? warp_seed_chain<CAP, HOT>(D, pin, bkt, ws, rsx, &n_eval, &n_a, &need) : kMapNoHit;
+  int st = qlen > 0 ? warp_seed_chain<CAP, T>(D, pin, bkt, ws, rsx, &n_eval, &n_a, &need) : kMapNoHit;
   if (st == kMapOkColinear) {
     st = warp_chain_tail_colinear(D.P, qlen, hlen, pin.name_hash, ws, n_a);
     n_regs = 1;
-  } else if (st == kMapOk) {
-    st = warp_chain_tail_fast(D.P, qlen, hlen, pin.name_hash, ws, n_a);
-    n_regs = 1;
-    if (st == -2) {
-      if constexpr (HOT) {
-        st = kMapCold;
-        if (lane == 0) atomicAdd((unsigned long long*)&D.ctr[C_COLD_TAIL], 1ULL);
-      } else {
+  } else if constexpr (!LEAN) {
+    if (st == kMapOk) {
+      st = warp_chain_tail_fast(D.P, qlen, hlen, pin.name_hash, ws, n_a);
+      n_regs = 1;
+      if (st == -2) {
         __syncwarp();  // the lanes' reads of the workspace in the fast form are done before lane 0 rewrites it
         if (lane == 0) st = map_chain_tail<1>(D.P, qlen, hlen, pin.name_hash, ws, rsx, n_a, &n_regs);
         st = __shfl_sync(full, st, 0);
@@ -710,7 +714,10 @@ __device__ __forceinline__ void chain_pair(const Dev& D, int r, int h, int g, in
     }
   }
   if (st == kMapCold) {  // computed (and counted) by the cold kernel
-    if (lane == 0) cold_push(D, r, h);
+    if (lane == 0) {
+      atomicAdd((unsigned long long*)&D.ctr[C_LEAN_DEFER], 1ULL);
+      cold_push(D, r, h);
+    }
     __syncwarp();
     return;
   }
@@ -766,6 +773,7 @@ __device__ __forceinline__ void chain_pair(const Dev& D, int r, int h, int g, in
     __syncwarp();
     return;
   }
+  if constexpr (LEAN) return;  // the lean tier finishes single-reg pairs only
   long long first = -1;
   if (lane == 0) {
     first = atomicAdd((unsigned long long*)&D.ctr[C_REGS], (unsigned long long)n_regs);
@@ -795,35 +803,32 @@ __device__ __forceinline__ void chain_pair(const Dev& D, int r, int h, int g, in
   __syncwarp();
 }
 
-// shared memory of the chain kernels: per-warp workspace, per-warp RegRec slot, and (hot kernel) the
+// shared memory of the chain kernels: per-warp workspace, per-warp RegRec slot, and (lean kernel) the
 // staged minimizer table + bucket directory of the CTA's haplotype
-__host__ __device__ inline size_t chain_smem_bytes(int cap, bool hot) {
-  // the hot kernel takes the compact layout for 128 anchors (reads beyond 160 bp), where shared memory bounds its
-  // occupancy: +15 % there; at 64 anchors the full layout measured 1-3 % faster
-  return (size_t)kWarpsPerCta * ((hot && cap > 64 ? Ws<1, true>::elems(cap, kRegCap) : Ws<1>::elems(cap, kRegCap)) * sizeof(int32_t) + sizeof(RegRec)) +
-         (hot ? (size_t)kTabCap * sizeof(uint64_t) + (size_t)(kBuckets + 2) * sizeof(uint16_t) : 0) + 16;
+__host__ __device__ inline size_t chain_smem_bytes(int cap, bool lean) {
+  return (size_t)kWarpsPerCta * ((lean ? Ws<1, true>::elems(cap, 1) : Ws<1>::elems(cap, kRegCap)) * sizeof(int32_t) + sizeof(RegRec)) +
+         (lean ? (size_t)kTabCap * sizeof(uint64_t) + (size_t)(kBuckets + 2) * sizeof(uint16_t) : 0) + 16;
 }
 
-// Phase A, hot kernel.  A CTA takes a work item = (haplotype, up to item_reads consecutive reads of its
-// group), stages that haplotype's sorted minimizer table and 513-entry bucket directory in shared
-// memory (every seed lookup of every read of the item then stays on chip: the dependent
-// minimizer → bucket → table loads were the top stall of the round-1 kernel), and its warps take the
-// item's reads one at a time from a shared counter.  Rare shapes are queued for k_chain_cold.
+// Phase A, lean kernel: the first chain launch, which every pair enters.  A CTA takes a work item =
+// (haplotype, up to item_reads consecutive reads of its group), stages that haplotype's sorted minimizer
+// table and 513-entry bucket directory in shared memory (every seed lookup of every read of the item then
+// stays on chip: the dependent minimizer → bucket → table loads were the top stall of the round-1
+// kernel), and its warps take the item's reads one at a time from a shared counter.  Only sorted
+// co-linear pairs finish here; every other shape is queued for k_chain_cold (Tier::Lean).
 template <int CAP>
-__global__ void __launch_bounds__(kWarpsPerCta * 32, LGR_CHAIN_MINB) k_chain_warp(const __grid_constant__ Dev D) {
+__global__ void __launch_bounds__(kWarpsPerCta * 32, LGR_CHAIN_MINB) k_chain_lean(const __grid_constant__ Dev D) {
   extern __shared__ __align__(16) unsigned char smem_raw[];
   uint64_t* s_tab = reinterpret_cast<uint64_t*>(smem_raw);
   int32_t* s_ws = reinterpret_cast<int32_t*>(smem_raw + (size_t)kTabCap * sizeof(uint64_t));
-  using HotWs = Ws<1, (CAP > 64)>;
-  RegRec* s_regs = reinterpret_cast<RegRec*>(s_ws + (size_t)kWarpsPerCta * HotWs::elems(CAP, kRegCap));
+  using LeanWs = Ws<1, true>;
+  RegRec* s_regs = reinterpret_cast<RegRec*>(s_ws + (size_t)kWarpsPerCta * LeanWs::elems(CAP, 1));
   uint16_t* s_bkt = reinterpret_cast<uint16_t*>(s_regs + kWarpsPerCta);
   __shared__ long long s_item;
   __shared__ int s_next;
   const unsigned full = 0xffffffffu;
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-  const int gwarp = blockIdx.x * kWarpsPerCta + warp;
-  HotWs ws{s_ws + (size_t)warp * HotWs::elems(CAP, kRegCap), HotWs::pack(CAP, kRegCap)};
-  RadixScratch* rsx = D.rsx_scratch + gwarp;
+  LeanWs ws{s_ws + (size_t)warp * LeanWs::elems(CAP, 1), LeanWs::pack(CAP, 1)};
   ChainCounters ctr{0, 0, 0, 0};
   for (;;) {
     __syncthreads();  // every warp is done with the previous item's table
@@ -854,12 +859,12 @@ __global__ void __launch_bounds__(kWarpsPerCta * 32, LGR_CHAIN_MINB) k_chain_war
     }
     __syncthreads();
 #if LGR_CHAIN_LOCKSTEP
-    // the CTA's warps start every pair together: they then run the same stretch of this (large) kernel at about
-    // the same time and share its instruction-cache lines, at the price of waiting for the slowest pair of a round
+    // the CTA's warps start every pair together: they then run the same stretch of this kernel at about the
+    // same time and share its instruction-cache lines, at the price of waiting for the slowest pair of a round
     for (int base = 0; base < nr; base += kWarpsPerCta) {
       __syncthreads();
       const int rr = base + warp;
-      if (rr < nr) chain_pair<CAP, true>(D, r0 + rr, h, g, h_local, mid_occ, hapc, hlen, s_tab, idx_n, s_bkt, ws, rsx, &s_regs[warp], ctr);
+      if (rr < nr) chain_pair<CAP, Tier::Lean>(D, r0 + rr, h, g, h_local, mid_occ, hapc, hlen, s_tab, idx_n, s_bkt, ws, nullptr, &s_regs[warp], ctr);
     }
 #else
     for (;;) {
@@ -867,7 +872,7 @@ __global__ void __launch_bounds__(kWarpsPerCta * 32, LGR_CHAIN_MINB) k_chain_war
       if (lane == 0) rr = atomicAdd(&s_next, 1);
       rr = __shfl_sync(full, rr, 0);
       if (rr >= nr) break;
-      chain_pair<CAP, true>(D, r0 + rr, h, g, h_local, mid_occ, hapc, hlen, s_tab, idx_n, s_bkt, ws, rsx, &s_regs[warp], ctr);
+      chain_pair<CAP, Tier::Lean>(D, r0 + rr, h, g, h_local, mid_occ, hapc, hlen, s_tab, idx_n, s_bkt, ws, nullptr, &s_regs[warp], ctr);
     }
 #endif
   }
@@ -878,8 +883,9 @@ __global__ void __launch_bounds__(kWarpsPerCta * 32, LGR_CHAIN_MINB) k_chain_war
   }
 }
 
-// Phase A, cold kernel: the pairs the hot kernel queued, one warp per pair, the complete code
-// (mm_seed_select, the radix-pass emulation, the general chain tail), tables read from HBM.
+// Phase A, cold kernel: the pairs the lean kernel queued, one warp per pair, the complete code
+// (mm_seed_select, the radix-pass emulation, the general chain DP and tail, several regs per pair),
+// tables read from HBM (Tier::Cold).
 template <int CAP>
 __global__ void LGR_COLD_BOUNDS k_chain_cold(const __grid_constant__ Dev D) {
   extern __shared__ __align__(16) unsigned char smem_raw[];
@@ -901,7 +907,7 @@ __global__ void LGR_COLD_BOUNDS k_chain_cold(const __grid_constant__ Dev D) {
     const int r = D.cold_read[i], h = D.cold_hap[i];
     const int64_t hoff = D.hap_off[h];
     const int g = D.hap_grp[h];
-    chain_pair<CAP, false>(D, r, h, g, h - D.grp_hap_begin[g], D.grp_mid[g], D.hap_codes + hoff, (int)(D.hap_off[h + 1] - hoff),
+    chain_pair<CAP, Tier::Cold>(D, r, h, g, h - D.grp_hap_begin[g], D.grp_mid[g], D.hap_codes + hoff, (int)(D.hap_off[h + 1] - hoff),
                            D.idx + hoff, D.idx_n[h], D.bkt + (size_t)h * (kBuckets + 1), ws, rsx, &s_regs[warp], ctr);
   }
   if (lane == 0) {

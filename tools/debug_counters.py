@@ -14,7 +14,7 @@ from lancet2_b200.realign import GpuRealigner  # noqa: E402
 
 NAMES = ["ITEM", "NTASK0", "NTASK1", "NTASK2", "NTASK3", "NTASK4", "REGS", "EXTARENA", "CIGARENA", "NOVF", "ERR", "EVALS", "ANCH", "CELLS", "CELLSFULL",
          "ALIGNED", "TASKPOS0", "TASKPOS1", "TASKPOS2", "TASKPOS3", "TASKPOS4", "FINPOS", "OVFPOS", "OVFNEED", "NCOLD", "COLDPOS", "COLD_HIGH",
-         "COLD_SORT", "COLD_TAIL", "COLD_LONG"]
+         "COLD_SORT", "COLD_LONG", "LEAN_DEFER"]
 
 
 def main():
