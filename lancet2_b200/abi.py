@@ -428,7 +428,7 @@ _SYMBOLS = [
     "lgr_pair_offsets", "lgr_create", "lgr_destroy", "lgr_hap_mid_occ", "lgr_genotype_batch",
     "lgr_upload", "lgr_run_resident", "lgr_download", "lgr_stream", "lgr_submit", "lgr_wait",
     "lgr_alloc_pinned", "lgr_free_pinned",
-    "lgr_set_notify", "lgr_reserve", "lgr_arena_bytes", "lgr_check_limits", "lgr_packed_group_bytes", "lgr_pack_group", "lgr_genotype_packed", "lgr_submit_packed", "lgr_upload_packed",
+    "lgr_set_notify", "lgr_set_graph_mode", "lgr_graph_counters", "lgr_reserve", "lgr_arena_bytes", "lgr_check_limits", "lgr_packed_group_bytes", "lgr_pack_group", "lgr_genotype_packed", "lgr_submit_packed", "lgr_upload_packed",
     "lgr_format_create", "lgr_format_destroy", "lgr_format_last_error", "lgr_format_metrics",
     "lgr_format_from_assign", "lgr_resident_assign", "lgr_format_debug_evidence",
     "lgr_repeat_create", "lgr_repeat_destroy", "lgr_repeat_last_error", "lgr_repeat_scan", "lgr_repeat_reserve",
@@ -482,6 +482,10 @@ def load_library(path: Optional[str] = None) -> C.CDLL:
     lib.lgr_free_pinned.restype = None
     lib.lgr_set_notify.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p]
     lib.lgr_set_notify.restype = C.c_int
+    lib.lgr_set_graph_mode.argtypes = [C.c_void_p, C.c_int]
+    lib.lgr_set_graph_mode.restype = C.c_int
+    lib.lgr_graph_counters.argtypes = [C.c_void_p, C.POINTER(C.c_int64), C.POINTER(C.c_int64), C.POINTER(C.c_int64)]
+    lib.lgr_graph_counters.restype = C.c_int
     lib.lgr_reserve.argtypes = [C.c_void_p, C.c_int64, C.c_int]
     lib.lgr_reserve.restype = C.c_int
     lib.lgr_arena_bytes.argtypes = [C.c_void_p]

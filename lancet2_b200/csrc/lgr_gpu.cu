@@ -26,6 +26,7 @@
 //     k_assign            one lane per (read, variant): local scoring + best-allele selection
 //   lgr_dev.cuh           device descriptor, counters, records, launch-shape knobs
 //   lgr_core.cuh          __host__ __device__ per-lane core shared with tests/hostemu
+// Graph mode (lgr_set_graph_mode) captures the same launch list (enqueue_pass) as a CUDA graph and replays it.
 // There is no host fallback: every entry point fails with an error code when CUDA fails.
 #include <cuda_runtime.h>
 
@@ -58,6 +59,14 @@ struct DevBuf {   // a device buffer: either its own cudaMalloc block (arena, ov
   void* p = nullptr;
   size_t cap = 0;
   size_t off = 0;  // offset in the context's arena (views)
+};
+
+// graph mode (lgr_set_graph_mode): one executable per topology of the captured pass, least recently used evicted
+constexpr int kGraphCache = 8;
+struct GraphSlot {
+  cudaGraphExec_t exec = nullptr;
+  uint32_t key = 0;
+  uint64_t used = 0;
 };
 
 }  // namespace
@@ -93,6 +102,11 @@ struct lgr_ctx {
   cudaEvent_t ev[12];
   long long* h_ctr = nullptr;  // pinned copy of the device counters
   int launches = 0;
+  // graph mode of the blocking calls: the pass is captured and replayed as a CUDA graph (run_launch_graph)
+  bool graph_mode = false, capturing = false;
+  GraphSlot graphs[kGraphCache];
+  uint64_t graph_tick = 0;
+  int64_t graph_instantiated = 0, graph_updated = 0, graph_replayed = 0;
   // asynchronous submissions (lgr_submit/lgr_wait): child contexts, one per slot in flight
   lgr_ctx* slot[LGR_MAX_INFLIGHT] = {};
   bool slot_busy[LGR_MAX_INFLIGHT] = {};
@@ -261,6 +275,8 @@ void lgr_destroy(lgr_ctx* c) {
     ch = nullptr;
   }
   cudaSetDevice(c->device);
+  for (GraphSlot& g : c->graphs)
+    if (g.exec) cudaGraphExecDestroy(g.exec);
   if (c->h_ctr) cudaFreeHost(c->h_ctr);
   if (c->arena.p) cudaFree(c->arena.p);
   if (c->b_ws_big.p) cudaFree(c->b_ws_big.p);
@@ -656,16 +672,28 @@ static void launch_tail(lgr_ctx* c, const Dev& D, cudaStream_t s, int* launches)
   *launches += 2;
 }
 
-// enqueue one pass of the whole path on the context's streams; no host synchronisation
-static int run_launch(lgr_ctx* c) {
-  if (!c->resident) { c->err = "no batch uploaded"; return LGR_E_ARG; }
-  LGR_CUDA(c, cudaSetDevice(c->device));
+// which k_hap_sketch instance the parameters select: 0 / 1 = warp kernel on 32- / 64-bit keys, 2 = generic
+static int hap_sketch_variant(const DevParams& P) {
+  if (P.w == 5 && (P.k & 1)) return 2 * P.k + 8 <= 32 ? 0 : 1;
+  return 2;
+}
+
+// timing event i: an event-record node when the pass is being captured, so that the stage times of lgr_stats
+// stay meaningful in graph mode (a plain record inside a capture only orders the streams)
+static void mark(lgr_ctx* c, int i, cudaStream_t s) {
+  if (c->capturing) cudaEventRecordWithFlags(c->ev[i], s, cudaEventRecordExternal);
+  else cudaEventRecord(c->ev[i], s);
+}
+
+// enqueue one pass of the whole path on the context's streams; no host synchronisation.  Graph mode captures
+// exactly this code.
+static int enqueue_pass(lgr_ctx* c) {
   Dev& D = c->D;
   cudaStream_t s = c->stream;
   int launches = 0;
   LGR_CUDA(c, cudaMemsetAsync(D.ctr, 0, sizeof(long long) * C_COUNT, s));
   LGR_CUDA(c, cudaMemsetAsync(D.grp_err, 0, sizeof(int32_t) * (D.n_groups + 1), s));
-  cudaEventRecord(c->ev[0], s);
+  mark(c, 0, s);
   const int64_t hb = c->hap_bytes, rb = c->read_bytes;
   if (c->packed && D.n_groups > 0) {
     k_unpack_scan<<<1, 1024, 0, s>>>(D);
@@ -688,17 +716,18 @@ static int run_launch(lgr_ctx* c) {
     k_read_sketch<<<(D.n_reads + 127) / 128, 128, 0, s2>>>(D);
     cudaEventRecord(c->ev_join, s2);
     if (!c->packed) k_encode<<<enc_blocks, 256, 0, s>>>(D.hap_bases, D.hap_codes, hb), ++launches;
-    if (D.P.w == 5 && (D.P.k & 1) && 2 * D.P.k + 8 <= 32) k_hap_sketch_warp<uint32_t><<<(D.n_haps + 3) / 4, 128, 0, s>>>(D);
-    else if (D.P.w == 5 && (D.P.k & 1)) k_hap_sketch_warp<uint64_t><<<(D.n_haps + 3) / 4, 128, 0, s>>>(D);
+    const int sketch = hap_sketch_variant(D.P);
+    if (sketch == 0) k_hap_sketch_warp<uint32_t><<<(D.n_haps + 3) / 4, 128, 0, s>>>(D);
+    else if (sketch == 1) k_hap_sketch_warp<uint64_t><<<(D.n_haps + 3) / 4, 128, 0, s>>>(D);
     else k_hap_sketch<<<(D.n_haps + 63) / 64, 64, 0, s>>>(D);
     k_hap_sort<<<D.n_haps, 128, 2048 * sizeof(uint64_t), s>>>(D, c->prm.mid_occ_frac, c->prm.min_mid_occ, c->prm.max_mid_occ);
     k_group_mid<<<(D.n_groups + 127) / 128, 128, 0, s>>>(D, c->prm.min_mid_occ);
     cudaStreamWaitEvent(s, c->ev_join, 0);
     launches += 4;
-    cudaEventRecord(c->ev[1], s);
+    mark(c, 1, s);
     k_read_filter<<<(D.n_reads + 127) / 128, 128, 0, s>>>(D);
     launches += 1;
-    cudaEventRecord(c->ev[2], s);
+    mark(c, 2, s);
     if (c->warp_cap == 64) {
       k_chain_lean<64><<<c->warp_blocks, kWarpsPerCta * 32, c->warp_smem, s>>>(D);
       k_chain_cold<64><<<c->cold_blocks, kWarpsPerCta * 32, c->cold_smem, s>>>(D);
@@ -707,21 +736,96 @@ static int run_launch(lgr_ctx* c) {
       k_chain_cold<128><<<c->cold_blocks, kWarpsPerCta * 32, c->cold_smem, s>>>(D);
     }
     launches += 2;
-    cudaEventRecord(c->ev[9], s);
+    mark(c, 9, s);
     launch_tail(c, D, s, &launches);
-    cudaEventRecord(c->ev[3], s);
+    mark(c, 3, s);
     if (D.n_assign > 0) {
       k_assign<<<(unsigned)((D.n_assign + 127) / 128), 128, 0, s>>>(D);
       launches += 1;
     }
   } else {
     if (D.n_groups > 0) k_group_mid<<<(D.n_groups + 127) / 128, 128, 0, s>>>(D, c->prm.min_mid_occ), ++launches;
-    cudaEventRecord(c->ev[1], s), cudaEventRecord(c->ev[2], s), cudaEventRecord(c->ev[9], s), cudaEventRecord(c->ev[3], s);
+    mark(c, 1, s), mark(c, 2, s), mark(c, 9, s), mark(c, 3, s);
   }
-  cudaEventRecord(c->ev[4], s);
+  mark(c, 4, s);
   LGR_CUDA(c, cudaMemcpyAsync(c->h_ctr, D.ctr, sizeof(long long) * C_COUNT, cudaMemcpyDeviceToHost, s));
   c->launches = launches;
   return LGR_OK;
+}
+
+// every batch-dependent branch of enqueue_pass: batches with equal keys capture graphs of the same topology
+static uint32_t graph_key(const lgr_ctx* c) {
+  const Dev& D = c->D;
+  return (uint32_t)c->packed | (uint32_t)(D.n_groups > 0) << 1 | (uint32_t)((long long)D.n_haps + D.n_reads > 0) << 2 |
+         (uint32_t)(D.n_pairs > 0) << 3 | (uint32_t)(D.n_assign > 0) << 4 | (uint32_t)(c->warp_cap == 128) << 5 |
+         (uint32_t)hap_sketch_variant(D.P) << 6;
+}
+
+// Graph mode: capture enqueue_pass on the context's streams, bring the cached executable of its topology up to
+// this batch with cudaGraphExecUpdate (grid sizes and the Dev descriptor are captured by value, so batches of any
+// size share one executable) or instantiate one when there is none or the update is refused, and launch it.  One
+// cudaGraphLaunch replaces the pass's dozen dependent launches and the gaps between them.
+static int run_launch_graph(lgr_ctx* c) {
+  cudaStream_t s = c->stream;
+  LGR_CUDA(c, cudaStreamBeginCapture(s, cudaStreamCaptureModeThreadLocal));
+  c->capturing = true;
+  int rc = enqueue_pass(c);
+  c->capturing = false;
+  cudaGraph_t graph = nullptr;
+  const cudaError_t ec = cudaStreamEndCapture(s, &graph);  // always ends the capture, also after a failed enqueue
+  if (rc != LGR_OK || ec != cudaSuccess) {
+    if (graph) cudaGraphDestroy(graph);
+    const cudaError_t el = cudaGetLastError();  // a launch that invalidated the capture
+    if (rc == LGR_OK) {
+      c->err = std::string("stream capture of the pass: ") + cudaGetErrorString(el != cudaSuccess ? el : ec);
+      rc = LGR_E_CUDA;
+    }
+    return rc;
+  }
+  const uint32_t key = graph_key(c);
+  GraphSlot* slot = nullptr;
+  for (GraphSlot& g : c->graphs)
+    if (g.exec && g.key == key) slot = &g;
+  if (slot) {
+    cudaGraphExecUpdateResultInfo info;
+    if (cudaGraphExecUpdate(slot->exec, graph, &info) == cudaSuccess) {
+      ++c->graph_updated;
+    } else {  // topology or a parameter the update cannot take: instantiate afresh
+      (void)cudaGetLastError();
+      cudaGraphExecDestroy(slot->exec);
+      slot->exec = nullptr;
+    }
+  } else {
+    slot = &c->graphs[0];
+    for (GraphSlot& g : c->graphs)
+      if (!g.exec || (slot->exec && g.used < slot->used)) slot = &g;
+    if (slot->exec) cudaGraphExecDestroy(slot->exec);
+    slot->exec = nullptr;
+  }
+  if (!slot->exec) {
+    const cudaError_t ei = cudaGraphInstantiate(&slot->exec, graph, 0);
+    if (ei != cudaSuccess) {
+      (void)cudaGetLastError();
+      slot->exec = nullptr;
+      cudaGraphDestroy(graph);
+      c->err = std::string("cudaGraphInstantiate: ") + cudaGetErrorString(ei);
+      return LGR_E_CUDA;
+    }
+    slot->key = key;
+    ++c->graph_instantiated;
+  }
+  slot->used = ++c->graph_tick;
+  cudaGraphDestroy(graph);
+  LGR_CUDA(c, cudaGraphLaunch(slot->exec, s));
+  ++c->graph_replayed;
+  return LGR_OK;
+}
+
+// one pass of the whole path, as separate launches or (graph = true) as one CUDA graph
+static int run_launch(lgr_ctx* c, bool graph) {
+  if (!c->resident) { c->err = "no batch uploaded"; return LGR_E_ARG; }
+  LGR_CUDA(c, cudaSetDevice(c->device));
+  return graph ? run_launch_graph(c) : enqueue_pass(c);
 }
 
 // Overflow pass, host driven, after the main pass has drained: the pairs whose seeds / anchors /
@@ -802,7 +906,7 @@ static int run_finish(lgr_ctx* c, lgr_stats* st) {
 }
 
 static int run_impl(lgr_ctx* c, lgr_stats* st) {
-  int rc = run_launch(c);
+  int rc = run_launch(c, c->graph_mode);
   if (rc != LGR_OK) return rc;
   LGR_CUDA(c, cudaStreamSynchronize(c->stream));
   return run_finish(c, st);
@@ -955,7 +1059,7 @@ static int submit_async(lgr_ctx* c, const void* in, lgr_batch_out* out, lgr_tick
   int rc = up(ch, in, &h2d);
   if (rc == LGR_OK) {
     cudaEventRecord(ch->ev[6], ch->stream);
-    rc = run_launch(ch);
+    rc = run_launch(ch, false);  // the pipelined path hides its launches behind the batch in flight
   }
   if (rc == LGR_OK) {
     cudaEventRecord(ch->ev[7], ch->stream);
@@ -1021,6 +1125,20 @@ int lgr_debug_counters(lgr_ctx* c, long long* out, int n) {
 int lgr_set_notify(lgr_ctx* c, lgr_notify_fn fn, void* user) {
   if (!c) return LGR_E_ARG;
   c->notify_fn = fn, c->notify_user = user;
+  return LGR_OK;
+}
+
+int lgr_set_graph_mode(lgr_ctx* c, int on) {
+  if (!c) return LGR_E_ARG;
+  c->graph_mode = on != 0;  // the cached executables stay: switching back on reuses them
+  return LGR_OK;
+}
+
+int lgr_graph_counters(lgr_ctx* c, int64_t* instantiated, int64_t* updated, int64_t* replayed) {
+  if (!c) return LGR_E_ARG;
+  if (instantiated) *instantiated = c->graph_instantiated;
+  if (updated) *updated = c->graph_updated;
+  if (replayed) *replayed = c->graph_replayed;
   return LGR_OK;
 }
 

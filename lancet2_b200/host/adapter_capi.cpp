@@ -244,7 +244,7 @@ static int BatcherRun(int device, const lgr_batch_in* in, const char* names, con
                              const int* sample_id, const long long* start0, const long long* isize,
                              const unsigned short* sam_flag, const unsigned char* mapq, const unsigned char* softclip,
                              int n_threads, int rounds, int window, int n_devices, unsigned long long* counters, int n_counters,
-                             char* out, long long cap, bool dump) {
+                             char* out, long long cap, bool dump, bool direct_graph = false) {
   try {
     JobSet js;
     BuildJobs(in, names, samples, sample_id, start0, isize, sam_flag, mapq, softclip, js);
@@ -253,7 +253,9 @@ static int BatcherRun(int device, const lgr_batch_in* in, const char* names, con
     {
       std::vector<int> devices;
       for (int d = 0; d < (n_devices > 1 ? n_devices : 1); ++d) devices.push_back(device + d);
-      lancet_gpu::GenotypeDispatcher batcher(devices, X31OfView);
+      lancet_gpu::GenotypeBatcher::Options opt;
+      opt.direct_graph = direct_graph;
+      lancet_gpu::GenotypeDispatcher batcher(devices, X31OfView, opt);
       std::vector<std::thread> workers;
       const auto t0 = std::chrono::steady_clock::now();
       for (int t = 0; t < n_threads; ++t) {
@@ -294,10 +296,12 @@ static int BatcherRun(int device, const lgr_batch_in* in, const char* names, con
         c.max_jobs_in_batch = std::max(c.max_jobs_in_batch, cd.max_jobs_in_batch);
         c.ns_pack += cd.ns_pack, c.ns_submit += cd.ns_submit, c.ns_wait += cd.ns_wait, c.ns_deliver += cd.ns_deliver;
         c.h2d_bytes += cd.h2d_bytes, c.d2h_bytes += cd.d2h_bytes, c.retried_alone += cd.retried_alone, c.ns_seal_wait += cd.ns_seal_wait;
+        c.graph_launches += cd.graph_launches;
         if (counters && d < 8) counters[9 + d] = cd.jobs;
       }
       if (counters && n_counters >= 20) counters[17] = c.h2d_bytes, counters[18] = c.d2h_bytes, counters[19] = c.retried_alone;
       if (counters && n_counters >= 21) counters[20] = c.ns_seal_wait;
+      if (counters && n_counters >= 22) counters[21] = c.graph_launches;
       if (counters) {
         counters[0] = c.batches, counters[1] = c.jobs, counters[2] = c.pairs, counters[3] = c.max_jobs_in_batch;
         counters[4] = (unsigned long long)std::chrono::duration_cast<std::chrono::nanoseconds>(t1 - t0).count();
@@ -333,6 +337,18 @@ int lgr_adapter_batcher_bench(int device, const lgr_batch_in* in, const char* na
   const int rc = BatcherRun(device, in, names, samples, sample_id, start0, isize, sam_flag, mapq, softclip, n_threads, rounds,
                             window, n_devices, counters, 21, err, err_cap, false);
   return rc;
+}
+
+// The blocking call shape on one device with GenotypeBatcher::Options::direct_graph off (0) or on: every group is a
+// Genotype() call from one of n_threads threads, `rounds` times.  counters[22] as lgr_adapter_batcher_bench plus
+// [21] calls whose device pass ran as a CUDA graph.  cap <= 0 skips the dump (timing runs).
+int lgr_adapter_direct_graph_run(int device, const lgr_batch_in* in, const char* names, const char* samples,
+                                 const int* sample_id, const long long* start0, const long long* isize,
+                                 const unsigned short* sam_flag, const unsigned char* mapq, const unsigned char* softclip,
+                                 int n_threads, int rounds, int direct_graph, unsigned long long* counters, char* out,
+                                 long long cap) {
+  return BatcherRun(device, in, names, samples, sample_id, start0, isize, sam_flag, mapq, softclip, n_threads, rounds, 1, 1,
+                    counters, 22, out, cap, true, direct_graph != 0);
 }
 
 // Failure isolation of the batcher: ONE worker enqueues every group before it collects the first (so they

@@ -344,6 +344,8 @@ GpuGenotyper::~GpuGenotyper() {
   lgr_destroy(mCtx);
 }
 
+void GpuGenotyper::SetGraphMode(bool on) { Check(mCtx, lgr_set_graph_mode(mCtx, on ? 1 : 0)); }
+
 Result GpuGenotyper::Genotype(const std::string* haps, std::size_t n_haps, const ReadIn* reads, std::size_t n_reads,
                               const VariantIn* variants, std::size_t n_variants, const NameHashFn& name_hash) {
   std::vector<GenotypeJob> jobs{GenotypeJob{haps, n_haps, reads, n_reads, variants, n_variants}};
@@ -456,6 +458,7 @@ struct GenotypeBatcher::DirectSlot {
   std::size_t slab_cap = 0;
   lgr_assign* assign = nullptr;  // pinned [assign_cap + 1] followed by one int32 status
   std::size_t assign_cap = 0;
+  std::int64_t graph_replayed = 0;  // lgr_graph_counters of ctx after the previous call
   PackScratch sc;
   ~DirectSlot() {
     if (ctx) lgr_destroy(ctx);
@@ -875,6 +878,7 @@ GenotypeBatcher::DirectSlot* GenotypeBatcher::DirectFor() {
   if (!slot) {
     auto s = std::make_unique<DirectSlot>();
     Check(nullptr, lgr_create(mOpt.device, &mParams, &s->ctx));
+    if (mOpt.direct_graph) Check(s->ctx, lgr_set_graph_mode(s->ctx, 1));
     std::lock_guard<std::mutex> lk(mDirectMu);
     slot = s.get();
     mDirect.push_back(std::move(s));
@@ -922,7 +926,12 @@ Result GenotypeBatcher::GenotypeDirect(const GenotypeJob& job) {
   const std::uint64_t t2 = NowNs();
   Result res = PackedBatch::BuildResult(job, ds->assign, mNameHash);
   const std::uint64_t t3 = NowNs();
+  std::int64_t replayed = ds->graph_replayed;
+  lgr_graph_counters(ds->ctx, nullptr, nullptr, &replayed);
+  const std::uint64_t graph_launches = static_cast<std::uint64_t>(replayed - ds->graph_replayed);
+  ds->graph_replayed = replayed;
   std::lock_guard<std::mutex> lk(mMu);
+  mCounters.graph_launches += graph_launches;
   mCounters.ns_pack += t1 - t0, mCounters.ns_submit += t2 - t1, mCounters.ns_deliver += t3 - t2;
   mCounters.batches += 1, mCounters.jobs += 1, mCounters.pairs += static_cast<std::uint64_t>(job.n_reads * job.n_haps);
   mCounters.h2d_bytes += in.slab_bytes, mCounters.d2h_bytes += n_asg * sizeof(lgr_assign);

@@ -246,6 +246,10 @@ class GpuGenotyper {
 
   [[nodiscard]] const lgr_stats& LastStats() const noexcept { return mStats; }
 
+  // lgr_set_graph_mode on this genotyper's context: every later call runs its device pass as one CUDA graph
+  // (same results, one launch per call instead of a dozen)
+  void SetGraphMode(bool on);
+
  private:
   lgr_ctx* mCtx = nullptr;
   lgr_params mParams;
@@ -303,6 +307,8 @@ class GenotypeBatcher {
                                       // 16 blocking threads: 2.2 K / 7.6 K / 10.7 K / 11.8 K, against 1.3 K / 3.6 K / 6.7 K /
                                       // 10.5 K with everything through the batcher (0) and 3.9 K at 16 threads with
                                       // everything direct (the callers then contend inside the driver)
+    bool direct_graph = false;        // the direct contexts above run their device pass as one CUDA graph
+                                      // (lgr_set_graph_mode): same results, one launch per call instead of a dozen
     const lgr_params* params = nullptr;
   };
   struct Counters {
@@ -312,6 +318,7 @@ class GenotypeBatcher {
     std::uint64_t ns_seal_wait = 0;  // ... of which waiting for workers that were still writing their record
     std::uint64_t ns_wait = 0;     // batcher thread: lgr_wait (statistics, rare overflow pass)
     std::uint64_t ns_deliver = 0;  // worker time: AddToTable (summed over workers)
+    std::uint64_t graph_launches = 0;  // direct calls whose device pass ran as a CUDA graph (Options::direct_graph)
   };
   GenotypeBatcher(const Options& opt, NameHashFn name_hash);
   ~GenotypeBatcher();  // drains what is queued, then joins

@@ -137,6 +137,17 @@ class GpuRealigner:
         self._check(self.lib.lgr_download(self._ctx, C.byref(bo)))
         return res
 
+    def set_graph_mode(self, on: bool = True):
+        """`lgr_set_graph_mode`: run the device pass of genotype_batch / genotype_packed / run_resident as one CUDA
+        graph (same results); submit / submit_packed are unaffected."""
+        self._check(self.lib.lgr_set_graph_mode(self._ctx, 1 if on else 0))
+
+    def graph_counters(self) -> Tuple[int, int, int]:
+        """(instantiated, updated, replayed) executables of graph mode since the context was created"""
+        i, u, r = C.c_int64(0), C.c_int64(0), C.c_int64(0)
+        self._check(self.lib.lgr_graph_counters(self._ctx, C.byref(i), C.byref(u), C.byref(r)))
+        return int(i.value), int(u.value), int(r.value)
+
     def resident_assign(self):
         """(device address, count) of the lgr_assign records of the batch this context ran last: the input of
         GpuFormatMetrics.from_assign(dev_assign=...), so the assignments never visit the host."""
