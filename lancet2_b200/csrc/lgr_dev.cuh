@@ -101,7 +101,6 @@ struct Dev {      // everything the kernels need, passed by value
   uint8_t* dir_scratch; int64_t dir_per_warp;
   int32_t* bnd_scratch; int64_t bnd_per_warp;   // Hb/Fb boundary rows
   uint32_t* wcig_scratch; int wcig_cap;
-  RegRec* wreg_scratch;          // [warps][CAP] regs of the pair a warp is working on
   RadixScratch* rsx_scratch;     // [warps]
   // outputs
   AlnOut* aln; uint32_t* cigar_inline; uint32_t* cigar_arena; int64_t cigar_arena_cap;

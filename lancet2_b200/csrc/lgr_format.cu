@@ -11,6 +11,7 @@
 #include <vector>
 
 #include "lgr_format.cuh"
+#include "lgr_host.h"
 
 namespace {
 
@@ -297,11 +298,6 @@ __global__ void __launch_bounds__(lgr_fmt::kThreads) k_fmt_metrics(const __grid_
   }
 }
 
-struct Buf {
-  void* p = nullptr;
-  size_t cap = 0;
-};
-
 }  // namespace
 
 struct lgr_fmt_ctx {
@@ -310,36 +306,12 @@ struct lgr_fmt_ctx {
   cudaStream_t stream = nullptr;
   cudaEvent_t ev0 = nullptr, ev1 = nullptr;
   std::string err;
-  Buf b_in, b_keep, b_out;  // one packed input arena, the dedup flags, the results
-  Buf b_ev, b_key;           // lgr_format_from_assign: per-read / per-variant inputs + slots, support keys
+  DeviceBuffer b_in, b_keep, b_out;  // one packed input arena, the dedup flags, the results
+  DeviceBuffer b_ev, b_key;           // lgr_format_from_assign: per-read / per-variant inputs + slots, support keys
   lgr_evidence_in last_ev{};  // device pointers of the columns the last call worked on (lgr_format_debug_evidence)
 };
 
 static thread_local std::string g_fmt_create_err;
-
-#define FMT_CUDA(ctx, call)                                            \
-  do {                                                                 \
-    cudaError_t e_ = (call);                                           \
-    if (e_ != cudaSuccess) {                                           \
-      (ctx)->err = std::string(#call) + ": " + cudaGetErrorString(e_); \
-      return LGR_E_CUDA;                                               \
-    }                                                                  \
-  } while (0)
-
-static int fmt_ensure(lgr_fmt_ctx* c, Buf& b, size_t bytes) {
-  if (bytes < 256) bytes = 256;
-  if (b.cap >= bytes) return LGR_OK;
-  if (b.p) cudaFree(b.p);
-  b.p = nullptr, b.cap = 0;
-  const size_t want = bytes + bytes / 2;
-  cudaError_t e = cudaMalloc(&b.p, want);
-  if (e != cudaSuccess) {
-    c->err = std::string("cudaMalloc(") + std::to_string(want) + "): " + cudaGetErrorString(e);
-    return LGR_E_NOMEM;
-  }
-  b.cap = want;
-  return LGR_OK;
-}
 
 extern "C" {
 
@@ -364,7 +336,7 @@ int lgr_format_create(int device_ordinal, lgr_fmt_ctx** out) {
   if (e == cudaSuccess) e = cudaEventCreate(&c->ev1);
   if (e != cudaSuccess) {
     g_fmt_create_err = std::string("lgr_format_create: ") + cudaGetErrorString(e);
-    delete c;
+    lgr_format_destroy(c);
     return LGR_E_CUDA;
   }
   *out = c;
@@ -374,12 +346,10 @@ int lgr_format_create(int device_ordinal, lgr_fmt_ctx** out) {
 void lgr_format_destroy(lgr_fmt_ctx* c) {
   if (!c) return;
   cudaSetDevice(c->device);
-  for (Buf* b : {&c->b_in, &c->b_keep, &c->b_out})
-    if (b->p) cudaFree(b->p);
   if (c->ev0) cudaEventDestroy(c->ev0);
   if (c->ev1) cudaEventDestroy(c->ev1);
   if (c->stream) cudaStreamDestroy(c->stream);
-  delete c;
+  delete c;  // frees the device buffers
 }
 
 const char* lgr_format_last_error(const lgr_fmt_ctx* c) { return c ? c->err.c_str() : g_fmt_create_err.c_str(); }
@@ -408,7 +378,7 @@ int lgr_format_metrics(lgr_fmt_ctx* c, const lgr_evidence_in* in, lgr_format* ou
     for (int64_t i = in->sup_begin[s]; i < in->sup_begin[s + 1]; ++i)
       if (in->allele[i] >= in->sup_n_alleles[s]) return c->err = "evidence allele index >= the support's allele count", LGR_E_ARG;
 
-  FMT_CUDA(c, cudaSetDevice(c->device));
+  LGR_CUDA(c, cudaSetDevice(c->device));
   // one packed arena: 8-byte arrays first, then 4-byte, then bytes (every section 16-byte aligned)
   auto up16 = [](size_t x) { return (x + 15) & ~(size_t)15; };
   const size_t n = (size_t)N;
@@ -423,29 +393,29 @@ int lgr_format_metrics(lgr_fmt_ctx* c, const lgr_evidence_in* in, lgr_format* ou
                o_hash = take(n * 4), o_rnm = take(n * 4), o_onm = take(n * 4), o_hid = take(n * 4), o_al = take(n),
                o_fl = take(n), o_bq = take(n), o_mq = take(n);
   int rc;
-  if ((rc = fmt_ensure(c, c->b_in, off)) != LGR_OK) return rc;
-  if ((rc = fmt_ensure(c, c->b_keep, n)) != LGR_OK) return rc;
-  if ((rc = fmt_ensure(c, c->b_out, (size_t)S * sizeof(lgr_format))) != LGR_OK) return rc;
+  if ((rc = c->b_in.ensure(off, false, c->err)) != LGR_OK) return rc;
+  if ((rc = c->b_keep.ensure(n, false, c->err)) != LGR_OK) return rc;
+  if ((rc = c->b_out.ensure((size_t)S * sizeof(lgr_format), false, c->err)) != LGR_OK) return rc;
   char* base = (char*)c->b_in.p;
   auto h2d = [&](size_t o, const void* src, size_t bytes) -> cudaError_t {
     return bytes ? cudaMemcpyAsync(base + o, src, bytes, cudaMemcpyHostToDevice, c->stream) : cudaSuccess;
   };
-  FMT_CUDA(c, h2d(o_begin, in->sup_begin, (size_t)(S + 1) * 8));
-  FMT_CUDA(c, h2d(o_k, in->sup_n_alleles, (size_t)S * 4));
-  FMT_CUDA(c, h2d(o_vl, in->sup_variant_len, (size_t)S * 4));
-  FMT_CUDA(c, h2d(o_th, in->sup_total_haps, (size_t)S * 4));
-  FMT_CUDA(c, h2d(o_isz, in->insert_size, n * 8));
-  FMT_CUDA(c, h2d(o_start, in->aln_start, n * 8));
-  FMT_CUDA(c, h2d(o_aln, in->aln_score, n * 8));
-  FMT_CUDA(c, h2d(o_fold, in->folded_pos, n * 8));
-  FMT_CUDA(c, h2d(o_hash, in->rname_hash, n * 4));
-  FMT_CUDA(c, h2d(o_rnm, in->ref_nm, n * 4));
-  FMT_CUDA(c, h2d(o_onm, in->own_hap_nm, n * 4));
-  FMT_CUDA(c, h2d(o_hid, in->hap_id, n * 4));
-  FMT_CUDA(c, h2d(o_al, in->allele, n));
-  FMT_CUDA(c, h2d(o_fl, in->flags, n));
-  FMT_CUDA(c, h2d(o_bq, in->base_qual, n));
-  FMT_CUDA(c, h2d(o_mq, in->map_qual, n));
+  LGR_CUDA(c, h2d(o_begin, in->sup_begin, (size_t)(S + 1) * 8));
+  LGR_CUDA(c, h2d(o_k, in->sup_n_alleles, (size_t)S * 4));
+  LGR_CUDA(c, h2d(o_vl, in->sup_variant_len, (size_t)S * 4));
+  LGR_CUDA(c, h2d(o_th, in->sup_total_haps, (size_t)S * 4));
+  LGR_CUDA(c, h2d(o_isz, in->insert_size, n * 8));
+  LGR_CUDA(c, h2d(o_start, in->aln_start, n * 8));
+  LGR_CUDA(c, h2d(o_aln, in->aln_score, n * 8));
+  LGR_CUDA(c, h2d(o_fold, in->folded_pos, n * 8));
+  LGR_CUDA(c, h2d(o_hash, in->rname_hash, n * 4));
+  LGR_CUDA(c, h2d(o_rnm, in->ref_nm, n * 4));
+  LGR_CUDA(c, h2d(o_onm, in->own_hap_nm, n * 4));
+  LGR_CUDA(c, h2d(o_hid, in->hap_id, n * 4));
+  LGR_CUDA(c, h2d(o_al, in->allele, n));
+  LGR_CUDA(c, h2d(o_fl, in->flags, n));
+  LGR_CUDA(c, h2d(o_bq, in->base_qual, n));
+  LGR_CUDA(c, h2d(o_mq, in->map_qual, n));
 
   FmtDev D;
   D.e.insert_size = (const int64_t*)(base + o_isz), D.e.aln_start = (const int64_t*)(base + o_start);
@@ -460,23 +430,23 @@ int lgr_format_metrics(lgr_fmt_ctx* c, const lgr_evidence_in* in, lgr_format* ou
   D.keep = (uint8_t*)c->b_keep.p, D.out = (lgr_format*)c->b_out.p;
   D.n_supports = S, D.n_evidence = N;
 
-  FMT_CUDA(c, cudaEventRecord(c->ev0, c->stream));
+  LGR_CUDA(c, cudaEventRecord(c->ev0, c->stream));
   if (N > 0) {
     const unsigned blocks = (unsigned)((N + 255) / 256);
     k_fmt_dedup<<<blocks, 256, 0, c->stream>>>(D);
-    FMT_CUDA(c, cudaGetLastError());
+    LGR_CUDA(c, cudaGetLastError());
   }
   {
     // one CTA per (support, task); beyond 32 CTAs per SM and task the supports are grid-strided
     const int cap = c->sm_count * 32;
     const dim3 grid((unsigned)(S < cap ? S : cap), (unsigned)lgr_fmt::kNumTasks);
     k_fmt_metrics<<<grid, lgr_fmt::kThreads, 0, c->stream>>>(D);
-    FMT_CUDA(c, cudaGetLastError());
+    LGR_CUDA(c, cudaGetLastError());
   }
-  FMT_CUDA(c, cudaEventRecord(c->ev1, c->stream));
-  FMT_CUDA(c, cudaMemcpyAsync(out, c->b_out.p, (size_t)S * sizeof(lgr_format), cudaMemcpyDeviceToHost, c->stream));
-  FMT_CUDA(c, cudaStreamSynchronize(c->stream));
-  if (ms_kernels) FMT_CUDA(c, cudaEventElapsedTime(ms_kernels, c->ev0, c->ev1));
+  LGR_CUDA(c, cudaEventRecord(c->ev1, c->stream));
+  LGR_CUDA(c, cudaMemcpyAsync(out, c->b_out.p, (size_t)S * sizeof(lgr_format), cudaMemcpyDeviceToHost, c->stream));
+  LGR_CUDA(c, cudaStreamSynchronize(c->stream));
+  if (ms_kernels) LGR_CUDA(c, cudaEventElapsedTime(ms_kernels, c->ev0, c->ev1));
   if (n_wide > 0) {
     for (int s = 0; s < S; ++s)
       if (in->sup_n_alleles[s] > LGR_FMT_MAX_ALLELES) {
@@ -524,7 +494,7 @@ int lgr_format_from_assign(lgr_fmt_ctx* c, const lgr_assign_batch* in, lgr_forma
   const int64_t n_slots = (int64_t)NV * NS;
   if (n_slots > out_cap && (!out || !sup_key)) return c->err = "out / sup_key missing", LGR_E_ARG;
 
-  FMT_CUDA(c, cudaSetDevice(c->device));
+  LGR_CUDA(c, cudaSetDevice(c->device));
   auto up16 = [](size_t x) { return (x + 15) & ~(size_t)15; };
   size_t off = 0;
   auto take = [&](size_t bytes) {
@@ -540,7 +510,7 @@ int lgr_format_from_assign(lgr_fmt_ctx* c, const lgr_assign_batch* in, lgr_forma
                i_mq = take(nr), i_sc = take(nr), i_scnt = take((size_t)n_slots * 4), i_ssmp = take((size_t)n_slots * 4),
                i_sbeg = take((size_t)n_slots * 8), i_tot = take(3 * 8);
   int rc;
-  if ((rc = fmt_ensure(c, c->b_ev, off)) != LGR_OK) return rc;
+  if ((rc = c->b_ev.ensure(off, false, c->err)) != LGR_OK) return rc;
   char* eb = (char*)c->b_ev.p;
   // columns (capacity: one record per assign record, one support per slot)
   off = 0;
@@ -548,30 +518,30 @@ int lgr_format_from_assign(lgr_fmt_ctx* c, const lgr_assign_batch* in, lgr_forma
   const size_t o_begin = take((S_cap + 1) * 8), o_isz = take(na * 8), o_start = take(na * 8), o_aln = take(na * 8), o_fold = take(na * 8),
                o_k = take(S_cap * 4), o_vl = take(S_cap * 4), o_th = take(S_cap * 4), o_hash = take(na * 4), o_rnm = take(na * 4),
                o_onm = take(na * 4), o_hid = take(na * 4), o_al = take(na), o_fl = take(na), o_bq = take(na), o_mq = take(na);
-  if ((rc = fmt_ensure(c, c->b_in, off)) != LGR_OK) return rc;
-  if ((rc = fmt_ensure(c, c->b_keep, na)) != LGR_OK) return rc;
-  if ((rc = fmt_ensure(c, c->b_out, S_cap * sizeof(lgr_format))) != LGR_OK) return rc;
-  if ((rc = fmt_ensure(c, c->b_key, S_cap * 3 * sizeof(int32_t))) != LGR_OK) return rc;
+  if ((rc = c->b_in.ensure(off, false, c->err)) != LGR_OK) return rc;
+  if ((rc = c->b_keep.ensure(na, false, c->err)) != LGR_OK) return rc;
+  if ((rc = c->b_out.ensure(S_cap * sizeof(lgr_format), false, c->err)) != LGR_OK) return rc;
+  if ((rc = c->b_key.ensure(S_cap * 3 * sizeof(int32_t), false, c->err)) != LGR_OK) return rc;
   char* base = (char*)c->b_in.p;
   auto h2d = [&](size_t o, const void* src, size_t bytes) -> cudaError_t {
     return bytes ? cudaMemcpyAsync(eb + o, src, bytes, cudaMemcpyHostToDevice, c->stream) : cudaSuccess;
   };
-  if (!in->dev_assign) FMT_CUDA(c, h2d(i_asg, in->host_assign, na * sizeof(lgr_assign)));
-  FMT_CUDA(c, h2d(i_grb, in->grp_read_begin, (ng + 1) * 4));
-  FMT_CUDA(c, h2d(i_gvb, in->grp_var_begin, (ng + 1) * 4));
-  FMT_CUDA(c, h2d(i_gab, asg_begin.data(), (ng + 1) * 8));
-  FMT_CUDA(c, h2d(i_gnh, in->grp_n_haps, ng * 4));
-  FMT_CUDA(c, h2d(i_vg, var_grp.data(), nv * 4));
-  FMT_CUDA(c, h2d(i_vk, in->var_n_alleles, nv * 4));
-  FMT_CUDA(c, h2d(i_vl, in->var_len, nv * 4));
-  FMT_CUDA(c, h2d(i_ins, in->read_insert_size, nr * 8));
-  FMT_CUDA(c, h2d(i_st, in->read_aln_start, nr * 8));
-  FMT_CUDA(c, h2d(i_hash, in->read_name_hash, nr * 4));
-  FMT_CUDA(c, h2d(i_smp, in->read_sample, nr * 4));
-  FMT_CUDA(c, h2d(i_flag, in->read_sam_flag, nr * 2));
-  FMT_CUDA(c, h2d(i_mq, in->read_map_qual, nr));
-  FMT_CUDA(c, h2d(i_sc, in->read_soft_clipped, nr));
-  FMT_CUDA(c, cudaMemsetAsync(eb + i_tot, 0, 3 * 8, c->stream));
+  if (!in->dev_assign) LGR_CUDA(c, h2d(i_asg, in->host_assign, na * sizeof(lgr_assign)));
+  LGR_CUDA(c, h2d(i_grb, in->grp_read_begin, (ng + 1) * 4));
+  LGR_CUDA(c, h2d(i_gvb, in->grp_var_begin, (ng + 1) * 4));
+  LGR_CUDA(c, h2d(i_gab, asg_begin.data(), (ng + 1) * 8));
+  LGR_CUDA(c, h2d(i_gnh, in->grp_n_haps, ng * 4));
+  LGR_CUDA(c, h2d(i_vg, var_grp.data(), nv * 4));
+  LGR_CUDA(c, h2d(i_vk, in->var_n_alleles, nv * 4));
+  LGR_CUDA(c, h2d(i_vl, in->var_len, nv * 4));
+  LGR_CUDA(c, h2d(i_ins, in->read_insert_size, nr * 8));
+  LGR_CUDA(c, h2d(i_st, in->read_aln_start, nr * 8));
+  LGR_CUDA(c, h2d(i_hash, in->read_name_hash, nr * 4));
+  LGR_CUDA(c, h2d(i_smp, in->read_sample, nr * 4));
+  LGR_CUDA(c, h2d(i_flag, in->read_sam_flag, nr * 2));
+  LGR_CUDA(c, h2d(i_mq, in->read_map_qual, nr));
+  LGR_CUDA(c, h2d(i_sc, in->read_soft_clipped, nr));
+  LGR_CUDA(c, cudaMemsetAsync(eb + i_tot, 0, 3 * 8, c->stream));
 
   EvDev E;
   E.assign = in->dev_assign ? in->dev_assign : (const lgr_assign*)(eb + i_asg);
@@ -591,17 +561,17 @@ int lgr_format_from_assign(lgr_fmt_ctx* c, const lgr_assign_batch* in, lgr_forma
   E.o_onm = (uint32_t*)(base + o_onm), E.o_hid = (uint32_t*)(base + o_hid), E.o_allele = (uint8_t*)(base + o_al);
   E.o_flags = (uint8_t*)(base + o_fl), E.o_bq = (uint8_t*)(base + o_bq), E.o_mq = (uint8_t*)(base + o_mq);
 
-  FMT_CUDA(c, cudaEventRecord(c->ev0, c->stream));
+  LGR_CUDA(c, cudaEventRecord(c->ev0, c->stream));
   k_evidence_count<<<NV < c->sm_count * 16 ? NV : c->sm_count * 16, 128, 0, c->stream>>>(E);
   k_evidence_scan<<<1, 1024, 0, c->stream>>>(E);
   {
     const int64_t want = (n_slots + 3) / 4;
     k_evidence_scatter<<<(unsigned)(want < c->sm_count * 16 ? want : c->sm_count * 16), 128, 0, c->stream>>>(E);
   }
-  FMT_CUDA(c, cudaGetLastError());
+  LGR_CUDA(c, cudaGetLastError());
   long long totals[3] = {0, 0, 0};
-  FMT_CUDA(c, cudaMemcpyAsync(totals, eb + i_tot, sizeof(totals), cudaMemcpyDeviceToHost, c->stream));
-  FMT_CUDA(c, cudaStreamSynchronize(c->stream));
+  LGR_CUDA(c, cudaMemcpyAsync(totals, eb + i_tot, sizeof(totals), cudaMemcpyDeviceToHost, c->stream));
+  LGR_CUDA(c, cudaStreamSynchronize(c->stream));
   const int S = (int)totals[0];
   const int64_t N = totals[1];
   if (totals[2] != 0) return c->err = "an assignment names an allele outside its variant's allele count", LGR_E_ARG;
@@ -626,20 +596,20 @@ int lgr_format_from_assign(lgr_fmt_ctx* c, const lgr_assign_batch* in, lgr_forma
   if (S > 0) {
     if (N > 0) {
       k_fmt_dedup<<<(unsigned)((N + 255) / 256), 256, 0, c->stream>>>(D);
-      FMT_CUDA(c, cudaGetLastError());
+      LGR_CUDA(c, cudaGetLastError());
     }
     const int cap = c->sm_count * 32;
     const dim3 grid((unsigned)(S < cap ? S : cap), (unsigned)lgr_fmt::kNumTasks);
     k_fmt_metrics<<<grid, lgr_fmt::kThreads, 0, c->stream>>>(D);
-    FMT_CUDA(c, cudaGetLastError());
+    LGR_CUDA(c, cudaGetLastError());
   }
-  FMT_CUDA(c, cudaEventRecord(c->ev1, c->stream));
+  LGR_CUDA(c, cudaEventRecord(c->ev1, c->stream));
   if (S > 0) {
-    FMT_CUDA(c, cudaMemcpyAsync(out, c->b_out.p, (size_t)S * sizeof(lgr_format), cudaMemcpyDeviceToHost, c->stream));
-    FMT_CUDA(c, cudaMemcpyAsync(sup_key, c->b_key.p, (size_t)S * 3 * sizeof(int32_t), cudaMemcpyDeviceToHost, c->stream));
+    LGR_CUDA(c, cudaMemcpyAsync(out, c->b_out.p, (size_t)S * sizeof(lgr_format), cudaMemcpyDeviceToHost, c->stream));
+    LGR_CUDA(c, cudaMemcpyAsync(sup_key, c->b_key.p, (size_t)S * 3 * sizeof(int32_t), cudaMemcpyDeviceToHost, c->stream));
   }
-  FMT_CUDA(c, cudaStreamSynchronize(c->stream));
-  if (ms_kernels) FMT_CUDA(c, cudaEventElapsedTime(ms_kernels, c->ev0, c->ev1));
+  LGR_CUDA(c, cudaStreamSynchronize(c->stream));
+  if (ms_kernels) LGR_CUDA(c, cudaEventElapsedTime(ms_kernels, c->ev0, c->ev1));
   int n_wide = 0;
   for (int s = 0; s < S; ++s) {
     const int K = in->var_n_alleles[sup_key[3 * s + 1]];
@@ -663,28 +633,28 @@ int lgr_format_debug_evidence(lgr_fmt_ctx* c, lgr_evidence_in* dst) {
   const lgr_evidence_in& L = c->last_ev;
   const size_t n = (size_t)L.n_evidence, S = (size_t)L.n_supports;
   dst->n_supports = L.n_supports, dst->n_evidence = L.n_evidence;
-  FMT_CUDA(c, cudaSetDevice(c->device));
+  LGR_CUDA(c, cudaSetDevice(c->device));
   auto cp = [&](const void* d, const void* s, size_t bytes) -> cudaError_t {
     return d && s && bytes ? cudaMemcpy(const_cast<void*>(d), s, bytes, cudaMemcpyDeviceToHost) : cudaSuccess;
   };
   if (S > 0) {
-    FMT_CUDA(c, cp(dst->sup_begin, L.sup_begin, (S + 1) * 8));
-    FMT_CUDA(c, cp(dst->sup_n_alleles, L.sup_n_alleles, S * 4));
-    FMT_CUDA(c, cp(dst->sup_variant_len, L.sup_variant_len, S * 4));
-    FMT_CUDA(c, cp(dst->sup_total_haps, L.sup_total_haps, S * 4));
+    LGR_CUDA(c, cp(dst->sup_begin, L.sup_begin, (S + 1) * 8));
+    LGR_CUDA(c, cp(dst->sup_n_alleles, L.sup_n_alleles, S * 4));
+    LGR_CUDA(c, cp(dst->sup_variant_len, L.sup_variant_len, S * 4));
+    LGR_CUDA(c, cp(dst->sup_total_haps, L.sup_total_haps, S * 4));
   }
-  FMT_CUDA(c, cp(dst->insert_size, L.insert_size, n * 8));
-  FMT_CUDA(c, cp(dst->aln_start, L.aln_start, n * 8));
-  FMT_CUDA(c, cp(dst->aln_score, L.aln_score, n * 8));
-  FMT_CUDA(c, cp(dst->folded_pos, L.folded_pos, n * 8));
-  FMT_CUDA(c, cp(dst->rname_hash, L.rname_hash, n * 4));
-  FMT_CUDA(c, cp(dst->ref_nm, L.ref_nm, n * 4));
-  FMT_CUDA(c, cp(dst->own_hap_nm, L.own_hap_nm, n * 4));
-  FMT_CUDA(c, cp(dst->hap_id, L.hap_id, n * 4));
-  FMT_CUDA(c, cp(dst->allele, L.allele, n));
-  FMT_CUDA(c, cp(dst->flags, L.flags, n));
-  FMT_CUDA(c, cp(dst->base_qual, L.base_qual, n));
-  FMT_CUDA(c, cp(dst->map_qual, L.map_qual, n));
+  LGR_CUDA(c, cp(dst->insert_size, L.insert_size, n * 8));
+  LGR_CUDA(c, cp(dst->aln_start, L.aln_start, n * 8));
+  LGR_CUDA(c, cp(dst->aln_score, L.aln_score, n * 8));
+  LGR_CUDA(c, cp(dst->folded_pos, L.folded_pos, n * 8));
+  LGR_CUDA(c, cp(dst->rname_hash, L.rname_hash, n * 4));
+  LGR_CUDA(c, cp(dst->ref_nm, L.ref_nm, n * 4));
+  LGR_CUDA(c, cp(dst->own_hap_nm, L.own_hap_nm, n * 4));
+  LGR_CUDA(c, cp(dst->hap_id, L.hap_id, n * 4));
+  LGR_CUDA(c, cp(dst->allele, L.allele, n));
+  LGR_CUDA(c, cp(dst->flags, L.flags, n));
+  LGR_CUDA(c, cp(dst->base_qual, L.base_qual, n));
+  LGR_CUDA(c, cp(dst->map_qual, L.map_qual, n));
   return LGR_OK;
 }
 

@@ -36,10 +36,12 @@
 #include <cstdlib>
 #include <cstring>
 #include <string>
+#include <type_traits>
 #include <vector>
 
 #include "../../include/lancet_gpu_realign.h"
 #include "lgr_core.cuh"
+#include "lgr_host.h"
 
 #include "lgr_pack.h"
 
@@ -55,18 +57,19 @@ namespace {
 // =========================================================================================
 // host side
 // =========================================================================================
-struct DevBuf {   // a device buffer: either its own cudaMalloc block (arena, overflow workspace) or a view into the arena
-  void* p = nullptr;
-  size_t cap = 0;
-  size_t off = 0;  // offset in the context's arena (views)
-};
-
 // graph mode (lgr_set_graph_mode): one executable per topology of the captured pass, least recently used evicted
 constexpr int kGraphCache = 8;
 struct GraphSlot {
   cudaGraphExec_t exec = nullptr;
   uint32_t key = 0;
   uint64_t used = 0;
+};
+
+// timing events of a pass (stage times of lgr_stats) and of the copies around it (ms_h2d / ms_d2h)
+enum Ev {
+  EV_PASS_BEGIN, EV_INDEXED, EV_FILTERED, EV_CHAINED, EV_EXTENDED, EV_PASS_END,
+  EV_H2D_BEGIN, EV_H2D_END, EV_D2H_BEGIN, EV_D2H_END,
+  EV_COUNT
 };
 
 }  // namespace
@@ -79,19 +82,12 @@ struct lgr_ctx {
   DevParams P;
   std::string err;
   int sm_count = 0;
-  // ONE grow-only device arena per context; every per-batch buffer below is a view into it, laid out
-  // afresh by plan_batch.  A batch larger than any before costs one cudaFree + one cudaMalloc (cudaFree
-  // synchronises the whole device; sixty separately growing buffers made that sixty stalls per regrow
-  // and dominated the batcher's submit time in the first round-2 measurement).
-  DevBuf arena;
-  size_t arena_off = 0;
-  std::vector<DevBuf*> views;
-  DevBuf b_grp_hap, b_grp_read, b_grp_var, b_hap_off, b_read_off, b_var_hap_off, b_hap_bases, b_read_bases, b_read_quals,
-      b_name_hash, b_var_start, b_var_len, b_var_allele, b_read_grp, b_hap_grp, b_pair_off, b_asg_off, b_item_hap, b_item_r0,
-      b_item_n, b_hap_codes, b_read_codes, b_idx, b_idx_n, b_hap_mid, b_grp_mid, b_mz_x, b_mz_y, b_mz_n, b_fin, b_regs,
-      b_pair_reg, b_ext_arena, b_ovf_read, b_ovf_hap, b_dir, b_bnd, b_wcig, b_aln, b_cig_inline, b_cig_arena, b_assign,
-      b_ctr, b_ws_big, b_wreg, b_rsx, b_bkt, b_mz_cnt, b_tasks, b_grp_mid_req, b_grp_err, b_slab, b_dir_tab, b_grp_hapbase,
-      b_grp_readbase, b_grp_vh, b_grp_pair, b_grp_asg, b_grp_item, b_cold_read, b_cold_hap, b_hap_chk, b_read_chk, b_read_qoff, b_grp_lut;
+  // ONE grow-only device arena per context; every per-batch array of D is a view into it, laid out afresh by
+  // plan_batch.  A batch larger than any before costs one cudaFree + one cudaMalloc (cudaFree synchronises the
+  // whole device; sixty separately growing buffers made that sixty stalls per regrow and dominated the batcher's
+  // submit time in the first round-2 measurement).
+  DeviceBuffer arena;
+  DeviceBuffer ws_big;  // the overflow pass's chain workspace, sized to measure
   Dev D;
   bool resident = false, packed = false;
   int occ_cap = 0, warp_blocks_full = 0, ext_blocks_full = 0, fin_blocks_full = 0, overflow_passes = 0;
@@ -99,7 +95,7 @@ struct lgr_ctx {
   int64_t hap_bytes = 0, read_bytes = 0;
   int ext_blocks = 0, fin_blocks = 0, warp_blocks = 0, cold_blocks = 0, cold_blocks_full = 0, warp_cap = 64;
   size_t warp_smem = 0, cold_smem = 0;
-  cudaEvent_t ev[12];
+  cudaEvent_t ev[EV_COUNT] = {};
   long long* h_ctr = nullptr;  // pinned copy of the device counters
   int launches = 0;
   // graph mode of the blocking calls: the pass is captured and replayed as a CUDA graph (run_launch_graph)
@@ -122,28 +118,30 @@ struct lgr_ctx {
 
 static thread_local std::string g_create_err;
 
-#define LGR_CUDA(ctx, call)                                                                  \
-  do {                                                                                       \
-    cudaError_t e_ = (call);                                                                 \
-    if (e_ != cudaSuccess) {                                                                 \
-      (ctx)->err = std::string(#call) + ": " + cudaGetErrorString(e_);                       \
-      return LGR_E_CUDA;                                                                     \
-    }                                                                                        \
-  } while (0)
+// the chain kernels of one anchor cap: their launch attributes, and how many blocks of each an SM holds
+template <int CAP>
+static bool chain_occupancy(const lgr_ctx* c, int* per_sm, int* per_sm_cold) {
+  const cudaError_t e1 = cudaFuncSetAttribute(k_chain_lean<CAP>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)c->warp_smem);
+  cudaFuncSetAttribute(k_chain_lean<CAP>, cudaFuncAttributePreferredSharedMemoryCarveout, LGR_CHAIN_CARVEOUT);
+  const cudaError_t e2 = cudaOccupancyMaxActiveBlocksPerMultiprocessor(per_sm, k_chain_lean<CAP>, kWarpsPerCta * 32, c->warp_smem);
+  const cudaError_t e3 = cudaFuncSetAttribute(k_chain_cold<CAP>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)c->cold_smem);
+  const cudaError_t e4 = cudaOccupancyMaxActiveBlocksPerMultiprocessor(per_sm_cold, k_chain_cold<CAP>, kWarpsPerCta * 32, c->cold_smem);
+  return e1 == cudaSuccess && e2 == cudaSuccess && e3 == cudaSuccess && e4 == cudaSuccess;
+}
 
-static int ensure(lgr_ctx* c, DevBuf& b, size_t bytes) {
-  if (bytes < 256) bytes = 256;
-  if (b.cap >= bytes) return LGR_OK;
-  if (b.p) cudaFree(b.p);
-  b.p = nullptr, b.cap = 0;
-  size_t want = bytes + bytes / 2;  // cudaFree/cudaMalloc synchronise the device: regrow rarely
-  cudaError_t e = cudaMalloc(&b.p, want);
-  if (e != cudaSuccess) {
-    c->err = std::string("cudaMalloc(") + std::to_string(want) + "): " + cudaGetErrorString(e);
-    return LGR_E_NOMEM;
-  }
-  b.cap = want;
-  return LGR_OK;
+template <int CAP>
+static void launch_chain(const lgr_ctx* c, const Dev& D, cudaStream_t s) {
+  k_chain_lean<CAP><<<c->warp_blocks, kWarpsPerCta * 32, c->warp_smem, s>>>(D);
+  k_chain_cold<CAP><<<c->cold_blocks, kWarpsPerCta * 32, c->cold_smem, s>>>(D);
+}
+
+// one host→device copy into the arena view dst (a const input field of D): `count` elements, as layout_arena
+// sized the view; adds the bytes to h2d
+template <class T>
+static cudaError_t copy_in(lgr_ctx* c, const T* dst, const void* src, size_t count, int64_t& h2d) {
+  const size_t bytes = count * sizeof(T);
+  h2d += bytes;
+  return bytes ? cudaMemcpyAsync(const_cast<T*>(dst), src, bytes, cudaMemcpyHostToDevice, c->stream) : cudaSuccess;
 }
 
 extern "C" {
@@ -239,7 +237,7 @@ int lgr_create(int device_ordinal, const lgr_params* params, lgr_ctx** out) {
   c->prm = p;
   if (cudaSetDevice(device_ordinal) != cudaSuccess || cudaStreamCreateWithFlags(&c->stream, cudaStreamNonBlocking) != cudaSuccess) {
     g_create_err = "cudaSetDevice/cudaStreamCreate failed";
-    delete c;
+    lgr_destroy(c);
     return LGR_E_CUDA;
   }
   cudaDeviceProp prop;
@@ -248,7 +246,7 @@ int lgr_create(int device_ordinal, const lgr_params* params, lgr_ctx** out) {
   for (auto& e : c->ev) cudaEventCreate(&e);
   if (cudaMallocHost((void**)&c->h_ctr, sizeof(long long) * (C_COUNT + 8)) != cudaSuccess) {
     g_create_err = "cudaMallocHost failed";
-    delete c;
+    lgr_destroy(c);
     return LGR_E_CUDA;
   }
   cudaStreamCreateWithFlags(&c->stream2, cudaStreamNonBlocking);
@@ -278,14 +276,13 @@ void lgr_destroy(lgr_ctx* c) {
   for (GraphSlot& g : c->graphs)
     if (g.exec) cudaGraphExecDestroy(g.exec);
   if (c->h_ctr) cudaFreeHost(c->h_ctr);
-  if (c->arena.p) cudaFree(c->arena.p);
-  if (c->b_ws_big.p) cudaFree(c->b_ws_big.p);
-  for (auto& e : c->ev) cudaEventDestroy(e);
+  for (cudaEvent_t e : c->ev)
+    if (e) cudaEventDestroy(e);
   if (c->ev_fork) cudaEventDestroy(c->ev_fork);
   if (c->ev_join) cudaEventDestroy(c->ev_join);
   if (c->stream2) cudaStreamDestroy(c->stream2);
   if (c->stream) cudaStreamDestroy(c->stream);
-  delete c;
+  delete c;  // frees the device buffers
 }
 
 #ifdef LGR_EXT_HIST
@@ -321,7 +318,7 @@ static constexpr int kBigCapMax = 65535;          // anchors per pair the chain 
 // everything the buffer plan needs to know about a batch (from lgr_batch_in or from the packed directory)
 struct BatchSizes {
   bool ascii = true;                       // plain form (ASCII strings) or packed slab
-  size_t slab_bytes = 0, dir_bytes = 0;    // packed form: bytes of the slab / of a directory outside the slab
+  size_t slab_bytes = 0, dir_entries = 0;  // packed form: bytes of the slab / directory entries outside the slab
   int G = 0, NH = 0, NR = 0, NV = 0;
   int64_t hap_bytes = 0, read_bytes = 0, nvh = 0, n_pairs = 0, n_assign = 0, n_items = 0;
   int item_reads = 1, max_read_len = 0, max_hap_len = 0;
@@ -409,61 +406,87 @@ static int validate_batch(lgr_ctx* c, const lgr_batch_in* in, BatchSizes* z) {
   return check_limits(c, *z);
 }
 
-// device buffers + the Dev descriptor for a batch of these sizes (grow-only; no copies here)
-static int plan_batch(lgr_ctx* c, const BatchSizes& z) {
-  int rc;
-  LGR_CUDA(c, cudaSetDevice(c->device));
-  const int G = z.G, NH = z.NH, NR = z.NR, NV = z.NV;
-  const int64_t hap_bytes = z.hap_bytes, read_bytes = z.read_bytes, nvh = z.nvh, n_pairs = z.n_pairs, n_assign = z.n_assign;
-  c->max_read_len = z.max_read_len, c->max_hap_len = z.max_hap_len;
-  c->hap_bytes = hap_bytes, c->read_bytes = read_bytes;
-  c->arena_off = 0;
-  c->views.clear();
-  auto take = [&](DevBuf& b, size_t bytes) {
-    if (bytes < 256) bytes = 256;
-    b.off = c->arena_off, b.cap = bytes, b.p = nullptr;
-    c->arena_off += (bytes + 255) & ~(size_t)255;
-    c->views.push_back(&b);
-  };
-#define ENS(buf, bytes) take(c->buf, (size_t)(bytes))
-  (void)rc;
-  ENS(b_grp_hap, sizeof(int32_t) * (G + 1)); ENS(b_grp_read, sizeof(int32_t) * (G + 1)); ENS(b_grp_var, sizeof(int32_t) * (G + 1));
-  ENS(b_hap_off, sizeof(int64_t) * (NH + 1)); ENS(b_read_off, sizeof(int64_t) * (NR + 1)); ENS(b_var_hap_off, sizeof(int64_t) * (NV + 1));
-  ENS(b_read_quals, read_bytes); ENS(b_name_hash, sizeof(uint32_t) * NR);
-  ENS(b_var_start, sizeof(int32_t) * nvh); ENS(b_var_len, sizeof(int32_t) * nvh); ENS(b_var_allele, nvh);
-  ENS(b_read_grp, sizeof(int32_t) * NR); ENS(b_hap_grp, sizeof(int32_t) * NH);
-  ENS(b_pair_off, sizeof(int64_t) * (NR + 1)); ENS(b_asg_off, sizeof(int64_t) * (NR + 1));
-  ENS(b_item_hap, sizeof(int32_t) * z.n_items); ENS(b_item_r0, sizeof(int32_t) * z.n_items); ENS(b_item_n, sizeof(int32_t) * z.n_items);
-  ENS(b_grp_mid_req, sizeof(int32_t) * G); ENS(b_grp_mid, sizeof(int32_t) * G); ENS(b_grp_err, sizeof(int32_t) * (G + 1));
-  ENS(b_hap_codes, hap_bytes); ENS(b_read_codes, read_bytes);
-  ENS(b_idx, sizeof(uint64_t) * hap_bytes); ENS(b_idx_n, sizeof(int32_t) * NH); ENS(b_hap_mid, sizeof(int32_t) * NH);
-  ENS(b_bkt, sizeof(uint16_t) * (size_t)NH * (kBuckets + 1));
-  ENS(b_mz_x, sizeof(uint64_t) * read_bytes); ENS(b_mz_y, sizeof(uint32_t) * read_bytes); ENS(b_mz_n, sizeof(int32_t) * NR);
-  ENS(b_mz_cnt, sizeof(uint64_t) * 2 * (size_t)NR);
-  const int fin_cap = 2 * c->max_read_len + 16;
-  const int Lm = std::max(c->max_read_len, 1);
+// The Dev descriptor of a batch of these sizes: its scalars, and every per-batch array as a view into the arena at
+// `base`, in one fixed order, each rounded up to 256 bytes and so 256-byte aligned (k_encode relies on that).
+// base == 0 only measures.  Returns the arena bytes the batch needs.  The grids (plan_batch) must be set.
+static size_t layout_arena(Dev& D, const lgr_ctx* c, const BatchSizes& z, uintptr_t base) {
+  std::memset(&D, 0, sizeof(D));  // D.ws / D.ws_cap: k_chain_overflow's workspace, set by overflow_pass
+  D.P = c->P;
+  D.n_groups = z.G, D.n_haps = z.NH, D.n_reads = z.NR, D.n_vars = z.NV, D.n_pairs = z.n_pairs, D.n_assign = z.n_assign;
+  D.n_items = (int)z.n_items, D.item_reads = z.item_reads, D.mid_occ_param = c->prm.mid_occ;
+  D.bkt_shift = 2 * c->prm.k > kBucketBits ? 2 * c->prm.k - kBucketBits : 0;
+  const int Lm = std::max(z.max_read_len, 1);
   const int Tmax = Lm + ((c->prm.a + std::max(c->prm.b, c->prm.sc_ambi)) * Lm) / c->prm.e + 2;
+  D.fin_cap = 2 * z.max_read_len + 16;
+  D.regs_cap = z.n_pairs + z.n_pairs / 4 + 1024;
+  D.tasks_cap = D.regs_cap * 2;
+  D.ext_arena_cap = 4 * z.n_pairs + (1 << 20);
+  D.ovf_cap = z.n_pairs;
+  D.dir_per_warp = (int64_t)((Lm + 31) / 32) * (Tmax + 32) * 32;
+  D.bnd_per_warp = 2 * (int64_t)(Tmax + 32);
+  D.wcig_cap = 2 * Lm + 8;
+  D.cigar_arena_cap = std::max<int64_t>(c->prm.cigar_arena_ops, 1024);
+  // per-warp scratch follows the grid that indexes it: extension / finish kernels vs the cold chain kernel
+  const size_t ext_warps = (size_t)std::max(c->ext_blocks, c->fin_blocks) * 4;
+  const size_t chain_warps = (size_t)c->cold_blocks * kWarpsPerCta;  // the cold kernel's radix scratch
+  const size_t G = z.G, NH = z.NH, NR = z.NR, NV = z.NV, nvh = z.nvh, pairs = z.n_pairs;
+  const size_t hap_bytes = z.hap_bytes, read_bytes = z.read_bytes;
+  size_t off = 0;
+  auto take = [&](auto*& field, size_t count) {
+    field = reinterpret_cast<std::remove_reference_t<decltype(field)>>(base + off);
+    off += (std::max<size_t>(256, count * sizeof(*field)) + 255) & ~(size_t)255;
+  };
+  take(D.grp_hap_begin, G + 1), take(D.grp_read_begin, G + 1), take(D.grp_var_begin, G + 1);
+  take(D.hap_off, NH + 1), take(D.read_off, NR + 1), take(D.var_hap_off, NV + 1);
+  take(D.read_quals, read_bytes), take(D.name_hash, NR);
+  take(D.var_start, nvh), take(D.var_len, nvh), take(D.var_allele, nvh);
+  take(D.read_grp, NR), take(D.hap_grp, NH);
+  take(D.pair_off, NR + 1), take(D.asg_off, NR + 1);
+  take(D.item_hap, z.n_items), take(D.item_r0, z.n_items), take(D.item_n, z.n_items);
+  take(D.grp_mid_req, G), take(D.grp_mid, G), take(D.grp_err, G + 1);
+  take(D.hap_codes, hap_bytes), take(D.read_codes, read_bytes);
+  take(D.idx, hap_bytes), take(D.idx_n, NH), take(D.hap_mid, NH);
+  take(D.bkt, NH * (kBuckets + 1));
+  take(D.mz_x, read_bytes), take(D.mz_y, read_bytes), take(D.mz_n, NR);
+  take(D.mz_cnt, 2 * NR);
+  take(D.rsx_scratch, chain_warps);
+  take(D.fin_scratch, ext_warps * 2 * D.fin_cap);
+  take(D.regs, D.regs_cap), take(D.pair_reg, pairs);
+  take(D.tasks, D.tasks_cap * kExtClasses);
+  take(D.ext_arena, D.ext_arena_cap);
+  take(D.ovf_read, pairs + 32), take(D.ovf_hap, pairs + 32);
+  take(D.cold_read, pairs + 32), take(D.cold_hap, pairs + 32);
+  take(D.dir_scratch, ext_warps * D.dir_per_warp);
+  take(D.bnd_scratch, ext_warps * D.bnd_per_warp);
+  take(D.wcig_scratch, ext_warps * D.wcig_cap);
+  take(D.aln, pairs);
+  take(D.cigar_inline, pairs * LGR_CIGAR_INLINE);
+  take(D.cigar_arena, D.cigar_arena_cap);
+  take(D.assign, z.n_assign), take(D.ctr, C_COUNT);
+  // inputs as they arrive: ASCII strings (plain form) or the slab (+ directory, + directory scans) of the packed form
+  take(D.hap_bases, z.ascii ? hap_bytes : 0), take(D.read_bases, z.ascii ? read_bytes : 0);
+  take(D.slab, z.slab_bytes), take(D.dir, z.dir_entries);
+  take(D.grp_hapbase, G + 1), take(D.grp_readbase, G + 1), take(D.grp_vh, G + 1);
+  take(D.grp_pair, G + 1), take(D.grp_asg, G + 1), take(D.grp_item, G + 1);
+  take(D.hap_plane, z.ascii ? 0 : NH), take(D.read_plane, z.ascii ? 0 : NR);
+  take(D.read_qoff, z.ascii ? 0 : NR), take(D.grp_lut, z.ascii ? 0 : 4 * G);
+  return off;
+}
+
+// grids, arena and Dev descriptor for a batch of these sizes (grow-only; no copies here)
+static int plan_batch(lgr_ctx* c, const BatchSizes& z) {
+  LGR_CUDA(c, cudaSetDevice(c->device));
+  const int64_t n_pairs = z.n_pairs;
+  c->max_read_len = z.max_read_len, c->max_hap_len = z.max_hap_len;
+  c->hap_bytes = z.hap_bytes, c->read_bytes = z.read_bytes;
   // warp-per-pair kernel: CAP anchors per pair in shared memory
   c->warp_cap = c->max_read_len <= 160 ? 64 : 128;
   c->warp_smem = chain_smem_bytes(c->warp_cap, true);
   c->cold_smem = chain_smem_bytes(c->warp_cap, false);
   if (c->occ_cap != c->warp_cap) {  // occupancy of the persistent kernels: once per context and shape
     int per_sm = 0, per_sm_cold = 0;
-    cudaError_t e1, e2, e3, e4;
-    if (c->warp_cap == 64) {
-      e1 = cudaFuncSetAttribute(k_chain_lean<64>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)c->warp_smem);
-      cudaFuncSetAttribute(k_chain_lean<64>, cudaFuncAttributePreferredSharedMemoryCarveout, LGR_CHAIN_CARVEOUT);
-      e2 = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_chain_lean<64>, kWarpsPerCta * 32, c->warp_smem);
-      e3 = cudaFuncSetAttribute(k_chain_cold<64>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)c->cold_smem);
-      e4 = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm_cold, k_chain_cold<64>, kWarpsPerCta * 32, c->cold_smem);
-    } else {
-      e1 = cudaFuncSetAttribute(k_chain_lean<128>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)c->warp_smem);
-      cudaFuncSetAttribute(k_chain_lean<128>, cudaFuncAttributePreferredSharedMemoryCarveout, LGR_CHAIN_CARVEOUT);
-      e2 = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_chain_lean<128>, kWarpsPerCta * 32, c->warp_smem);
-      e3 = cudaFuncSetAttribute(k_chain_cold<128>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)c->cold_smem);
-      e4 = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm_cold, k_chain_cold<128>, kWarpsPerCta * 32, c->cold_smem);
-    }
-    if (e1 != cudaSuccess || e2 != cudaSuccess || e3 != cudaSuccess || e4 != cudaSuccess || per_sm < 1 || per_sm_cold < 1) {
+    const bool ok = c->warp_cap == 64 ? chain_occupancy<64>(c, &per_sm, &per_sm_cold) : chain_occupancy<128>(c, &per_sm, &per_sm_cold);
+    if (!ok || per_sm < 1 || per_sm_cold < 1) {
       c->err = "the chain kernels do not fit on this device (shared memory / registers)";
       return LGR_E_CUDA;
     }
@@ -480,84 +503,12 @@ static int plan_batch(lgr_ctx* c, const BatchSizes& z) {
   c->cold_blocks = (int)std::max<int64_t>(1, std::min<int64_t>(c->cold_blocks_full, (n_pairs + kWarpsPerCta - 1) / kWarpsPerCta));
   c->ext_blocks = (int)std::max<int64_t>(1, std::min<int64_t>(c->ext_blocks_full, (n_pairs + 15) / 16));  // ~0.3 queued extensions per pair
   c->fin_blocks = (int)std::max<int64_t>(1, std::min<int64_t>(c->fin_blocks_full, (n_pairs + 4 * kFinChunk - 1) / (4 * kFinChunk)));
-  // per-warp scratch follows the grid that indexes it: extension / finish kernels vs the chain kernels
-  const int64_t ext_warps = (int64_t)std::max(c->ext_blocks, c->fin_blocks) * 4;
-  const int64_t chain_warps = (int64_t)c->cold_blocks * kWarpsPerCta;  // the cold kernel's radix scratch
-  const int64_t dir_per_warp = (int64_t)((Lm + 31) / 32) * (Tmax + 32) * 32;
-  const int64_t bnd_per_warp = 2 * (int64_t)(Tmax + 32);
-  const int wcig_cap = 2 * Lm + 8;
-  const int64_t regs_cap = n_pairs + n_pairs / 4 + 1024;
-  const int64_t ext_arena_cap = 4 * n_pairs + (1 << 20);
-  const int64_t cig_arena_cap = std::max<int64_t>(c->prm.cigar_arena_ops, 1024);
-  ENS(b_rsx, sizeof(RadixScratch) * (size_t)chain_warps);
-  ENS(b_fin, sizeof(uint32_t) * (size_t)ext_warps * 2 * fin_cap);
-  ENS(b_regs, sizeof(RegRec) * (size_t)regs_cap); ENS(b_pair_reg, sizeof(PairReg) * (size_t)n_pairs);
-  ENS(b_tasks, sizeof(TaskRec) * (size_t)regs_cap * 2 * kExtClasses);
-  ENS(b_ext_arena, sizeof(uint32_t) * (size_t)ext_arena_cap);
-  ENS(b_ovf_read, sizeof(int32_t) * (size_t)(n_pairs + 32)); ENS(b_ovf_hap, sizeof(int32_t) * (size_t)(n_pairs + 32));
-  ENS(b_cold_read, sizeof(int32_t) * (size_t)(n_pairs + 32)); ENS(b_cold_hap, sizeof(int32_t) * (size_t)(n_pairs + 32));
-  ENS(b_dir, (size_t)ext_warps * dir_per_warp);
-  ENS(b_bnd, sizeof(int32_t) * (size_t)ext_warps * bnd_per_warp);
-  ENS(b_wcig, sizeof(uint32_t) * (size_t)ext_warps * wcig_cap);
-  ENS(b_aln, sizeof(AlnOut) * (size_t)n_pairs);
-  ENS(b_cig_inline, sizeof(uint32_t) * (size_t)n_pairs * LGR_CIGAR_INLINE);
-  ENS(b_cig_arena, sizeof(uint32_t) * (size_t)cig_arena_cap);
-  ENS(b_assign, sizeof(AssignOut) * (size_t)n_assign); ENS(b_ctr, sizeof(long long) * C_COUNT);
-  // inputs as they arrive: ASCII strings (plain form) or the slab (+ directory, + directory scans) of the packed form
-  ENS(b_hap_bases, z.ascii ? hap_bytes : 0); ENS(b_read_bases, z.ascii ? read_bytes : 0);
-  ENS(b_slab, z.slab_bytes); ENS(b_dir_tab, z.dir_bytes);
-  ENS(b_grp_hapbase, sizeof(int64_t) * (G + 1)); ENS(b_grp_readbase, sizeof(int64_t) * (G + 1)); ENS(b_grp_vh, sizeof(int64_t) * (G + 1));
-  ENS(b_grp_pair, sizeof(int64_t) * (G + 1)); ENS(b_grp_asg, sizeof(int64_t) * (G + 1)); ENS(b_grp_item, sizeof(int32_t) * (G + 1));
-  ENS(b_hap_chk, z.ascii ? 0 : sizeof(uint64_t) * NH); ENS(b_read_chk, z.ascii ? 0 : sizeof(uint64_t) * NR);
-  ENS(b_read_qoff, z.ascii ? 0 : sizeof(uint64_t) * NR); ENS(b_grp_lut, z.ascii ? 0 : 16 * (size_t)G);
-  if ((rc = ensure(c, c->arena, c->arena_off)) != LGR_OK) return rc;
-  for (DevBuf* b : c->views) b->p = static_cast<uint8_t*>(c->arena.p) + b->off;
-  Dev& D = c->D;
-  std::memset(&D, 0, sizeof(D));
-  D.P = c->P;
-  D.n_groups = G, D.n_haps = NH, D.n_reads = NR, D.n_vars = NV, D.n_pairs = n_pairs, D.n_assign = n_assign;
-  D.grp_hap_begin = (int32_t*)c->b_grp_hap.p, D.grp_read_begin = (int32_t*)c->b_grp_read.p, D.grp_var_begin = (int32_t*)c->b_grp_var.p;
-  D.hap_off = (int64_t*)c->b_hap_off.p, D.read_off = (int64_t*)c->b_read_off.p, D.var_hap_off = (int64_t*)c->b_var_hap_off.p;
-  D.read_quals = (uint8_t*)c->b_read_quals.p;
-  D.name_hash = (uint32_t*)c->b_name_hash.p;
-  D.var_start = (int32_t*)c->b_var_start.p, D.var_len = (int32_t*)c->b_var_len.p, D.var_allele = (int8_t*)c->b_var_allele.p;
-  D.read_grp = (int32_t*)c->b_read_grp.p, D.hap_grp = (int32_t*)c->b_hap_grp.p;
-  D.pair_off = (int64_t*)c->b_pair_off.p, D.asg_off = (int64_t*)c->b_asg_off.p;
-  D.item_hap = (int32_t*)c->b_item_hap.p, D.item_r0 = (int32_t*)c->b_item_r0.p, D.item_n = (int32_t*)c->b_item_n.p;
-  D.n_items = (int)z.n_items, D.item_reads = z.item_reads, D.mid_occ_param = c->prm.mid_occ;
-  D.hap_codes = (uint8_t*)c->b_hap_codes.p, D.read_codes = (uint8_t*)c->b_read_codes.p;
-  D.idx = (uint64_t*)c->b_idx.p, D.idx_n = (int32_t*)c->b_idx_n.p, D.hap_mid = (int32_t*)c->b_hap_mid.p;
-  D.grp_mid_req = (int32_t*)c->b_grp_mid_req.p, D.grp_mid = (int32_t*)c->b_grp_mid.p, D.grp_err = (int32_t*)c->b_grp_err.p;
-  D.bkt = (uint16_t*)c->b_bkt.p;
-  D.bkt_shift = 2 * c->prm.k > kBucketBits ? 2 * c->prm.k - kBucketBits : 0;
-  D.mz_x = (uint64_t*)c->b_mz_x.p, D.mz_y = (uint32_t*)c->b_mz_y.p, D.mz_n = (int32_t*)c->b_mz_n.p;
-  D.mz_cnt = (uint64_t*)c->b_mz_cnt.p;
-  D.ws = nullptr, D.ws_cap = 0;
-  D.wreg_scratch = nullptr, D.rsx_scratch = (RadixScratch*)c->b_rsx.p;
-  D.fin_scratch = (uint32_t*)c->b_fin.p, D.fin_cap = fin_cap;
-  D.regs = (RegRec*)c->b_regs.p, D.regs_cap = regs_cap;
-  D.pair_reg = (PairReg*)c->b_pair_reg.p;
-  D.tasks = (TaskRec*)c->b_tasks.p, D.tasks_cap = regs_cap * 2;
-  D.ext_arena = (uint32_t*)c->b_ext_arena.p, D.ext_arena_cap = ext_arena_cap;
-  D.ovf_read = (int32_t*)c->b_ovf_read.p, D.ovf_hap = (int32_t*)c->b_ovf_hap.p, D.ovf_cap = n_pairs;
-  D.cold_read = (int32_t*)c->b_cold_read.p, D.cold_hap = (int32_t*)c->b_cold_hap.p;
-  D.dir_scratch = (uint8_t*)c->b_dir.p, D.dir_per_warp = dir_per_warp;
-  D.bnd_scratch = (int32_t*)c->b_bnd.p, D.bnd_per_warp = bnd_per_warp;
-  D.wcig_scratch = (uint32_t*)c->b_wcig.p, D.wcig_cap = wcig_cap;
-  D.aln = (AlnOut*)c->b_aln.p, D.cigar_inline = (uint32_t*)c->b_cig_inline.p, D.cigar_arena = (uint32_t*)c->b_cig_arena.p;
-  D.cigar_arena_cap = cig_arena_cap;
-  D.assign = (AssignOut*)c->b_assign.p;
-  D.ctr = (long long*)c->b_ctr.p;
+  Dev measured;
+  const int rc = c->arena.ensure(layout_arena(measured, c, z, 0), false, c->err);
+  if (rc != LGR_OK) return rc;
+  layout_arena(c->D, c, z, reinterpret_cast<uintptr_t>(c->arena.p));
   return LGR_OK;
-#undef ENS
 }
-
-#define UP(buf, src, bytes)                                                                              \
-  do {                                                                                                   \
-    if (c->buf.cap < (size_t)(bytes)) { c->err = "internal: buffer plan too small"; return LGR_E_ARG; }   \
-    if ((bytes) > 0) LGR_CUDA(c, cudaMemcpyAsync(c->buf.p, (src), (bytes), cudaMemcpyHostToDevice, c->stream)); \
-    h2d += (bytes);                                                                                      \
-  } while (0)
 
 // plain form: 13 caller arrays + the host-derived helper arrays, one copy each
 static int upload_impl(lgr_ctx* c, const lgr_batch_in* in, int64_t* h2d_bytes) {
@@ -580,7 +531,7 @@ static int upload_impl(lgr_ctx* c, const lgr_batch_in* in, int64_t* h2d_bytes) {
       c->h_read_grp[r] = g, c->h_pair_off[r] = po, c->h_asg_off[r] = ao;
       po += h1 - h0, ao += V;
     }
-    for (int h = h0; h < h1; ++h)
+    for (int h = h0; h < h1; ++h)  // z.n_items work items in all (validate_batch counts them the same way)
       for (int r = r0; r < r1; r += z.item_reads) {
         c->h_item_hap.push_back(h), c->h_item_r0.push_back(r), c->h_item_n.push_back(std::min(z.item_reads, r1 - r));
       }
@@ -589,28 +540,28 @@ static int upload_impl(lgr_ctx* c, const lgr_batch_in* in, int64_t* h2d_bytes) {
     c->h_grp_mid[g] = mid;
   }
   c->h_pair_off[NR] = po, c->h_asg_off[NR] = ao;
-  UP(b_grp_hap, in->grp_hap_begin, sizeof(int32_t) * (G + 1));
-  UP(b_grp_read, in->grp_read_begin, sizeof(int32_t) * (G + 1));
-  UP(b_grp_var, in->grp_var_begin, sizeof(int32_t) * (G + 1));
-  UP(b_hap_off, in->hap_off, sizeof(int64_t) * (NH + 1));
-  UP(b_read_off, in->read_off, sizeof(int64_t) * (NR + 1));
-  UP(b_var_hap_off, in->var_hap_off, sizeof(int64_t) * (NV + 1));
-  UP(b_hap_bases, in->hap_bases, (size_t)z.hap_bytes);
-  UP(b_read_bases, in->read_bases, (size_t)z.read_bytes);
-  UP(b_read_quals, in->read_quals, (size_t)z.read_bytes);
-  UP(b_name_hash, in->read_name_hash, sizeof(uint32_t) * NR);
-  UP(b_var_start, in->var_start, sizeof(int32_t) * z.nvh);
-  UP(b_var_len, in->var_len, sizeof(int32_t) * z.nvh);
-  UP(b_var_allele, in->var_allele, (size_t)z.nvh);
-  UP(b_read_grp, c->h_read_grp.data(), sizeof(int32_t) * NR);
-  UP(b_hap_grp, c->h_hap_grp.data(), sizeof(int32_t) * NH);
-  UP(b_pair_off, c->h_pair_off.data(), sizeof(int64_t) * (NR + 1));
-  UP(b_asg_off, c->h_asg_off.data(), sizeof(int64_t) * (NR + 1));
-  UP(b_item_hap, c->h_item_hap.data(), sizeof(int32_t) * c->h_item_hap.size());
-  UP(b_item_r0, c->h_item_r0.data(), sizeof(int32_t) * c->h_item_r0.size());
-  UP(b_item_n, c->h_item_n.data(), sizeof(int32_t) * c->h_item_n.size());
-  UP(b_grp_mid_req, c->h_grp_mid.data(), sizeof(int32_t) * G);
-  c->D.hap_bases = (uint8_t*)c->b_hap_bases.p, c->D.read_bases = (uint8_t*)c->b_read_bases.p;
+  const Dev& D = c->D;
+  LGR_CUDA(c, copy_in(c, D.grp_hap_begin, in->grp_hap_begin, G + 1, h2d));
+  LGR_CUDA(c, copy_in(c, D.grp_read_begin, in->grp_read_begin, G + 1, h2d));
+  LGR_CUDA(c, copy_in(c, D.grp_var_begin, in->grp_var_begin, G + 1, h2d));
+  LGR_CUDA(c, copy_in(c, D.hap_off, in->hap_off, NH + 1, h2d));
+  LGR_CUDA(c, copy_in(c, D.read_off, in->read_off, NR + 1, h2d));
+  LGR_CUDA(c, copy_in(c, D.var_hap_off, in->var_hap_off, NV + 1, h2d));
+  LGR_CUDA(c, copy_in(c, D.hap_bases, in->hap_bases, z.hap_bytes, h2d));
+  LGR_CUDA(c, copy_in(c, D.read_bases, in->read_bases, z.read_bytes, h2d));
+  LGR_CUDA(c, copy_in(c, D.read_quals, in->read_quals, z.read_bytes, h2d));
+  LGR_CUDA(c, copy_in(c, D.name_hash, in->read_name_hash, NR, h2d));
+  LGR_CUDA(c, copy_in(c, D.var_start, in->var_start, z.nvh, h2d));
+  LGR_CUDA(c, copy_in(c, D.var_len, in->var_len, z.nvh, h2d));
+  LGR_CUDA(c, copy_in(c, D.var_allele, in->var_allele, z.nvh, h2d));
+  LGR_CUDA(c, copy_in(c, D.read_grp, c->h_read_grp.data(), NR, h2d));
+  LGR_CUDA(c, copy_in(c, D.hap_grp, c->h_hap_grp.data(), NH, h2d));
+  LGR_CUDA(c, copy_in(c, D.pair_off, c->h_pair_off.data(), NR + 1, h2d));
+  LGR_CUDA(c, copy_in(c, D.asg_off, c->h_asg_off.data(), NR + 1, h2d));
+  LGR_CUDA(c, copy_in(c, D.item_hap, c->h_item_hap.data(), z.n_items, h2d));
+  LGR_CUDA(c, copy_in(c, D.item_r0, c->h_item_r0.data(), z.n_items, h2d));
+  LGR_CUDA(c, copy_in(c, D.item_n, c->h_item_n.data(), z.n_items, h2d));
+  LGR_CUDA(c, copy_in(c, D.grp_mid_req, c->h_grp_mid.data(), G, h2d));
   c->packed = false;
   c->resident = true;
   if (h2d_bytes) *h2d_bytes = h2d;
@@ -645,31 +596,32 @@ static int upload_packed_impl(lgr_ctx* c, const lgr_packed_in* in, int64_t* h2d_
   if (rc != LGR_OK) return rc;
   const uint8_t* slab = static_cast<const uint8_t*>(in->slab);
   const uint8_t* dirp = reinterpret_cast<const uint8_t*>(in->dir);
-  const size_t dir_bytes = sizeof(lgr_group_dir) * (size_t)z.G;
-  const bool dir_inside = z.G > 0 && dirp >= slab && dirp + dir_bytes <= slab + in->slab_bytes;
-  z.ascii = false, z.slab_bytes = in->slab_bytes, z.dir_bytes = dir_inside ? 0 : dir_bytes;
+  const bool dir_inside = z.G > 0 && dirp >= slab && dirp + sizeof(lgr_group_dir) * (size_t)z.G <= slab + in->slab_bytes;
+  z.ascii = false, z.slab_bytes = in->slab_bytes, z.dir_entries = dir_inside ? 0 : z.G;
   if ((rc = plan_batch(c, z)) != LGR_OK) return rc;
   int64_t h2d = 0;
-  UP(b_slab, in->slab, in->slab_bytes);
-  if (!dir_inside) UP(b_dir_tab, in->dir, dir_bytes);
   Dev& D = c->D;
-  D.slab = (const uint8_t*)c->b_slab.p;
-  D.dir = dir_inside ? reinterpret_cast<const lgr_group_dir*>(D.slab + (dirp - slab)) : (const lgr_group_dir*)c->b_dir_tab.p;
-  D.grp_hapbase = (int64_t*)c->b_grp_hapbase.p, D.grp_readbase = (int64_t*)c->b_grp_readbase.p, D.grp_vh = (int64_t*)c->b_grp_vh.p;
-  D.grp_pair = (int64_t*)c->b_grp_pair.p, D.grp_asg = (int64_t*)c->b_grp_asg.p, D.grp_item = (int32_t*)c->b_grp_item.p;
-  D.hap_plane = (uint64_t*)c->b_hap_chk.p, D.read_plane = (uint64_t*)c->b_read_chk.p;
-  D.read_qoff = (uint64_t*)c->b_read_qoff.p, D.grp_lut = (uint32_t*)c->b_grp_lut.p;
+  LGR_CUDA(c, copy_in(c, D.slab, in->slab, z.slab_bytes, h2d));
+  if (dir_inside) D.dir = reinterpret_cast<const lgr_group_dir*>(D.slab + (dirp - slab));
+  else LGR_CUDA(c, copy_in(c, D.dir, in->dir, z.dir_entries, h2d));
   c->packed = true;
   c->resident = true;
   if (h2d_bytes) *h2d_bytes = h2d;
   return LGR_OK;
 }
 
-// phase B (extensions, finish) + assignment, used by the main pass and the overflow pass
+// phase B (extensions, finish), used by the main pass and the overflow pass
 static void launch_tail(lgr_ctx* c, const Dev& D, cudaStream_t s, int* launches) {
   k_ext_warp<<<c->ext_blocks, 128, 0, s>>>(D);
   k_finish_warp<<<c->fin_blocks, 128, 0, s>>>(D);
   *launches += 2;
+}
+
+// assignment, after phase B of the main pass and of the overflow pass
+static void launch_assign(const Dev& D, cudaStream_t s, int* launches) {
+  if (D.n_assign <= 0) return;
+  k_assign<<<(unsigned)((D.n_assign + 127) / 128), 128, 0, s>>>(D);
+  *launches += 1;
 }
 
 // which k_hap_sketch instance the parameters select: 0 / 1 = warp kernel on 32- / 64-bit keys, 2 = generic
@@ -680,7 +632,7 @@ static int hap_sketch_variant(const DevParams& P) {
 
 // timing event i: an event-record node when the pass is being captured, so that the stage times of lgr_stats
 // stay meaningful in graph mode (a plain record inside a capture only orders the streams)
-static void mark(lgr_ctx* c, int i, cudaStream_t s) {
+static void mark(lgr_ctx* c, Ev i, cudaStream_t s) {
   if (c->capturing) cudaEventRecordWithFlags(c->ev[i], s, cudaEventRecordExternal);
   else cudaEventRecord(c->ev[i], s);
 }
@@ -693,7 +645,7 @@ static int enqueue_pass(lgr_ctx* c) {
   int launches = 0;
   LGR_CUDA(c, cudaMemsetAsync(D.ctr, 0, sizeof(long long) * C_COUNT, s));
   LGR_CUDA(c, cudaMemsetAsync(D.grp_err, 0, sizeof(int32_t) * (D.n_groups + 1), s));
-  mark(c, 0, s);
+  mark(c, EV_PASS_BEGIN, s);
   const int64_t hb = c->hap_bytes, rb = c->read_bytes;
   if (c->packed && D.n_groups > 0) {
     k_unpack_scan<<<1, 1024, 0, s>>>(D);
@@ -724,30 +676,21 @@ static int enqueue_pass(lgr_ctx* c) {
     k_group_mid<<<(D.n_groups + 127) / 128, 128, 0, s>>>(D, c->prm.min_mid_occ);
     cudaStreamWaitEvent(s, c->ev_join, 0);
     launches += 4;
-    mark(c, 1, s);
+    mark(c, EV_INDEXED, s);
     k_read_filter<<<(D.n_reads + 127) / 128, 128, 0, s>>>(D);
     launches += 1;
-    mark(c, 2, s);
-    if (c->warp_cap == 64) {
-      k_chain_lean<64><<<c->warp_blocks, kWarpsPerCta * 32, c->warp_smem, s>>>(D);
-      k_chain_cold<64><<<c->cold_blocks, kWarpsPerCta * 32, c->cold_smem, s>>>(D);
-    } else {
-      k_chain_lean<128><<<c->warp_blocks, kWarpsPerCta * 32, c->warp_smem, s>>>(D);
-      k_chain_cold<128><<<c->cold_blocks, kWarpsPerCta * 32, c->cold_smem, s>>>(D);
-    }
+    mark(c, EV_FILTERED, s);
+    c->warp_cap == 64 ? launch_chain<64>(c, D, s) : launch_chain<128>(c, D, s);
     launches += 2;
-    mark(c, 9, s);
+    mark(c, EV_CHAINED, s);
     launch_tail(c, D, s, &launches);
-    mark(c, 3, s);
-    if (D.n_assign > 0) {
-      k_assign<<<(unsigned)((D.n_assign + 127) / 128), 128, 0, s>>>(D);
-      launches += 1;
-    }
+    mark(c, EV_EXTENDED, s);
+    launch_assign(D, s, &launches);
   } else {
     if (D.n_groups > 0) k_group_mid<<<(D.n_groups + 127) / 128, 128, 0, s>>>(D, c->prm.min_mid_occ), ++launches;
-    mark(c, 1, s), mark(c, 2, s), mark(c, 9, s), mark(c, 3, s);
+    mark(c, EV_INDEXED, s), mark(c, EV_FILTERED, s), mark(c, EV_CHAINED, s), mark(c, EV_EXTENDED, s);
   }
-  mark(c, 4, s);
+  mark(c, EV_PASS_END, s);
   LGR_CUDA(c, cudaMemcpyAsync(c->h_ctr, D.ctr, sizeof(long long) * C_COUNT, cudaMemcpyDeviceToHost, s));
   c->launches = launches;
   return LGR_OK;
@@ -842,10 +785,10 @@ static int overflow_pass(lgr_ctx* c) {
   long long need = std::max<long long>(c->h_ctr[C_OVFNEED], 256);
   need = std::min<long long>((need + 255) / 256 * 256, kBigCapMax);
   const int lanes = (int)std::min<long long>((n_ovf + 127) / 128 * 128, kBigLanesMax);
-  int rc = ensure(c, c->b_ws_big, sizeof(int32_t) * (size_t)lanes * A_COUNT * (size_t)need);
+  int rc = c->ws_big.ensure(sizeof(int32_t) * (size_t)lanes * A_COUNT * (size_t)need, false, c->err);
   if (rc != LGR_OK) return rc;
   Dev D2 = D;
-  D2.ws = (int32_t*)c->b_ws_big.p, D2.ws_cap = (int)need;
+  D2.ws = (int32_t*)c->ws_big.p, D2.ws_cap = (int)need;
   // restart the queues of phase B: extensions continue after the tasks already done, finish and
   // assignment redo every pair (idempotent; the overflow cigar arena is refilled from 0)
   long long* hc = c->h_ctr + C_COUNT + 2;  // pinned staging of the counter patch
@@ -859,10 +802,7 @@ static int overflow_pass(lgr_ctx* c) {
   k_chain_overflow<<<lanes / 128, 128, 0, s>>>(D2);
   ++launches;
   launch_tail(c, D, s, &launches);
-  if (D.n_assign > 0) {
-    k_assign<<<(unsigned)((D.n_assign + 127) / 128), 128, 0, s>>>(D);
-    ++launches;
-  }
+  launch_assign(D, s, &launches);
   LGR_CUDA(c, cudaMemcpyAsync(c->h_ctr, D.ctr, sizeof(long long) * C_COUNT, cudaMemcpyDeviceToHost, s));
   LGR_CUDA(c, cudaStreamSynchronize(s));
   c->launches += launches;
@@ -882,13 +822,12 @@ static int run_finish(lgr_ctx* c, lgr_stats* st) {
   const long long* hctr = c->h_ctr;
   const int launches = c->launches;
   if (st) {
-    float ms;
-    cudaEventElapsedTime(&ms, c->ev[0], c->ev[4]); st->ms_kernels = ms;
-    cudaEventElapsedTime(&ms, c->ev[0], c->ev[1]); st->ms_k_index = ms;
-    cudaEventElapsedTime(&ms, c->ev[1], c->ev[2]); st->ms_k_sketch = ms;
-    cudaEventElapsedTime(&ms, c->ev[2], c->ev[9]); st->ms_k_map = ms;
-    cudaEventElapsedTime(&ms, c->ev[9], c->ev[3]); st->ms_k_ext = ms;
-    cudaEventElapsedTime(&ms, c->ev[3], c->ev[4]); st->ms_k_assign = ms;
+    cudaEventElapsedTime(&st->ms_kernels, c->ev[EV_PASS_BEGIN], c->ev[EV_PASS_END]);
+    cudaEventElapsedTime(&st->ms_k_index, c->ev[EV_PASS_BEGIN], c->ev[EV_INDEXED]);
+    cudaEventElapsedTime(&st->ms_k_sketch, c->ev[EV_INDEXED], c->ev[EV_FILTERED]);
+    cudaEventElapsedTime(&st->ms_k_map, c->ev[EV_FILTERED], c->ev[EV_CHAINED]);
+    cudaEventElapsedTime(&st->ms_k_ext, c->ev[EV_CHAINED], c->ev[EV_EXTENDED]);
+    cudaEventElapsedTime(&st->ms_k_assign, c->ev[EV_EXTENDED], c->ev[EV_PASS_END]);
     st->n_pairs = D.n_pairs, st->n_aligned = hctr[C_ALIGNED];
     st->dp_cells = hctr[C_CELLS], st->dp_cells_full = hctr[C_CELLSFULL];
     st->chain_evals = hctr[C_EVALS], st->n_anchors = hctr[C_ANCH];
@@ -1006,6 +945,12 @@ int lgr_download(lgr_ctx* c, lgr_batch_out* out) {
   return download_impl(c, out, nullptr);
 }
 
+// ms_h2d / ms_d2h of lgr_stats: the events genotype_sync and submit_async record around the copies
+static void copy_times(const lgr_ctx* c, lgr_stats* st) {
+  cudaEventElapsedTime(&st->ms_h2d, c->ev[EV_H2D_BEGIN], c->ev[EV_H2D_END]);
+  cudaEventElapsedTime(&st->ms_d2h, c->ev[EV_D2H_BEGIN], c->ev[EV_D2H_END]);
+}
+
 // synchronous: upload (either form), all kernels, download
 typedef int (*upload_fn)(lgr_ctx*, const void*, int64_t*);
 static int up_plain(lgr_ctx* c, const void* in, int64_t* b) { return upload_impl(c, static_cast<const lgr_batch_in*>(in), b); }
@@ -1016,20 +961,18 @@ static int genotype_sync(lgr_ctx* c, const void* in, lgr_batch_out* out, lgr_sta
   lgr_stats st;
   std::memset(&st, 0, sizeof(st));
   int64_t h2d = 0, d2h = 0;
-  cudaEventRecord(c->ev[5], c->stream);
+  cudaEventRecord(c->ev[EV_H2D_BEGIN], c->stream);
   int rc = up(c, in, &h2d);
   if (rc != LGR_OK) return rc;
-  cudaEventRecord(c->ev[6], c->stream);
+  cudaEventRecord(c->ev[EV_H2D_END], c->stream);
   rc = run_impl(c, &st);
   if (rc != LGR_OK && rc != LGR_E_LIMIT && rc != LGR_E_CIGAR_OVERFLOW) return rc;
   const int run_rc = limit_code(rc, out);
-  cudaEventRecord(c->ev[7], c->stream);
+  cudaEventRecord(c->ev[EV_D2H_BEGIN], c->stream);
   rc = download_impl(c, out, &d2h);
-  cudaEventRecord(c->ev[8], c->stream);
+  cudaEventRecord(c->ev[EV_D2H_END], c->stream);
   cudaStreamSynchronize(c->stream);
-  float ms;
-  cudaEventElapsedTime(&ms, c->ev[5], c->ev[6]); st.ms_h2d = ms;
-  cudaEventElapsedTime(&ms, c->ev[7], c->ev[8]); st.ms_d2h = ms;
+  copy_times(c, &st);
   st.h2d_bytes = h2d, st.d2h_bytes = d2h;
   if (stats) *stats = st;
   return run_rc != LGR_OK ? run_rc : rc;
@@ -1055,16 +998,16 @@ static int submit_async(lgr_ctx* c, const void* in, lgr_batch_out* out, lgr_tick
   }
   lgr_ctx* ch = c->slot[t];
   int64_t h2d = 0, d2h = 0;
-  cudaEventRecord(ch->ev[5], ch->stream);
+  cudaEventRecord(ch->ev[EV_H2D_BEGIN], ch->stream);
   int rc = up(ch, in, &h2d);
   if (rc == LGR_OK) {
-    cudaEventRecord(ch->ev[6], ch->stream);
+    cudaEventRecord(ch->ev[EV_H2D_END], ch->stream);
     rc = run_launch(ch, false);  // the pipelined path hides its launches behind the batch in flight
   }
   if (rc == LGR_OK) {
-    cudaEventRecord(ch->ev[7], ch->stream);
+    cudaEventRecord(ch->ev[EV_D2H_BEGIN], ch->stream);
     rc = download_launch(ch, out, &d2h);
-    cudaEventRecord(ch->ev[8], ch->stream);
+    cudaEventRecord(ch->ev[EV_D2H_END], ch->stream);
   }
   if (rc != LGR_OK) {
     cudaStreamSynchronize(ch->stream);  // leave the slot idle
@@ -1092,8 +1035,8 @@ int lgr_reserve(lgr_ctx* c, int64_t arena_bytes, int n_slots) {
       int rc = lgr_create(c->device, &c->prm, &c->slot[t]);
       if (rc != LGR_OK) { c->err = g_create_err; return rc; }
     }
-    int rc = ensure(c->slot[t], c->slot[t]->arena, (size_t)arena_bytes);
-    if (rc != LGR_OK) { c->err = c->slot[t]->err; return rc; }
+    const int rc = c->slot[t]->arena.ensure((size_t)arena_bytes, false, c->err);
+    if (rc != LGR_OK) return rc;
   }
   return LGR_OK;
 }
@@ -1181,9 +1124,7 @@ int lgr_wait(lgr_ctx* c, lgr_ticket t, lgr_stats* stats) {
     if (rc == LGR_OK) rc = download_finish(ch, c->slot_out[t], &d2h);
   }
   run_rc = limit_code(run_rc, c->slot_out[t]);
-  float ms;
-  cudaEventElapsedTime(&ms, ch->ev[5], ch->ev[6]); st.ms_h2d = ms;
-  cudaEventElapsedTime(&ms, ch->ev[7], ch->ev[8]); st.ms_d2h = ms;
+  copy_times(ch, &st);
   st.h2d_bytes = c->slot_h2d[t], st.d2h_bytes = d2h;
   if (stats) *stats = st;
   if (run_rc != LGR_OK || rc != LGR_OK) c->err = ch->err;

@@ -32,6 +32,7 @@
 #include <vector>
 
 #include "../../include/lancet_gpu_realign.h"
+#include "lgr_host.h"
 
 namespace {
 
@@ -173,8 +174,7 @@ struct lgr_rep_ctx {
   int device = 0, sm_count = 0;
   cudaStream_t stream = nullptr;
   cudaEvent_t ev0 = nullptr, ev1 = nullptr;
-  void *d_seq = nullptr, *d_jobs = nullptr, *d_out = nullptr, *d_items = nullptr, *d_ctr = nullptr;
-  size_t cap_seq = 0, cap_jobs = 0, cap_out = 0, cap_items = 0, cap_ctr = 0;
+  DeviceBuffer d_seq, d_jobs, d_out, d_items, d_ctr;
   struct Group {
     int32_t first, n, k_min;
   };
@@ -185,40 +185,16 @@ struct lgr_rep_ctx {
 
 static thread_local std::string g_rep_create_err;
 
-#define REP_CUDA(c, call)                                                      \
-  do {                                                                         \
-    cudaError_t e_ = (call);                                                   \
-    if (e_ != cudaSuccess) {                                                   \
-      (c)->err = std::string(#call) + ": " + cudaGetErrorString(e_);           \
-      return LGR_E_CUDA;                                                       \
-    }                                                                          \
-  } while (0)
-
-// grows *p to at least `bytes` (half as much again on a regrow inside lgr_repeat_scan, exactly on a reservation)
-static int rep_ensure(lgr_rep_ctx* c, void** p, size_t* cap, size_t bytes, bool exact = false) {
-  if (bytes < 256) bytes = 256;
-  if (*cap >= bytes) return LGR_OK;
-  if (*p) cudaFree(*p);
-  *p = nullptr, *cap = 0;
-  const size_t want = exact ? bytes : bytes + bytes / 2;
-  if (cudaMalloc(p, want) != cudaSuccess) {
-    c->err = "cudaMalloc failed";
-    (void)cudaGetLastError();
-    return LGR_E_NOMEM;
-  }
-  *cap = want;
-  return LGR_OK;
-}
-
 // device buffers of a batch of n_jobs jobs over seq_bytes bytes: the work items are at most max(n_jobs, resident CTAs)
-// (a group gets several slices only while there are fewer groups than resident CTAs), the counter words 1 + 2 per group
+// (a group gets several slices only while there are fewer groups than resident CTAs), the counter words 1 + 2 per group.
+// Half as much again on a regrow inside lgr_repeat_scan, exactly on a reservation.
 static int rep_buffers(lgr_rep_ctx* c, size_t seq_bytes, size_t n_jobs, size_t n_items, size_t ctr_words, bool exact) {
   int rc;
-  if ((rc = rep_ensure(c, &c->d_seq, &c->cap_seq, seq_bytes, exact)) != LGR_OK) return rc;
-  if ((rc = rep_ensure(c, &c->d_jobs, &c->cap_jobs, sizeof(lgr_repeat_job) * n_jobs, exact)) != LGR_OK) return rc;
-  if ((rc = rep_ensure(c, &c->d_out, &c->cap_out, n_jobs, exact)) != LGR_OK) return rc;
-  if ((rc = rep_ensure(c, &c->d_items, &c->cap_items, sizeof(RepItem) * n_items, exact)) != LGR_OK) return rc;
-  return rep_ensure(c, &c->d_ctr, &c->cap_ctr, sizeof(unsigned) * ctr_words, exact);
+  if ((rc = c->d_seq.ensure(seq_bytes, exact, c->err)) != LGR_OK) return rc;
+  if ((rc = c->d_jobs.ensure(sizeof(lgr_repeat_job) * n_jobs, exact, c->err)) != LGR_OK) return rc;
+  if ((rc = c->d_out.ensure(n_jobs, exact, c->err)) != LGR_OK) return rc;
+  if ((rc = c->d_items.ensure(sizeof(RepItem) * n_items, exact, c->err)) != LGR_OK) return rc;
+  return c->d_ctr.ensure(sizeof(unsigned) * ctr_words, exact, c->err);
 }
 
 extern "C" {
@@ -238,7 +214,7 @@ int lgr_repeat_create(int device_ordinal, lgr_rep_ctx** out) {
   if (cudaSetDevice(device_ordinal) != cudaSuccess || cudaGetDeviceProperties(&prop, device_ordinal) != cudaSuccess ||
       cudaStreamCreateWithFlags(&c->stream, cudaStreamNonBlocking) != cudaSuccess) {
     g_rep_create_err = "cudaSetDevice / cudaStreamCreate failed";
-    delete c;
+    lgr_repeat_destroy(c);
     return LGR_E_CUDA;
   }
   c->sm_count = prop.multiProcessorCount;
@@ -250,15 +226,10 @@ int lgr_repeat_create(int device_ordinal, lgr_rep_ctx** out) {
 void lgr_repeat_destroy(lgr_rep_ctx* c) {
   if (!c) return;
   cudaSetDevice(c->device);
-  if (c->d_seq) cudaFree(c->d_seq);
-  if (c->d_jobs) cudaFree(c->d_jobs);
-  if (c->d_out) cudaFree(c->d_out);
-  if (c->d_items) cudaFree(c->d_items);
-  if (c->d_ctr) cudaFree(c->d_ctr);
   if (c->ev0) cudaEventDestroy(c->ev0);
   if (c->ev1) cudaEventDestroy(c->ev1);
   if (c->stream) cudaStreamDestroy(c->stream);
-  delete c;
+  delete c;  // frees the device buffers
 }
 
 const char* lgr_repeat_last_error(const lgr_rep_ctx* c) { return c ? c->err.c_str() : g_rep_create_err.c_str(); }
@@ -310,27 +281,27 @@ int lgr_repeat_scan(lgr_rep_ctx* c, const uint8_t* seqs, int64_t seq_bytes, cons
   }
   const int n_items = (int)items.size();
   const size_t ctr_words = 1 + 2 * (size_t)n_sliced;  // queue counter, then found[n_sliced], done[n_sliced]
-  REP_CUDA(c, cudaSetDevice(c->device));
+  LGR_CUDA(c, cudaSetDevice(c->device));
   int rc;
   if ((rc = rep_buffers(c, (size_t)seq_bytes, (size_t)n_jobs, (size_t)n_items, ctr_words, false)) != LGR_OK) return rc;
-  REP_CUDA(c, cudaMemsetAsync(c->d_ctr, 0, sizeof(unsigned) * ctr_words, c->stream));
-  if (seq_bytes > 0) REP_CUDA(c, cudaMemcpyAsync(c->d_seq, seqs, (size_t)seq_bytes, cudaMemcpyHostToDevice, c->stream));
-  REP_CUDA(c, cudaMemcpyAsync(c->d_jobs, jobs, sizeof(lgr_repeat_job) * (size_t)n_jobs, cudaMemcpyHostToDevice, c->stream));
-  REP_CUDA(c, cudaMemcpyAsync(c->d_items, items.data(), sizeof(RepItem) * items.size(), cudaMemcpyHostToDevice, c->stream));
-  unsigned* ctr = (unsigned*)c->d_ctr;
-  RepDev D{(const uint8_t*)c->d_seq, (const lgr_repeat_job*)c->d_jobs, (const RepItem*)c->d_items, (uint8_t*)c->d_out,
+  LGR_CUDA(c, cudaMemsetAsync(c->d_ctr.p, 0, sizeof(unsigned) * ctr_words, c->stream));
+  if (seq_bytes > 0) LGR_CUDA(c, cudaMemcpyAsync(c->d_seq.p, seqs, (size_t)seq_bytes, cudaMemcpyHostToDevice, c->stream));
+  LGR_CUDA(c, cudaMemcpyAsync(c->d_jobs.p, jobs, sizeof(lgr_repeat_job) * (size_t)n_jobs, cudaMemcpyHostToDevice, c->stream));
+  LGR_CUDA(c, cudaMemcpyAsync(c->d_items.p, items.data(), sizeof(RepItem) * items.size(), cudaMemcpyHostToDevice, c->stream));
+  unsigned* ctr = (unsigned*)c->d_ctr.p;
+  RepDev D{(const uint8_t*)c->d_seq.p, (const lgr_repeat_job*)c->d_jobs.p, (const RepItem*)c->d_items.p, (uint8_t*)c->d_out.p,
            (int*)ctr, ctr + 1, ctr + 1 + n_sliced, n_items};
-  REP_CUDA(c, cudaEventRecord(c->ev0, c->stream));
+  LGR_CUDA(c, cudaEventRecord(c->ev0, c->stream));
   const int grid = n_items < resident ? n_items : resident;
   if (n_sliced > 0)
     k_repeat_scan<true><<<grid, kRepThreads, 0, c->stream>>>(D);
   else
     k_repeat_scan<false><<<grid, kRepThreads, 0, c->stream>>>(D);
-  REP_CUDA(c, cudaGetLastError());
-  REP_CUDA(c, cudaEventRecord(c->ev1, c->stream));
-  REP_CUDA(c, cudaMemcpyAsync(has_repeat, c->d_out, (size_t)n_jobs, cudaMemcpyDeviceToHost, c->stream));
-  REP_CUDA(c, cudaStreamSynchronize(c->stream));
-  if (ms_kernels) REP_CUDA(c, cudaEventElapsedTime(ms_kernels, c->ev0, c->ev1));
+  LGR_CUDA(c, cudaGetLastError());
+  LGR_CUDA(c, cudaEventRecord(c->ev1, c->stream));
+  LGR_CUDA(c, cudaMemcpyAsync(has_repeat, c->d_out.p, (size_t)n_jobs, cudaMemcpyDeviceToHost, c->stream));
+  LGR_CUDA(c, cudaStreamSynchronize(c->stream));
+  if (ms_kernels) LGR_CUDA(c, cudaEventElapsedTime(ms_kernels, c->ev0, c->ev1));
   if (too_long) {
     c->err = "some sequences are longer than LGR_REPEAT_MAX_LEN (their answers are LGR_REPEAT_TOO_LONG)";
     return LGR_E_PARTIAL;
@@ -341,7 +312,7 @@ int lgr_repeat_scan(lgr_rep_ctx* c, const uint8_t* seqs, int64_t seq_bytes, cons
 int lgr_repeat_reserve(lgr_rep_ctx* c, int64_t seq_bytes, int32_t n_jobs) {
   if (!c || seq_bytes < 0 || n_jobs < 0) return LGR_E_ARG;
   c->err.clear();
-  REP_CUDA(c, cudaSetDevice(c->device));
+  LGR_CUDA(c, cudaSetDevice(c->device));
   const size_t resident = (size_t)c->sm_count * kRepCtasPerSm;
   const int rc = rep_buffers(c, (size_t)seq_bytes, (size_t)n_jobs, std::max((size_t)n_jobs, resident), 1 + 2 * (size_t)n_jobs, true);
   c->groups.reserve((size_t)n_jobs);
