@@ -482,6 +482,71 @@ int lgr_resident_assign(lgr_ctx* ctx, const lgr_assign** dev_assign, int64_t* n_
 /* test hook: the evidence columns lgr_format_from_assign built last, copied into dst's (caller-allocated) arrays */
 int lgr_format_debug_evidence(lgr_fmt_ctx* ctx, lgr_evidence_in* dst);
 
+/* Packed evidence (one block per window).  Lancet2 computes FORMAT fields per window on the worker thread right after
+ * Genotype() (CollectSupportedCalls -> VariantCall); lgr_format_metrics copies every column of a call separately.  Here
+ * each worker packs its window ONCE into a slab (pure host code, any thread), and a whole batch of windows crosses PCIe
+ * in ONE copy:
+ *
+ *   slab  := block, block, ...  [directory]                        (blocks 16-byte aligned)
+ *   block := lgr_fmt_blk_hdr | sup_begin i64[S+1] (window-local, [0, N]) | insert_size, aln_start, aln_score,
+ *            folded_pos (8-byte)[N] | sup_n_alleles, sup_variant_len, sup_total_haps i32[S] | rname_hash, ref_nm,
+ *            own_hap_nm, hap_id u32[N] | allele, flags, base_qual, map_qual u8[N]
+ *   every section 16-byte aligned, zero padded; the order is that of the device arena of lgr_format_metrics.
+ * The device scatters the blocks into that arena (sup_begin rebased to the batch) and runs the same two kernels, so a
+ * window's records equal lgr_format_metrics on that window alone, byte for byte, whatever batch it travels in. */
+#define LGR_FMT_MAGIC 0x31544d46u /* "FMT1" */
+#define LGR_FMT_SECTIONS 16
+typedef struct lgr_fmt_blk_hdr {   /* first 160 bytes of a block */
+  uint32_t magic;                   /* LGR_FMT_MAGIC */
+  int32_t n_supports;               /* S */
+  int64_t n_evidence;               /* N */
+  uint64_t rec_bytes;               /* size of the block (multiple of 16) */
+  uint64_t reserved;
+  uint64_t off[LGR_FMT_SECTIONS];   /* byte offset of each section from the block start, in the order above */
+} lgr_fmt_blk_hdr;
+
+typedef struct lgr_fmt_dir {       /* directory entry of one window (48 bytes) */
+  uint64_t rec_off;                 /* byte offset of the block in the slab (multiple of 16) */
+  int64_t n_evidence;               /* N of the block */
+  int64_t ev_base;                  /* first record of the window in the batch: sum of n_evidence of the windows before */
+  int32_t n_supports;               /* S of the block */
+  int32_t sup_base;                 /* first support of the window in the batch: sum of n_supports of the windows before */
+  int32_t n_wide;                   /* supports with more than LGR_FMT_MAX_ALLELES alleles */
+  int32_t reserved[3];
+} lgr_fmt_dir;
+
+typedef struct lgr_fmt_packed_in {
+  int32_t n_windows;
+  int32_t reserved;
+  const void* slab;                 /* host memory (pinned for an asynchronous copy) */
+  size_t slab_bytes;                /* bytes to copy */
+  const lgr_fmt_dir* dir;           /* [n_windows]; inside [slab, slab + slab_bytes) => ONE copy, else a second small one */
+} lgr_fmt_packed_in;
+
+/* bytes lgr_format_pack writes for this window (upper bound, multiple of 16); 0 on a malformed input (NULL, negative
+ * sizes) */
+size_t lgr_format_packed_bytes(const lgr_evidence_in* in);
+/* Pack one window into dst[0..cap).  Validates what lgr_format_metrics validates (lgr_format.cu:358-379: negative sizes,
+ * missing arrays, sup_begin spanning [0, N] and monotone, K >= 1, allele < K) and returns LGR_E_ARG for a malformed
+ * window or a too small cap.  Fills *dir (may be NULL) except rec_off / sup_base / ev_base: the caller places the block.
+ * Pure host code (no CUDA call), safe on any thread.  A window without supports packs as an empty block. */
+int lgr_format_pack(const lgr_evidence_in* in, void* dst, size_t cap, lgr_fmt_dir* dir);
+/* lgr_format_metrics over many packed windows: ONE H2D of the slab (plus the directory when it lies outside),
+ * k_fmt_unpack scatters the blocks into the arena lgr_format_metrics builds, then the same k_fmt_dedup / k_fmt_metrics,
+ * ONE D2H of out[S] for S = the windows' supports in directory order.  The host checks the directory only (magic,
+ * counts and rec_bytes of each block's header, blocks inside the slab, sup_base / ev_base the prefix sums of the
+ * counts): anything else is LGR_E_ARG before any CUDA call.  Records the device finds malformed (sup_begin outside
+ * [0, N] or not monotone, K < 1, allele >= K, a wide support in a window whose n_wide is 0) are computed as empty
+ * supports and the call returns LGR_E_ARG.  Wide supports as in lgr_format_metrics (LGR_FMT_WIDE, LGR_E_PARTIAL).
+ * ms_kernels (may be NULL) = CUDA-event time of the three kernels. */
+int lgr_format_metrics_packed(lgr_fmt_ctx* ctx, const lgr_fmt_packed_in* in, lgr_format* out, float* ms_kernels);
+/* allocate every device buffer of a packed call of up to slab_bytes bytes (directory inside), n_supports supports and
+ * n_evidence records now: lgr_format_metrics_packed then never regrows them within these sizes (a regrow frees and
+ * allocates device memory, which synchronises the whole device) */
+int lgr_format_reserve(lgr_fmt_ctx* ctx, int64_t slab_bytes, int32_t n_supports, int64_t n_evidence);
+/* device bytes the context holds (all its buffers) */
+int64_t lgr_format_device_bytes(const lgr_fmt_ctx* ctx);
+
 /* ------------------------------------------------------------------------------------------
  * SURVEY.md §8f #3 (first half) — repeat detection over the sliding k-mers of reference windows.
  *

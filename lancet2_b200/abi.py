@@ -415,6 +415,35 @@ class EvidenceBatch:
         return st
 
 
+# packed evidence: one block per window (lgr_format_pack / lgr_format_metrics_packed)
+LGR_FMT_MAGIC = 0x31544D46
+LGR_FMT_SECTIONS = 16
+# the sections of a block, in order: (name, element dtype, per support (+1 for sup_begin) or per record)
+FMT_SECTIONS = [("sup_begin", np.int64, "S+1")] + [(n, d, "N") for n, d in EVIDENCE_FIELDS[:4]] + \
+    [("sup_n_alleles", np.int32, "S"), ("sup_variant_len", np.int32, "S"), ("sup_total_haps", np.int32, "S")] + \
+    [(n, d, "N") for n, d in EVIDENCE_FIELDS[4:]]
+
+
+class LgrFmtBlkHdr(C.Structure):
+    _fields_ = [("magic", C.c_uint32), ("n_supports", C.c_int32), ("n_evidence", C.c_int64), ("rec_bytes", C.c_uint64),
+                ("reserved", C.c_uint64), ("off", C.c_uint64 * LGR_FMT_SECTIONS)]
+
+
+class LgrFmtDir(C.Structure):
+    _fields_ = [("rec_off", C.c_uint64), ("n_evidence", C.c_int64), ("ev_base", C.c_int64), ("n_supports", C.c_int32),
+                ("sup_base", C.c_int32), ("n_wide", C.c_int32), ("reserved", C.c_int32 * 3)]
+
+
+FMT_DIR_DTYPE = np.dtype([("rec_off", "<u8"), ("n_evidence", "<i8"), ("ev_base", "<i8"), ("n_supports", "<i4"),
+                          ("sup_base", "<i4"), ("n_wide", "<i4"), ("reserved", "<i4", (3,))])
+assert FMT_DIR_DTYPE.itemsize == C.sizeof(LgrFmtDir) == 48 and C.sizeof(LgrFmtBlkHdr) == 160
+
+
+class LgrFmtPackedIn(C.Structure):
+    _fields_ = [("n_windows", C.c_int32), ("reserved", C.c_int32), ("slab", C.c_void_p), ("slab_bytes", C.c_size_t),
+                ("dir", C.c_void_p)]
+
+
 class LgrRepeatJob(C.Structure):
     _fields_ = [("seq_off", C.c_int64), ("seq_len", C.c_int32), ("k", C.c_int32), ("max_mismatches", C.c_int32),
                 ("reserved", C.c_int32)]
@@ -431,6 +460,7 @@ _SYMBOLS = [
     "lgr_set_notify", "lgr_set_graph_mode", "lgr_graph_counters", "lgr_reserve", "lgr_arena_bytes", "lgr_check_limits", "lgr_packed_group_bytes", "lgr_pack_group", "lgr_genotype_packed", "lgr_submit_packed", "lgr_upload_packed",
     "lgr_format_create", "lgr_format_destroy", "lgr_format_last_error", "lgr_format_metrics",
     "lgr_format_from_assign", "lgr_resident_assign", "lgr_format_debug_evidence",
+    "lgr_format_packed_bytes", "lgr_format_pack", "lgr_format_metrics_packed", "lgr_format_reserve", "lgr_format_device_bytes",
     "lgr_repeat_create", "lgr_repeat_destroy", "lgr_repeat_last_error", "lgr_repeat_scan", "lgr_repeat_reserve",
 ]
 
@@ -519,6 +549,16 @@ def load_library(path: Optional[str] = None) -> C.CDLL:
     lib.lgr_resident_assign.restype = C.c_int
     lib.lgr_format_debug_evidence.argtypes = [C.c_void_p, C.POINTER(LgrEvidenceIn)]
     lib.lgr_format_debug_evidence.restype = C.c_int
+    lib.lgr_format_packed_bytes.argtypes = [C.POINTER(LgrEvidenceIn)]
+    lib.lgr_format_packed_bytes.restype = C.c_size_t
+    lib.lgr_format_pack.argtypes = [C.POINTER(LgrEvidenceIn), C.c_void_p, C.c_size_t, C.POINTER(LgrFmtDir)]
+    lib.lgr_format_pack.restype = C.c_int
+    lib.lgr_format_metrics_packed.argtypes = [C.c_void_p, C.POINTER(LgrFmtPackedIn), C.c_void_p, C.POINTER(C.c_float)]
+    lib.lgr_format_metrics_packed.restype = C.c_int
+    lib.lgr_format_reserve.argtypes = [C.c_void_p, C.c_int64, C.c_int32, C.c_int64]
+    lib.lgr_format_reserve.restype = C.c_int
+    lib.lgr_format_device_bytes.argtypes = [C.c_void_p]
+    lib.lgr_format_device_bytes.restype = C.c_int64
     lib.lgr_repeat_create.argtypes = [C.c_int, C.POINTER(C.c_void_p)]
     lib.lgr_repeat_create.restype = C.c_int
     lib.lgr_repeat_destroy.argtypes = [C.c_void_p]

@@ -298,6 +298,144 @@ __global__ void __launch_bounds__(lgr_fmt::kThreads) k_fmt_metrics(const __grid_
   }
 }
 
+// ---------------------------------------------------------------------------------------------
+// Packed windows (lgr_format_pack / lgr_format_metrics_packed).  A block and the device arena of lgr_format_metrics
+// share one section order (lgr_format.cu:391-394); fmt_layout gives the 16 offsets from `base` (the header size for a
+// block, 0 for the arena) and returns the end.
+// ---------------------------------------------------------------------------------------------
+constexpr int kSecBegin = 0, kSecK = 5, kSecVl = 6, kSecTh = 7, kSecAllele = 12;
+__host__ __device__ constexpr int fmt_sec_size(int k) { return k <= 4 ? 8 : k <= 11 ? 4 : 1; }
+__host__ __device__ constexpr bool fmt_sec_per_support(int k) { return k == kSecBegin || (k >= kSecK && k <= kSecTh); }
+
+__host__ __device__ inline uint64_t fmt_layout(int64_t S, int64_t N, uint64_t base, uint64_t* off) {
+  uint64_t o = base;
+  for (int k = 0; k < LGR_FMT_SECTIONS; ++k) {
+    const uint64_t n = k == kSecBegin ? (uint64_t)S + 1 : fmt_sec_per_support(k) ? (uint64_t)S : (uint64_t)N;
+    off[k] = o;
+    o += (n * fmt_sec_size(k) + 15) & ~(uint64_t)15;
+  }
+  return o;
+}
+
+// offset of section k alone (the kernel's form of fmt_layout: no per-thread offset array in local memory)
+__device__ __forceinline__ uint64_t fmt_sec_off(int64_t S, int64_t N, uint64_t base, int k) {
+  uint64_t o = base;
+#pragma unroll
+  for (int j = 0; j < LGR_FMT_SECTIONS; ++j) {
+    const uint64_t n = j == kSecBegin ? (uint64_t)S + 1 : fmt_sec_per_support(j) ? (uint64_t)S : (uint64_t)N;
+    if (j < k) o += (n * fmt_sec_size(j) + 15) & ~(uint64_t)15;
+  }
+  return o;
+}
+
+struct UnpackDev {
+  const uint8_t* slab;      // device copy of the slab
+  const lgr_fmt_dir* dir;   // device copy of the directory
+  int32_t n_windows, n_supports;
+  int64_t n_evidence;
+  int64_t n_rec_ctas;       // CTAs [0, n_rec_ctas) copy records, the rest one support per warp
+  uint8_t* arena;           // lgr_format_metrics' arena, sections at aoff
+  uint64_t aoff[LGR_FMT_SECTIONS];
+  int* status;              // set to 1 when a block's records are malformed
+};
+constexpr int kUnpackThreads = 256, kUnpackWarps = kUnpackThreads / 32;
+constexpr int64_t kUnpackChunk = 512;  // records per CTA of the copy half (a cfg2 step: 228 CTAs)
+
+// last window whose base (ev_base or sup_base) is <= x: the window that holds record / support x (windows without any
+// share their base with the next one and are skipped)
+template <bool kEv>
+__device__ __forceinline__ int fmt_window_of(const lgr_fmt_dir* dir, int n_windows, int64_t x) {
+  int lo = 0, hi = n_windows;
+  while (hi - lo > 1) {
+    const int mid = (lo + hi) >> 1;
+    if ((kEv ? dir[mid].ev_base : (int64_t)dir[mid].sup_base) <= x) lo = mid;
+    else hi = mid;
+  }
+  return lo;
+}
+
+// one warp copies `bytes` bytes: 16-byte vectors when source and destination agree modulo 16, else elements of `es`
+// bytes (both are always aligned to their element size)
+__device__ __forceinline__ void fmt_copy_span(uint8_t* dst, const uint8_t* src, uint64_t bytes, int es, int lane) {
+  const uint64_t mis = ((uintptr_t)dst ^ (uintptr_t)src) & 15;
+  if (mis == 0) {
+    uint64_t head = (16 - ((uintptr_t)src & 15)) & 15;
+    if (head > bytes) head = bytes;
+    for (uint64_t i = lane; i < head; i += 32) dst[i] = src[i];
+    const uint64_t nvec = (bytes - head) >> 4;
+    const uint4* s4 = reinterpret_cast<const uint4*>(src + head);
+    uint4* d4 = reinterpret_cast<uint4*>(dst + head);
+    for (uint64_t i = lane; i < nvec; i += 32) d4[i] = s4[i];
+    for (uint64_t i = head + (nvec << 4) + lane; i < bytes; i += 32) dst[i] = src[i];
+  } else if (es == 8) {
+    for (uint64_t i = lane; i < bytes / 8; i += 32) reinterpret_cast<uint64_t*>(dst)[i] = reinterpret_cast<const uint64_t*>(src)[i];
+  } else if (es == 4) {
+    for (uint64_t i = lane; i < bytes / 4; i += 32) reinterpret_cast<uint32_t*>(dst)[i] = reinterpret_cast<const uint32_t*>(src)[i];
+  } else {
+    for (uint64_t i = lane; i < bytes; i += 32) dst[i] = src[i];
+  }
+}
+
+// Scatter of the packed blocks into the arena, over two kinds of work item so that one oversized window is spread
+// over the GPU like many small ones:
+//  * a CTA of the first kind owns kUnpackChunk consecutive records of the batch; its warps take the (window, column)
+//    pieces of that range and copy them;
+//  * a warp of the second kind owns one support: sup_begin[sup_base + s] = ev_base + local_begin[s] (and the final
+//    entry N), the three support columns, and the checks the host skipped.  A support whose range is not inside
+//    [0, N] and ordered, whose K < 1, whose records name an allele >= K, or that is wide in a window that declared no
+//    wide supports sets *status and is written as a wide (never computed) support with a clamped begin, so that
+//    k_fmt_dedup / k_fmt_metrics stay inside the arena whatever the slab holds.
+__global__ void __launch_bounds__(kUnpackThreads) k_fmt_unpack(const __grid_constant__ UnpackDev U) {
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  constexpr uint64_t kHdr = sizeof(lgr_fmt_blk_hdr);
+  if ((int64_t)blockIdx.x < U.n_rec_ctas) {
+    const int64_t lo = (int64_t)blockIdx.x * kUnpackChunk;
+    const int64_t hi = lo + kUnpackChunk < U.n_evidence ? lo + kUnpackChunk : U.n_evidence;
+    const int w0 = fmt_window_of<true>(U.dir, U.n_windows, lo);
+    constexpr int kCols = LGR_FMT_SECTIONS - 4;  // the twelve record columns
+    for (int piece = warp;; piece += kUnpackWarps) {
+      const int w = w0 + piece / kCols;
+      if (w >= U.n_windows) break;
+      const lgr_fmt_dir d = U.dir[w];
+      if (d.ev_base >= hi) break;
+      const int64_t a = lo > d.ev_base ? lo - d.ev_base : 0;
+      const int64_t b = hi - d.ev_base < d.n_evidence ? hi - d.ev_base : d.n_evidence;
+      if (a >= b) continue;
+      const int c = piece % kCols, k = c < 4 ? 1 + c : 4 + c;  // sections 1..4 and 8..15
+      const int es = fmt_sec_size(k);
+      fmt_copy_span(U.arena + U.aoff[k] + (uint64_t)(d.ev_base + a) * es,
+                    U.slab + d.rec_off + fmt_sec_off(d.n_supports, d.n_evidence, kHdr, k) + (uint64_t)a * es,
+                    (uint64_t)(b - a) * es, es, lane);
+    }
+    return;
+  }
+  const int64_t g = ((int64_t)blockIdx.x - U.n_rec_ctas) * kUnpackWarps + warp;
+  if (g >= U.n_supports) return;
+  const int w = fmt_window_of<false>(U.dir, U.n_windows, g);
+  const lgr_fmt_dir d = U.dir[w];
+  const int s = (int)(g - d.sup_base);
+  const uint8_t* blk = U.slab + d.rec_off;
+  const int64_t* lb = reinterpret_cast<const int64_t*>(blk + kHdr);
+  const int64_t N = d.n_evidence, b = lb[s], e = lb[s + 1];
+  const int K = reinterpret_cast<const int32_t*>(blk + fmt_sec_off(d.n_supports, N, kHdr, kSecK))[s];
+  bool ok = lb[0] == 0 && lb[d.n_supports] == N && 0 <= b && b <= e && e <= N && K >= 1 &&
+            (K <= LGR_FMT_MAX_ALLELES || d.n_wide > 0);
+  if (ok) {
+    const uint8_t* al = blk + fmt_sec_off(d.n_supports, N, kHdr, kSecAllele);
+    bool bad = false;
+    for (int64_t i = b + lane; i < e; i += 32) bad |= al[i] >= K;
+    ok = !__any_sync(0xffffffffu, bad);
+  }
+  if (lane == 0) {
+    reinterpret_cast<int64_t*>(U.arena + U.aoff[kSecBegin])[g] = d.ev_base + (b < 0 ? 0 : b > N ? N : b);
+    reinterpret_cast<int32_t*>(U.arena + U.aoff[kSecK])[g] = ok ? K : LGR_FMT_MAX_ALLELES + 1;
+    reinterpret_cast<int32_t*>(U.arena + U.aoff[kSecVl])[g] = reinterpret_cast<const int32_t*>(blk + fmt_sec_off(d.n_supports, N, kHdr, kSecVl))[s];
+    reinterpret_cast<int32_t*>(U.arena + U.aoff[kSecTh])[g] = reinterpret_cast<const int32_t*>(blk + fmt_sec_off(d.n_supports, N, kHdr, kSecTh))[s];
+    if (g == U.n_supports - 1) reinterpret_cast<int64_t*>(U.arena + U.aoff[kSecBegin])[g + 1] = U.n_evidence;
+    if (!ok) *U.status = 1;
+  }
+}
+
 }  // namespace
 
 struct lgr_fmt_ctx {
@@ -308,6 +446,7 @@ struct lgr_fmt_ctx {
   std::string err;
   DeviceBuffer b_in, b_keep, b_out;  // one packed input arena, the dedup flags, the results
   DeviceBuffer b_ev, b_key;           // lgr_format_from_assign: per-read / per-variant inputs + slots, support keys
+  DeviceBuffer b_slab, b_dir;         // lgr_format_metrics_packed: the slab (+ status word), a directory outside it
   lgr_evidence_in last_ev{};  // device pointers of the columns the last call worked on (lgr_format_debug_evidence)
 };
 
@@ -656,6 +795,193 @@ int lgr_format_debug_evidence(lgr_fmt_ctx* c, lgr_evidence_in* dst) {
   LGR_CUDA(c, cp(dst->base_qual, L.base_qual, n));
   LGR_CUDA(c, cp(dst->map_qual, L.map_qual, n));
   return LGR_OK;
+}
+
+size_t lgr_format_packed_bytes(const lgr_evidence_in* in) {
+  if (!in || in->n_supports < 0 || in->n_evidence < 0) return 0;
+  uint64_t off[LGR_FMT_SECTIONS];
+  // a window without supports packs as an empty block (lgr_format_metrics returns before looking at its records)
+  return in->n_supports == 0 ? fmt_layout(0, 0, sizeof(lgr_fmt_blk_hdr), off)
+                             : fmt_layout(in->n_supports, in->n_evidence, sizeof(lgr_fmt_blk_hdr), off);
+}
+
+int lgr_format_pack(const lgr_evidence_in* in, void* dst, size_t cap, lgr_fmt_dir* dir) {
+  if (!in || !dst || in->n_supports < 0 || in->n_evidence < 0) return LGR_E_ARG;
+  const int S = in->n_supports;
+  const int64_t N = S == 0 ? 0 : in->n_evidence;
+  int n_wide = 0;
+  if (S > 0) {  // the checks of lgr_format_metrics (lgr_format.cu:358-379), in the same order
+    if (!in->sup_begin || !in->sup_n_alleles || !in->sup_variant_len || !in->sup_total_haps) return LGR_E_ARG;
+    if (in->sup_begin[0] != 0 || in->sup_begin[S] != N) return LGR_E_ARG;
+    for (int s = 0; s < S; ++s) {
+      if (in->sup_begin[s + 1] < in->sup_begin[s] || in->sup_n_alleles[s] < 1) return LGR_E_ARG;
+      n_wide += in->sup_n_alleles[s] > LGR_FMT_MAX_ALLELES;
+    }
+    if (N > 0 && !(in->insert_size && in->aln_start && in->aln_score && in->folded_pos && in->rname_hash && in->ref_nm &&
+                   in->own_hap_nm && in->hap_id && in->allele && in->flags && in->base_qual && in->map_qual))
+      return LGR_E_ARG;
+    for (int s = 0; s < S; ++s)
+      for (int64_t i = in->sup_begin[s]; i < in->sup_begin[s + 1]; ++i)
+        if (in->allele[i] >= in->sup_n_alleles[s]) return LGR_E_ARG;
+  }
+  lgr_fmt_blk_hdr h{};
+  h.magic = LGR_FMT_MAGIC, h.n_supports = S, h.n_evidence = N;
+  h.rec_bytes = fmt_layout(S, N, sizeof(lgr_fmt_blk_hdr), h.off);
+  if (cap < h.rec_bytes) return LGR_E_ARG;
+  uint8_t* p = static_cast<uint8_t*>(dst);
+  std::memcpy(p, &h, sizeof(h));
+  const void* src[LGR_FMT_SECTIONS] = {in->sup_begin, in->insert_size, in->aln_start, in->aln_score, in->folded_pos,
+                                       in->sup_n_alleles, in->sup_variant_len, in->sup_total_haps, in->rname_hash,
+                                       in->ref_nm, in->own_hap_nm, in->hap_id, in->allele, in->flags, in->base_qual,
+                                       in->map_qual};
+  for (int k = 0; k < LGR_FMT_SECTIONS; ++k) {
+    const uint64_t end = k + 1 < LGR_FMT_SECTIONS ? h.off[k + 1] : h.rec_bytes;
+    const uint64_t n = S == 0 ? 0 : (k == kSecBegin ? (uint64_t)S + 1 : fmt_sec_per_support(k) ? (uint64_t)S : (uint64_t)N) * fmt_sec_size(k);
+    if (n) std::memcpy(p + h.off[k], src[k], n);
+    std::memset(p + h.off[k] + n, 0, end - h.off[k] - n);  // padding: the bytes of a block depend on the window only
+  }
+  if (dir) {
+    *dir = lgr_fmt_dir{};
+    dir->n_supports = S, dir->n_evidence = N, dir->n_wide = n_wide;
+  }
+  return LGR_OK;
+}
+
+int lgr_format_metrics_packed(lgr_fmt_ctx* c, const lgr_fmt_packed_in* in, lgr_format* out, float* ms_kernels) {
+  if (!c || !in) return LGR_E_ARG;
+  c->err.clear();
+  if (ms_kernels) *ms_kernels = 0.0f;
+  const int W = in->n_windows;
+  if (W < 0) return c->err = "negative n_windows", LGR_E_ARG;
+  if (W == 0) return LGR_OK;
+  if (!in->slab || !in->dir) return c->err = "missing slab or directory", LGR_E_ARG;
+  // the directory only: each block's header must agree with its entry and the block must lie inside the slab, so that
+  // every read of k_fmt_unpack stays inside the device copy of the slab
+  const uint8_t* slab = static_cast<const uint8_t*>(in->slab);
+  int64_t S = 0, N = 0, n_wide = 0;
+  for (int w = 0; w < W; ++w) {
+    const lgr_fmt_dir& d = in->dir[w];
+    if (d.sup_base != S || d.ev_base != N) return c->err = "sup_base / ev_base are not the prefix sums of the counts", LGR_E_ARG;
+    if (d.n_supports < 0 || d.n_evidence < 0 || d.n_wide < 0 || d.n_wide > d.n_supports)
+      return c->err = "negative or inconsistent counts in the directory", LGR_E_ARG;
+    if (d.rec_off % 16 != 0 || d.rec_off > in->slab_bytes || in->slab_bytes - d.rec_off < sizeof(lgr_fmt_blk_hdr))
+      return c->err = "rec_off outside the slab or not 16-byte aligned", LGR_E_ARG;
+    lgr_fmt_blk_hdr h;
+    std::memcpy(&h, slab + d.rec_off, sizeof(h));
+    uint64_t off[LGR_FMT_SECTIONS];
+    const uint64_t bytes = fmt_layout(d.n_supports, d.n_evidence, sizeof(lgr_fmt_blk_hdr), off);
+    if (h.magic != LGR_FMT_MAGIC) return c->err = "bad block magic", LGR_E_ARG;
+    if (h.n_supports != d.n_supports || h.n_evidence != d.n_evidence || h.rec_bytes != bytes)
+      return c->err = "block header disagrees with its directory entry", LGR_E_ARG;
+    if (in->slab_bytes - d.rec_off < bytes) return c->err = "block runs past the end of the slab", LGR_E_ARG;
+    S += d.n_supports, N += d.n_evidence, n_wide += d.n_wide;
+    if (S > INT32_MAX) return c->err = "more than 2^31 - 1 supports", LGR_E_ARG;
+  }
+  if (S == 0) return LGR_OK;
+  if (!out) return c->err = "missing out", LGR_E_ARG;
+
+  LGR_CUDA(c, cudaSetDevice(c->device));
+  const size_t slab_bytes = (in->slab_bytes + 15) & ~(size_t)15;
+  const char* dir_p = reinterpret_cast<const char*>(in->dir);
+  const size_t dir_bytes = (size_t)W * sizeof(lgr_fmt_dir);
+  const bool dir_inside = dir_p >= (const char*)slab && (size_t)(dir_p - (const char*)slab) <= in->slab_bytes &&
+                          in->slab_bytes - (size_t)(dir_p - (const char*)slab) >= dir_bytes && (dir_p - (const char*)slab) % 16 == 0;
+  UnpackDev U;
+  const uint64_t arena_bytes = fmt_layout(S, N, 0, U.aoff);
+  int rc;
+  if ((rc = c->b_slab.ensure(slab_bytes + 16, false, c->err)) != LGR_OK) return rc;
+  if (!dir_inside && (rc = c->b_dir.ensure(dir_bytes, false, c->err)) != LGR_OK) return rc;
+  if ((rc = c->b_in.ensure(arena_bytes, false, c->err)) != LGR_OK) return rc;
+  if ((rc = c->b_keep.ensure((size_t)N, false, c->err)) != LGR_OK) return rc;
+  if ((rc = c->b_out.ensure((size_t)S * sizeof(lgr_format), false, c->err)) != LGR_OK) return rc;
+  uint8_t* dslab = static_cast<uint8_t*>(c->b_slab.p);
+  int* status = reinterpret_cast<int*>(dslab + slab_bytes);
+  LGR_CUDA(c, cudaMemcpyAsync(dslab, slab, in->slab_bytes, cudaMemcpyHostToDevice, c->stream));
+  if (!dir_inside) LGR_CUDA(c, cudaMemcpyAsync(c->b_dir.p, in->dir, dir_bytes, cudaMemcpyHostToDevice, c->stream));
+  LGR_CUDA(c, cudaMemsetAsync(status, 0, sizeof(int), c->stream));
+
+  U.slab = dslab;
+  U.dir = dir_inside ? reinterpret_cast<const lgr_fmt_dir*>(dslab + (dir_p - (const char*)slab)) : (const lgr_fmt_dir*)c->b_dir.p;
+  U.n_windows = W, U.n_supports = (int32_t)S, U.n_evidence = N;
+  U.n_rec_ctas = (N + kUnpackChunk - 1) / kUnpackChunk;
+  U.arena = static_cast<uint8_t*>(c->b_in.p);
+  U.status = status;
+  uint8_t* base = U.arena;
+  FmtDev D;
+  D.e.insert_size = (const int64_t*)(base + U.aoff[1]), D.e.aln_start = (const int64_t*)(base + U.aoff[2]);
+  D.e.aln_score = (const double*)(base + U.aoff[3]), D.e.folded_pos = (const double*)(base + U.aoff[4]);
+  D.e.rname_hash = (const uint32_t*)(base + U.aoff[8]), D.e.ref_nm = (const uint32_t*)(base + U.aoff[9]);
+  D.e.own_hap_nm = (const uint32_t*)(base + U.aoff[10]), D.e.hap_id = (const uint32_t*)(base + U.aoff[11]);
+  D.e.allele = (const uint8_t*)(base + U.aoff[12]), D.e.flags = (const uint8_t*)(base + U.aoff[13]);
+  D.e.base_qual = (const uint8_t*)(base + U.aoff[14]), D.e.map_qual = (const uint8_t*)(base + U.aoff[15]);
+  D.e.keep = (const uint8_t*)c->b_keep.p;
+  D.sup_begin = (const int64_t*)(base + U.aoff[kSecBegin]), D.sup_n_alleles = (const int32_t*)(base + U.aoff[kSecK]);
+  D.sup_variant_len = (const int32_t*)(base + U.aoff[kSecVl]), D.sup_total_haps = (const int32_t*)(base + U.aoff[kSecTh]);
+  D.keep = (uint8_t*)c->b_keep.p, D.out = (lgr_format*)c->b_out.p;
+  D.n_supports = (int32_t)S, D.n_evidence = N;
+
+  LGR_CUDA(c, cudaEventRecord(c->ev0, c->stream));
+  {
+    const int64_t blocks = U.n_rec_ctas + (S + kUnpackWarps - 1) / kUnpackWarps;
+    k_fmt_unpack<<<(unsigned)blocks, kUnpackThreads, 0, c->stream>>>(U);
+    LGR_CUDA(c, cudaGetLastError());
+  }
+  if (N > 0) {  // the grid rule of lgr_format_metrics
+    k_fmt_dedup<<<(unsigned)((N + 255) / 256), 256, 0, c->stream>>>(D);
+    LGR_CUDA(c, cudaGetLastError());
+  }
+  {
+    const int64_t cap = (int64_t)c->sm_count * 32;
+    const dim3 grid((unsigned)(S < cap ? S : cap), (unsigned)lgr_fmt::kNumTasks);
+    k_fmt_metrics<<<grid, lgr_fmt::kThreads, 0, c->stream>>>(D);
+    LGR_CUDA(c, cudaGetLastError());
+  }
+  LGR_CUDA(c, cudaEventRecord(c->ev1, c->stream));
+  int bad = 0;
+  LGR_CUDA(c, cudaMemcpyAsync(out, c->b_out.p, (size_t)S * sizeof(lgr_format), cudaMemcpyDeviceToHost, c->stream));
+  LGR_CUDA(c, cudaMemcpyAsync(&bad, status, sizeof(int), cudaMemcpyDeviceToHost, c->stream));
+  LGR_CUDA(c, cudaStreamSynchronize(c->stream));
+  if (ms_kernels) LGR_CUDA(c, cudaEventElapsedTime(ms_kernels, c->ev0, c->ev1));
+  if (bad) return c->err = "a packed block holds malformed records (sup_begin, K or an allele >= K)", LGR_E_ARG;
+  if (n_wide == 0) return LGR_OK;
+  // wide supports: the records lgr_format_metrics gives them, found through the windows that declare some
+  int64_t seen = 0;
+  for (int w = 0; w < W; ++w) {
+    const lgr_fmt_dir& d = in->dir[w];
+    if (d.n_wide == 0) continue;
+    uint64_t off[LGR_FMT_SECTIONS];
+    fmt_layout(d.n_supports, d.n_evidence, sizeof(lgr_fmt_blk_hdr), off);
+    for (int s = 0; s < d.n_supports; ++s) {
+      int32_t K;
+      std::memcpy(&K, slab + d.rec_off + off[kSecK] + 4 * (size_t)s, 4);
+      if (K > LGR_FMT_MAX_ALLELES) {
+        lgr_format& r = out[d.sup_base + s];
+        std::memset(&r, 0, sizeof(lgr_format));
+        r.n_alleles = (uint32_t)K, r.valid = LGR_FMT_WIDE;
+        ++seen;
+      }
+    }
+  }
+  if (seen != n_wide) return c->err = "n_wide of the directory disagrees with the blocks", LGR_E_ARG;
+  c->err = "some supports have more than LGR_FMT_MAX_ALLELES alleles (records flagged LGR_FMT_WIDE)";
+  return LGR_E_PARTIAL;
+}
+
+int lgr_format_reserve(lgr_fmt_ctx* c, int64_t slab_bytes, int32_t n_supports, int64_t n_evidence) {
+  if (!c || slab_bytes < 0 || n_supports < 0 || n_evidence < 0) return LGR_E_ARG;
+  c->err.clear();
+  LGR_CUDA(c, cudaSetDevice(c->device));
+  uint64_t off[LGR_FMT_SECTIONS];
+  int rc;
+  if ((rc = c->b_slab.ensure((((size_t)slab_bytes + 15) & ~(size_t)15) + 16, true, c->err)) != LGR_OK) return rc;
+  if ((rc = c->b_in.ensure(fmt_layout(n_supports, n_evidence, 0, off), true, c->err)) != LGR_OK) return rc;
+  if ((rc = c->b_keep.ensure((size_t)n_evidence, true, c->err)) != LGR_OK) return rc;
+  return c->b_out.ensure((size_t)n_supports * sizeof(lgr_format), true, c->err);
+}
+
+int64_t lgr_format_device_bytes(const lgr_fmt_ctx* c) {
+  if (!c) return 0;
+  return (int64_t)(c->b_in.cap + c->b_keep.cap + c->b_out.cap + c->b_ev.cap + c->b_key.cap + c->b_slab.cap + c->b_dir.cap);
 }
 
 }  // extern "C"

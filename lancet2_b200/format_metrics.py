@@ -64,6 +64,36 @@ class GpuFormatMetrics:
                                f"{self._lib.lgr_format_last_error(self._ctx).decode()}")
         return out, float(ms.value)
 
+    def compute_packed(self, windows, dir_inside: bool = True) -> Tuple[np.ndarray, float]:
+        """The same records as compute() on every window's supports concatenated, through lgr_format_pack and ONE
+        lgr_format_metrics_packed.  `windows`: a sequence of windows (lists of support dicts) or a PackedWindows."""
+        pk = windows if isinstance(windows, PackedWindows) else PackedWindows(windows, self._main, dir_inside)
+        return self.metrics_packed(pk)
+
+    def metrics_packed(self, pk: PackedWindows, slab_ptr: int = 0) -> Tuple[np.ndarray, float]:
+        """lgr_format_metrics_packed on packed windows (slab_ptr: a copy of pk.slab to send instead, e.g. pinned).
+        → (records of every window's supports in directory order, CUDA-event ms of the three kernels)."""
+        if self._lib is not self._main:
+            raise RuntimeError("the packed path is not part of the A/B FORMAT libraries")
+        out = np.zeros(max(pk.n_supports, 1), dtype=abi.FORMAT_DTYPE)
+        st = pk.c_struct(slab_ptr)
+        ms = C.c_float(0.0)
+        rc = self._lib.lgr_format_metrics_packed(self._ctx, C.byref(st), out.ctypes.data, C.byref(ms))
+        self.last_rc = rc
+        if rc not in (0, abi.LGR_E_PARTIAL):
+            raise RuntimeError(f"lgr_format_metrics_packed failed ({self._main.lgr_strerror(rc).decode()}): "
+                               f"{self._lib.lgr_format_last_error(self._ctx).decode()}")
+        return out[:pk.n_supports], float(ms.value)
+
+    def reserve(self, slab_bytes: int, n_supports: int, n_evidence: int) -> None:
+        rc = self._main.lgr_format_reserve(self._ctx, slab_bytes, n_supports, n_evidence)
+        if rc != 0:
+            raise RuntimeError(f"lgr_format_reserve failed: {self._main.lgr_format_last_error(self._ctx).decode()}")
+
+    def device_bytes(self) -> int:
+        """device bytes the context holds (lgr_format_device_bytes)"""
+        return int(self._main.lgr_format_device_bytes(self._ctx))
+
     def from_assign(self, batch: "abi.Batch", *, n_samples: int, sample_id, start0, isize, sam_flag, mapq, softclip,
                     var_n_alleles, var_len, host_assign=None, dev_assign: int = 0):
         """AddToTable + FORMAT math on the device (lgr_format_from_assign): evidence columns are built by
@@ -115,3 +145,125 @@ class GpuFormatMetrics:
         if self._lib.lgr_format_debug_evidence(self._ctx, C.byref(st)) != 0:
             raise RuntimeError("lgr_format_debug_evidence failed")
         return cols
+
+
+class PackedWindows:
+    """Windows (each a list of support dicts, or an abi.EvidenceBatch) packed with lgr_format_pack into one slab, the
+    directory placed behind the blocks (one host->device copy) or, with dir_inside=False, in an array of its own.
+    `dir` is a numpy view (abi.FMT_DIR_DTYPE) that may be edited before the call."""
+
+    def __init__(self, windows, lib, dir_inside: bool = True):
+        self.batches = [w if isinstance(w, abi.EvidenceBatch) else abi.EvidenceBatch(w) for w in windows]
+        structs = [b.c_struct() for b in self.batches]
+        sizes = [int(lib.lgr_format_packed_bytes(C.byref(st))) for st in structs]
+        if any(n == 0 for n in sizes):
+            raise ValueError("malformed window (lgr_format_packed_bytes returned 0)")
+        self.rec_bytes = sum(sizes)
+        n = len(structs)
+        dir_bytes = n * abi.FMT_DIR_DTYPE.itemsize
+        self.slab = np.zeros(self.rec_bytes + (dir_bytes if dir_inside else 0) + 16, dtype=np.uint8)
+        self.slab_bytes = self.rec_bytes + (dir_bytes if dir_inside else 0)
+        if dir_inside:
+            self.dir = self.slab[self.rec_bytes:self.rec_bytes + dir_bytes].view(abi.FMT_DIR_DTYPE)
+        else:
+            self.dir = np.zeros(n, dtype=abi.FMT_DIR_DTYPE)
+        off = sup = ev = 0
+        d = abi.LgrFmtDir()
+        for w, (st, size) in enumerate(zip(structs, sizes)):
+            rc = lib.lgr_format_pack(C.byref(st), self.slab.ctypes.data + off, size, C.byref(d))
+            if rc != 0:
+                raise ValueError(f"lgr_format_pack refused window {w} ({rc})")
+            self.dir[w] = (off, d.n_evidence, ev, d.n_supports, sup, d.n_wide, (0, 0, 0))
+            off, sup, ev = off + size, sup + d.n_supports, ev + d.n_evidence
+        self.n_windows, self.n_supports, self.n_evidence = n, sup, ev
+
+    def c_struct(self, slab_ptr: int = 0) -> abi.LgrFmtPackedIn:
+        """slab_ptr: the address of a copy of self.slab (e.g. pinned memory) to hand over instead"""
+        st = abi.LgrFmtPackedIn()
+        st.n_windows, st.slab_bytes = self.n_windows, self.slab_bytes
+        st.slab = slab_ptr or self.slab.ctypes.data
+        inside = self.dir.base is not None and np.shares_memory(self.dir, self.slab)
+        st.dir = (st.slab + self.rec_bytes) if inside else self.dir.ctypes.data
+        return st
+
+
+def _bind_calculator(lib: C.CDLL) -> C.CDLL:
+    lib.lgr_adapter_format_calculator_create.argtypes = [C.c_int, C.c_longlong, C.c_longlong, C.c_longlong, C.c_char_p, C.c_int]
+    lib.lgr_adapter_format_calculator_create.restype = C.c_void_p
+    lib.lgr_adapter_format_calculator_destroy.argtypes = [C.c_void_p]
+    lib.lgr_adapter_format_calculator_destroy.restype = None
+    lib.lgr_adapter_format_calculator_run.argtypes = [C.c_void_p, C.POINTER(abi.LgrEvidenceIn), C.c_void_p, C.c_int, C.c_int,
+                                                      C.c_void_p, C.c_void_p, C.c_void_p]
+    lib.lgr_adapter_format_calculator_run.restype = C.c_int
+    lib.lgr_adapter_format_private_run.argtypes = [C.c_int, C.POINTER(abi.LgrEvidenceIn), C.c_void_p, C.c_int, C.c_int,
+                                                   C.c_void_p, C.c_void_p]
+    lib.lgr_adapter_format_private_run.restype = C.c_longlong
+    return lib
+
+
+class _FlatWindows:
+    """Windows as one flat EvidenceBatch plus the support range of each window (the adapter's run hooks)."""
+
+    def __init__(self, windows):
+        self.batch = abi.EvidenceBatch([s for w in windows for s in w])
+        self.win_sup_begin = np.concatenate([[0], np.cumsum([len(w) for w in windows])]).astype(np.int32)
+        self.n = len(windows)
+        self.st = self.batch.c_struct()
+        self.out = np.zeros(max(self.batch.n_supports, 1), dtype=abi.FORMAT_DTYPE)
+        self.status = np.full(self.n + 1, -1, dtype=np.int32)
+
+    def per_window(self):
+        return [self.out[self.win_sup_begin[w]:self.win_sup_begin[w + 1]].copy() for w in range(self.n)]
+
+
+class FormatCalculator:
+    """Handle on the C++ lancet_gpu::FormatCalculator (host/gpu_format.h): one calculator per GPU, called from many
+    C++ threads.  Construction raises without a GPU (no CPU fallback)."""
+
+    COUNTERS = ("batches", "windows", "supports", "evidence", "max_windows_in_batch", "alone", "ns_pack", "ns_seal_wait",
+                "ns_device", "ns_wall")
+
+    def __init__(self, device: int = 0, slab_bytes: int = 0, max_supports: int = 0, max_evidence: int = 0):
+        """slab_bytes / max_supports / max_evidence: the calculator's per-slab sizes (0 = its defaults)."""
+        self._lib = _bind_calculator(abi.load_library())
+        err = C.create_string_buffer(512)
+        self._h = self._lib.lgr_adapter_format_calculator_create(device, slab_bytes, max_supports, max_evidence, err, len(err))
+        if not self._h:
+            raise RuntimeError(f"FormatCalculator construction failed: {err.value.decode()}")
+
+    def close(self) -> None:
+        if getattr(self, "_h", None):
+            self._lib.lgr_adapter_format_calculator_destroy(self._h)
+            self._h = None
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
+
+    def run(self, windows, threads: int = 1):
+        """Every window (a list of support dicts) through FormatCalculator::Compute from `threads` C++ threads (window w
+        on thread w % threads).  → (records per window, status per window: 0 ok, 1 std::invalid_argument, 2 other
+        exception, counters)."""
+        if not self._h:
+            raise RuntimeError("FormatCalculator is closed")
+        fw = _FlatWindows(windows)
+        ctr = (C.c_ulonglong * len(self.COUNTERS))()
+        rc = self._lib.lgr_adapter_format_calculator_run(self._h, C.byref(fw.st), fw.win_sup_begin.ctypes.data, fw.n, threads,
+                                                         fw.out.ctypes.data, fw.status.ctypes.data, ctr)
+        if rc != 0:
+            raise RuntimeError(f"lgr_adapter_format_calculator_run failed ({rc})")
+        return fw.per_window(), fw.status[:fw.n].copy(), dict(zip(self.COUNTERS, list(ctr)))
+
+
+def private_contexts_run(windows, threads: int = 1, device: int = 0):
+    """The binding without a calculator: every C++ thread owns a FORMAT context and makes one lgr_format_metrics per
+    window.  → (records per window, status per window, wall ns)."""
+    lib = _bind_calculator(abi.load_library())
+    fw = _FlatWindows(windows)
+    ns = lib.lgr_adapter_format_private_run(device, C.byref(fw.st), fw.win_sup_begin.ctypes.data, fw.n, threads,
+                                            fw.out.ctypes.data, fw.status.ctypes.data)
+    if ns < 0:
+        raise RuntimeError("lgr_adapter_format_private_run: no FORMAT context")
+    return fw.per_window(), fw.status[:fw.n].copy(), int(ns)

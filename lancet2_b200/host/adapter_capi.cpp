@@ -12,6 +12,7 @@
 #include <thread>
 #include <vector>
 
+#include "gpu_format.h"
 #include "gpu_genotyper.h"
 #include "gpu_repeat.h"
 
@@ -606,6 +607,177 @@ long long lgr_adapter_repeat_private_run(int device, const unsigned char* seqs, 
   }
   for (auto* c : ctx) lgr_repeat_destroy(c);
   return wall;
+}
+
+}  // extern "C"
+
+namespace {
+
+// The windows of a FormatCalculator run: window w = supports win_sup_begin[w] .. win_sup_begin[w + 1] of the flat
+// columns `all`, as a window-local lgr_evidence_in (sup_begin rebased to 0, columns offset to its first record).
+// Built before any clock starts; records go to out[win_sup_begin[w] ..].
+struct FormatWindows {
+  std::vector<std::vector<std::int64_t>> begin;
+  std::vector<lgr_evidence_in> in;
+  const int* win_sup_begin;
+  FormatWindows(const lgr_evidence_in* all, const int* wsb, int n_windows) : begin((std::size_t)n_windows), in((std::size_t)n_windows), win_sup_begin(wsb) {
+    for (int w = 0; w < n_windows; ++w) {
+      const int s0 = wsb[w], s1 = wsb[w + 1];
+      const std::int64_t e0 = all->sup_begin[s0];
+      auto& b = begin[(std::size_t)w];
+      for (int s = s0; s <= s1; ++s) b.push_back(all->sup_begin[s] - e0);
+      lgr_evidence_in& x = in[(std::size_t)w];
+      x = *all;
+      x.n_supports = s1 - s0, x.n_evidence = b.back();
+      x.sup_begin = b.data(), x.sup_n_alleles = all->sup_n_alleles + s0, x.sup_variant_len = all->sup_variant_len + s0;
+      x.sup_total_haps = all->sup_total_haps + s0;
+      x.insert_size = all->insert_size + e0, x.aln_start = all->aln_start + e0, x.aln_score = all->aln_score + e0;
+      x.folded_pos = all->folded_pos + e0, x.rname_hash = all->rname_hash + e0, x.ref_nm = all->ref_nm + e0;
+      x.own_hap_nm = all->own_hap_nm + e0, x.hap_id = all->hap_id + e0, x.allele = all->allele + e0, x.flags = all->flags + e0;
+      x.base_qual = all->base_qual + e0, x.map_qual = all->map_qual + e0;
+    }
+  }
+};
+
+// n_threads threads; thread t computes windows t, t + n_threads, ... in order, one blocking call each.  ask(w, t)
+// returns the records of window w; status[w] = 0 ok, 1 std::invalid_argument, 2 any other exception.  Returns the wall
+// nanoseconds from the start to the last join.
+template <typename Ask>
+unsigned long long RunFormatWindows(const FormatWindows& win, int n_threads, lgr_format* out, int* status, Ask ask) {
+  const int n_windows = (int)win.in.size();
+  std::vector<std::thread> threads;
+  const auto t0 = std::chrono::steady_clock::now();
+  for (int t = 0; t < n_threads; ++t) {
+    threads.emplace_back([&, t] {
+      for (int w = t; w < n_windows; w += n_threads) {
+        try {
+          const std::vector<lgr_format> r = ask(w, t);
+          std::memcpy(out + win.win_sup_begin[w], r.data(), r.size() * sizeof(lgr_format));
+          status[w] = 0;
+        } catch (const std::invalid_argument&) {
+          status[w] = 1;
+        } catch (const std::exception&) {
+          status[w] = 2;
+        }
+      }
+    });
+  }
+  for (auto& th : threads) th.join();
+  return (unsigned long long)std::chrono::duration_cast<std::chrono::nanoseconds>(std::chrono::steady_clock::now() - t0).count();
+}
+
+}  // namespace
+
+extern "C" {
+
+// lancet_gpu::FormatCalculator for the tests and tools/bench_format_calculator.py.  Sizes <= 0 keep the defaults.
+// NULL (message in err) when construction throws, e.g. without a GPU.
+void* lgr_adapter_format_calculator_create(int device, long long slab_bytes, long long max_supports, long long max_evidence,
+                                           char* err, int err_cap) {
+  try {
+    lancet_gpu::FormatCalculator::Options opt;
+    opt.device = device;
+    if (slab_bytes > 0) opt.slab_bytes = (std::size_t)slab_bytes;
+    if (max_supports > 0) opt.max_supports = (std::size_t)max_supports;
+    if (max_evidence > 0) opt.max_evidence = (std::size_t)max_evidence;
+    return new lancet_gpu::FormatCalculator(opt);
+  } catch (const std::exception& e) {
+    if (err && err_cap > 0) std::snprintf(err, (size_t)err_cap, "%s", e.what());
+    return nullptr;
+  }
+}
+
+void lgr_adapter_format_calculator_destroy(void* calc) { delete static_cast<lancet_gpu::FormatCalculator*>(calc); }
+
+// n_threads C++ threads call FormatCalculator::Compute on their share of the windows (see RunFormatWindows).
+// counters[10] = batches, windows, supports, evidence, max windows in a batch, alone, ns_pack, ns_seal_wait, ns_device,
+// wall ns of the run.
+int lgr_adapter_format_calculator_run(void* calc, const lgr_evidence_in* all, const int* win_sup_begin, int n_windows,
+                                      int n_threads, lgr_format* out, int* status, unsigned long long* counters) {
+  if (!calc || !all || n_threads <= 0 || n_windows < 0) return -1;
+  auto* fc = static_cast<lancet_gpu::FormatCalculator*>(calc);
+  const FormatWindows win(all, win_sup_begin, n_windows);
+  const unsigned long long wall = RunFormatWindows(win, n_threads, out, status, [&](int w, int) { return fc->Compute(win.in[(std::size_t)w]); });
+  const lancet_gpu::FormatCalculator::Counters c = fc->Stats();
+  const std::uint64_t v[10] = {c.batches, c.windows, c.supports, c.evidence, c.max_windows_in_batch, c.alone, c.ns_pack,
+                               c.ns_seal_wait, c.ns_device, wall};
+  for (int i = 0; i < 10; ++i) counters[i] = v[i];
+  return 0;
+}
+
+// The binding without the calculator, for comparison: every thread owns an lgr_fmt_ctx (what GpuFormatMetrics wraps,
+// created before the clock starts) and makes one lgr_format_metrics per window.  Returns the wall ns of the run, < 0
+// when a context cannot be created.
+long long lgr_adapter_format_private_run(int device, const lgr_evidence_in* all, const int* win_sup_begin, int n_windows,
+                                         int n_threads, lgr_format* out, int* status) {
+  if (!all || n_threads <= 0 || n_windows < 0) return -1;
+  std::vector<lgr_fmt_ctx*> ctx((size_t)n_threads, nullptr);
+  bool ok = true;
+  for (auto& c : ctx) ok = ok && lgr_format_create(device, &c) == LGR_OK;
+  long long wall = -1;
+  if (ok) {
+    const FormatWindows win(all, win_sup_begin, n_windows);
+    wall = (long long)RunFormatWindows(win, n_threads, out, status, [&](int w, int t) {
+      const lgr_evidence_in& x = win.in[(std::size_t)w];
+      std::vector<lgr_format> r((std::size_t)std::max(x.n_supports, 0));
+      const int rc = lgr_format_metrics(ctx[(size_t)t], &x, r.data(), nullptr);
+      if (rc == LGR_E_ARG) throw std::invalid_argument(lgr_format_last_error(ctx[(size_t)t]));
+      if (rc != LGR_OK && rc != LGR_E_PARTIAL) throw std::runtime_error(lgr_format_last_error(ctx[(size_t)t]));
+      return r;
+    });
+  }
+  for (auto* c : ctx) lgr_format_destroy(c);
+  return wall;
+}
+
+// End to end: EvidenceColumns::AppendJob of every group of a realignment batch (the inputs of
+// lgr_adapter_format_metrics), one window per group.  n_threads threads compute the windows through one
+// FormatCalculator (out_calc), and GpuFormatMetrics::Compute computes the same columns (out_plain), both in the batch's
+// support order.  Returns the number of supports, < 0 on error (message in err).
+int lgr_adapter_format_calculator_columns(int device, const lgr_batch_in* in, const char* names, const char* samples,
+                                          const int* sample_id, const long long* start0, const long long* isize,
+                                          const unsigned short* sam_flag, const unsigned char* mapq, const unsigned char* softclip,
+                                          const lgr_assign* assign, int n_threads, lgr_format* out_calc, lgr_format* out_plain,
+                                          int n_out, char* err, int err_cap) {
+  try {
+    JobSet js;
+    BuildJobs(in, names, samples, sample_id, start0, isize, sam_flag, mapq, softclip, js);
+    std::vector<lancet_gpu::EvidenceColumns> cols(js.jobs.size());
+    std::vector<int> first(js.jobs.size() + 1, 0);
+    long long off = 0;
+    for (std::size_t g = 0; g < js.jobs.size(); ++g) {
+      cols[g].AppendJob(js.jobs[g], assign + off, X31OfView);
+      off += (long long)(js.jobs[g].n_reads * js.jobs[g].n_variants);
+      first[g + 1] = first[g] + (int)cols[g].NumSupports();
+    }
+    if (first.back() > n_out) throw std::runtime_error("output too small");
+    lancet_gpu::GpuFormatMetrics fm(device);
+    for (std::size_t g = 0; g < cols.size(); ++g) {
+      const std::vector<lgr_format> r = fm.Compute(cols[g]);
+      std::memcpy(out_plain + first[g], r.data(), r.size() * sizeof(lgr_format));
+    }
+    lancet_gpu::FormatCalculator fc(device);
+    std::vector<std::thread> threads;
+    std::vector<std::string> errors((std::size_t)std::max(n_threads, 1));
+    for (int t = 0; t < n_threads; ++t)
+      threads.emplace_back([&, t] {
+        try {
+          for (std::size_t g = (std::size_t)t; g < cols.size(); g += (std::size_t)n_threads) {
+            const std::vector<lgr_format> r = fc.Compute(cols[g]);
+            std::memcpy(out_calc + first[g], r.data(), r.size() * sizeof(lgr_format));
+          }
+        } catch (const std::exception& e) {
+          errors[(std::size_t)t] = e.what();
+        }
+      });
+    for (auto& th : threads) th.join();
+    for (const std::string& e : errors)
+      if (!e.empty()) throw std::runtime_error(e);
+    return first.back();
+  } catch (const std::exception& e) {
+    std::snprintf(err, (size_t)err_cap, "%s", e.what());
+    return -2;
+  }
 }
 
 }  // extern "C"
